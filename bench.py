@@ -2,6 +2,7 @@
 """Benchmark of the ReconfigISP hot path on B200 (driver contract: one JSON line on stdout from rank 0).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload tuning|search] [--impl b200|reference|torch_eager]
+                  [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...          (one rank per GPU, weak scaling)
 
 --workload tuning (default) = BASELINE.json configs[1], the configuration `metric` is quoted on: one proxy-tuning step
@@ -110,8 +111,9 @@ def opt_search():
 
 
 # ---- CPU arms (oracle port of the reference path; the only place bench.py executes oracle/) ---------------------------
-def cpu_tuning_rate(sample_hw, reps, threads=None):
-    """fwd + MSE + backward of the stage parameters on one frame of `sample_hw`.  -> (MP/s, cores, seconds per rep)."""
+def cpu_tuning_rate(sample_hw, reps, threads=None, warmup=1):
+    """fwd + MSE + backward of the stage parameters on one frame of `sample_hw`, `warmup` untimed then `reps` timed.
+    -> (MP/s, cores, seconds per rep)."""
     import torch
     from oracle import pipeline_oracle as PO
     from reconfigisp_b200.synthetic import synthetic_frames
@@ -126,7 +128,8 @@ def cpu_tuning_rate(sample_hw, reps, threads=None):
         loss = ((y - gt) ** 2).mean()
         nz = [l for l in pipe.logits if l.numel()]
         torch.autograd.grad(loss, nz)
-    step()
+    for _ in range(warmup):
+        step()
     t0 = time.perf_counter()
     for _ in range(reps):
         step()
@@ -134,9 +137,9 @@ def cpu_tuning_rate(sample_hw, reps, threads=None):
     return h * w / 1e6 / dt, torch.get_num_threads(), dt
 
 
-def cpu_search_rate(batch, size, reps):
-    """One DARTS iteration (5 supernet fwd+bwd passes) of the oracle supernet on `batch` patches of `size`^2.
-    -> (MP/s per pass, cores, seconds per iteration)."""
+def cpu_search_rate(batch, size, reps, warmup=0):
+    """One DARTS iteration (5 supernet fwd+bwd passes) of the oracle supernet on `batch` patches of `size`^2, `warmup` untimed
+    then `reps` timed.  -> (MP/s per pass, cores, seconds per iteration)."""
     import torch
     from oracle import pipeline_oracle as PO
     from reconfigisp_b200.synthetic import synthetic_frames
@@ -147,6 +150,8 @@ def cpu_search_rate(batch, size, reps):
 
     def it():
         PO.darts_step(netG, netV, raw[:batch], gt[:batch], raw[batch:], gt[batch:], 1e-3, 0.9, 1e-3)
+    for _ in range(warmup):
+        it()
     t0 = time.perf_counter()
     for _ in range(reps):
         it()
@@ -157,21 +162,21 @@ def cpu_search_rate(batch, size, reps):
 def run_reference(args):
     if int(os.environ.get('RANK', '0')) != 0:
         return 0
-    n = max(1, args.steps + args.warmup)
     if args.workload == 'search':
         # a step = one DARTS iteration of the CPU port on a bounded sample (2 patches of 64x64 take seconds: the supernet runs
-        # 51 candidates incl. median / NLM / bilateral five times); steps are capped so the run stays within a few minutes
-        n = min(n, 6)
-        rate, cores, dt = cpu_search_rate(2, 64, n)
-        sample = '2+2 patches of 64x64 per iteration (train/val halves), %d iterations (oracle/pipeline_oracle.py darts_step, torch CPU)' % n
+        # 51 candidates incl. median / NLM / bilateral five times)
+        rate, cores, dt = cpu_search_rate(2, 64, args.steps, args.warmup)
+        sample = '2+2 patches of 64x64 per iteration (train/val halves), %d iterations after %d warm-up (oracle/pipeline_oracle.py ' \
+                 'darts_step, torch CPU)' % (args.steps, args.warmup)
         metric, workload = METRIC_SEARCH, 'configs[2]: DARTS search iteration, n_step=3, 51 candidates; CPU sample: %s' % sample
     else:
         # a step = one fwd+bwd of the CPU port on a bounded crop of one 12 MP frame, sized from a probe so that the whole
         # --steps/--warmup run stays within ~2 minutes
         _, _, probe_dt = cpu_tuning_rate((752, 1000), 1)
+        n = args.steps + args.warmup
         scale = min(4.0, max(0.25, (120.0 / n) / max(probe_dt, 1e-3)))         # pixels relative to the probe crop
         hw = (int(752 * scale ** 0.5) // 2 * 2, int(1000 * scale ** 0.5) // 4 * 4)
-        rate, cores, dt = cpu_tuning_rate(hw, max(1, n - 1))
+        rate, cores, dt = cpu_tuning_rate(hw, args.steps, warmup=args.warmup)
         sample = '1 frame crop of %dx%d per step (oracle/pipeline_oracle.py FixedPipeline, torch CPU)' % hw
         metric, workload = METRIC, 'configs[1]: fixed pipeline %s fwd+bwd (proxy tuning), 12MP RGGB raws; CPU sample: %s' % (ARCH, sample)
     line = {'impl': 'reference', 'metric': metric, 'value': round(rate, 3), 'unit': 'MP/s', 'n_gpus': args.gpus,
@@ -210,6 +215,32 @@ class Timer:
         if self.world > 1:
             self.dist.all_reduce(ms, op=self.dist.ReduceOp.MAX)
         return float(ms.item())
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(net, params, **scalars):
+    """Host float32 copies of what a training step hands its caller: the given device scalars (the loss) and, by parameter
+    name, every trainable tensor after the update (`param.<name>`) with the gradient the step computed for it (`grad.<name>`)."""
+    keep = {id(p) for p in params}
+    out = dict(scalars)
+    for name, p in net.named_parameters():
+        if id(p) in keep and p.numel():
+            out['param.' + name] = p
+            if p.grad is not None:
+                out['grad.' + name] = p.grad
+    return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+
+
+def dump_outputs(path, arrays):
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError('--dump-outputs: %d bytes exceed the %d-byte limit' % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def teardown(world, dist, models):
@@ -257,6 +288,8 @@ def run_tuning(args):
     sampler.start()
     ms_step = timed(model.optimize_parameters, args.steps, args.warmup) / args.steps
     value = world * px / 1e6 / (ms_step / 1e3)
+    # taken now: the legs below keep training the same model
+    outputs = step_outputs(model.netG, model.netG.trainable_parameters, loss=model.log_dict['loss']) if args.dump_outputs else None
 
     # ---- e2e: host buffers through the public API; the copy of batch k+1 overlaps the step of batch k ------------
     def e2e_loop(batches):
@@ -356,6 +389,8 @@ def run_tuning(args):
                                           '(oracle/pipeline_oracle.py FixedPipeline, torch CPU)' % (H, W, 9 * dt)}
     if rank == 0:
         print(json.dumps(line), flush=True)
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
     teardown(world, dist, [model, light])
     return 0
 
@@ -391,10 +426,15 @@ def run_search(args):
     l0 = L.size('risp_launch_count')
     it()
     own_launches = L.size('risp_launch_count') - l0
-    steps = max(1, min(args.steps, 20))
+    steps = args.steps
     ms_it = timed(it, steps, min(args.warmup, 3)) / steps
     px = B * S * S
     value = world * 5 * px / 1e6 / (ms_it / 1e3)
+    outputs = None
+    if args.dump_outputs:
+        # taken now: the legs below keep searching with the same model
+        outputs = step_outputs(m.netG, list(m.netG.trainable_parameters) + list(m.netG.alphas), loss=m.log_dict['loss'],
+                               val_loss=m.val_loss)
 
     def e2e_it():
         m.feed_data(host)
@@ -452,6 +492,8 @@ def run_search(args):
                                 'sample': '2 iterations on 4+4 patches of 96x96 = %.1f s (oracle/pipeline_oracle.py darts_step, torch CPU)' % (2 * dt)}
     if rank == 0:
         print(json.dumps(line), flush=True)
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
     teardown(world, dist, [])
     return 0
 
@@ -504,7 +546,7 @@ def run_torch_eager(args):
     for _ in range(max(1, min(args.warmup, 3))):
         step()
     torch.cuda.synchronize()
-    n = max(2, min(args.steps, 10))
+    n = args.steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(n):
@@ -523,14 +565,22 @@ def run_torch_eager(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=200)
+    ap.add_argument('--steps', type=int, default=None, help='timed steps (default: 200 for tuning, 20 for search)')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference', 'torch_eager'])
     ap.add_argument('--workload', default='tuning', choices=['tuning', 'search'])
     ap.add_argument('--frames', type=int, default=FRAMES_PER_GPU, help='tuning: 12MP frames per GPU per step')
     ap.add_argument('--batch', type=int, default=SEARCH_BATCH, help='search: 256x256 patches per GPU (train half; as many again for validation)')
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='b200: write the loss, the updated parameters and their gradients of the '
+                    'last timed step to DIR/<name>.npy (float32)')
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 20 if args.workload == 'search' else 200        # a search iteration costs ~5000 tuning steps
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     if args.impl == 'reference':
         return run_reference(args)
