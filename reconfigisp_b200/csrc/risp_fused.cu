@@ -10,7 +10,8 @@
 //     summation order is fixed (bit-reproducible gradients);
 //   * a warp owns a 128-column strip and marches down the rows with the demosaic window in registers (horizontal halo
 //     by shuffle), two rows per loop trip so the CFA row parity is a compile-time constant;
-//   * the chain runs on pixel PAIRS with FFMA2/FMUL2/FADD2, coefficients from uniform registers (risp_fused.cuh).
+//   * the chain runs on pixel PAIRS with FFMA2/FMUL2/FADD2, coefficients from uniform registers; the FMA-heavy sites of the
+//     backward-carrying kernels use scalar FFMA and accumulate both pixels of a pair into one sum (risp_fused.cuh).
 #include "risp_fused.cuh"
 
 #include <cuda.h>
@@ -270,6 +271,7 @@ __host__ __device__ constexpr bool per_channel_from(int k) {     // stages k.. n
 template <unsigned SIG, int K, int MODE, int C, bool NOMASK = false>
 struct Tail {
   static constexpr EffChain E = Eff<SIG>::e;
+  static constexpr bool SC = !per_channel_from<SIG>(0);    // scalar fp32 sites: chains with the polynomial (risp_fused.cuh)
   static __device__ __forceinline__ float2 go(float2 x, float2 tgt, const float* __restrict__ cp, float2* acc, float2& loss,
                                               float2& yout, bool slow, float lane_w, uint32_t tbl) {
     if constexpr (K == E.n) {
@@ -277,12 +279,13 @@ struct Tail {
       if constexpr (MODE == MODE_BWD) return tgt;
       // d loss / d y up to the constant 2/numel (applied by the finaliser).  lane_w = 1 for lanes inside the frame (1*x - t is
       // exactly x - t) and 0 for the lanes of the last strip that hang over the right edge (their t is 0): no divergent branch
-      const float2 dd = __ffma2_rn(make_float2(lane_w, lane_w), x, make_float2(-tgt.x, -tgt.y));
+      const float2 dd = (kScalarLoss && SC) ? make_float2(fmaf(lane_w, x.x, -tgt.x), fmaf(lane_w, x.y, -tgt.y))
+                                    : __ffma2_rn(make_float2(lane_w, lane_w), x, make_float2(-tgt.x, -tgt.y));
       if constexpr (MODE == MODE_STEP_L1) {      // nn.L1Loss: sum |y - t| ; gradient sign(y - t) (0 at equality), 1/numel later
-        loss = add2(loss, make_float2(fabsf(dd.x), fabsf(dd.y)));
+        acc_add<kScalarLoss && SC>(loss, make_float2(fabsf(dd.x), fabsf(dd.y)));
         return make_float2((dd.x > 0.f ? 1.f : 0.f) - (dd.x < 0.f ? 1.f : 0.f), (dd.y > 0.f ? 1.f : 0.f) - (dd.y < 0.f ? 1.f : 0.f));
       }
-      loss = fma2(dd, dd, loss);
+      acc_fma<kScalarLoss && SC>(loss, dd, dd);
       return dd;
     } else {
       constexpr int OP = E.op[K];
@@ -302,7 +305,7 @@ struct Tail {
 #endif
         const float2 y = gamma_fwd2<IN01, RFORM>(x, gm, l2, c[1], &r);
         const float2 d = Tail<SIG, K + 1, MODE, C>::go(y, tgt, cp, acc, loss, yout, slow, lane_w, tbl);
-        return gamma_bwd2<IN01, NEED_DX, true, NOMASK, RFORM>(x, y, l2, d, gm, a[0], r);
+        return gamma_bwd2<IN01, NEED_DX, true, NOMASK, RFORM, SC>(x, y, l2, d, gm, a[0], r);
       } else if constexpr (OP == RISP_OP_GAIN) {
         const float2 y = mul2s(x, c[C]);
         const float2 d = Tail<SIG, K + 1, MODE, C>::go(y, tgt, cp, acc, loss, yout, slow, lane_w, tbl);
@@ -314,7 +317,7 @@ struct Tail {
         const float2 y = gtm_fwd2<kGtmTable>(x, c, hd, slow, m, tbl + K * kGtmTableBytes);
         float2 d = Tail<SIG, K + 1, MODE, C>::go(y, tgt, cp, acc, loss, yout, slow, lane_w, tbl);
         if (slow) d = mul2(d, m);
-        return gtm_bwd2<NEED_DX>(x, hd, d, c, a);
+        return gtm_bwd2<NEED_DX, SC>(x, hd, d, c, a);
       }
     }
   }
@@ -357,9 +360,16 @@ struct Run {
         phi[6] = x.b; phi[7] = x.g; phi[8] = x.r;
         auto channel = [&](auto ctag, float2 tg, float2& yo) {
           constexpr int C = decltype(ctag)::value;
-          float2 u = fma2ss(c[C * 10], phi[0], c[C * 10 + 9]);
+          float2 u;
+          if constexpr (kScalarPolyFwd) {
+            u = make_float2(fmaf(c[C * 10], phi[0].x, c[C * 10 + 9]), fmaf(c[C * 10], phi[0].y, c[C * 10 + 9]));
 #pragma unroll
-          for (int i = 1; i < 9; ++i) u = fma2s(c[C * 10 + i], phi[i], u);
+            for (int i = 1; i < 9; ++i) u = make_float2(fmaf(c[C * 10 + i], phi[i].x, u.x), fmaf(c[C * 10 + i], phi[i].y, u.y));
+          } else {
+            u = fma2ss(c[C * 10], phi[0], c[C * 10 + 9]);
+#pragma unroll
+            for (int i = 1; i < 9; ++i) u = fma2s(c[C * 10 + i], phi[i], u);
+          }
           const float2 y = sat2(u);
 #ifndef RISP_FUSED_NO_MERGED_MASK
           // a gamma directly behind the polynomial masks its gradient with [y >= eps]; together with the clamp mask
@@ -377,8 +387,8 @@ struct Run {
             e = sel2(u.x == y.x, u.y == y.y, d);     // clamp mask, inclusive: u in [0,1] <=> sat(u) == u
           }
 #pragma unroll
-          for (int i = 0; i < 9; ++i) a[C * 10 + i] = fma2(e, phi[i], a[C * 10 + i]);
-          a[C * 10 + 9] = add2(a[C * 10 + 9], e);
+          for (int i = 0; i < 9; ++i) acc_fma<kFoldS>(a[C * 10 + i], e, phi[i]);
+          acc_add<kFoldS>(a[C * 10 + 9], e);
         };
         channel(std::integral_constant<int, 0>{}, tgt.b, yout.b);
         channel(std::integral_constant<int, 1>{}, tgt.g, yout.g);

@@ -1,9 +1,10 @@
 // Packed-fp32 stage arithmetic of the fused raw -> BGR pipeline kernels (risp_fused.cu).
 //
-// Everything here works on a PAIR of neighbouring pixels held as float2 per channel, so every multiply /
-// add / fma of the chain is one Blackwell packed instruction (FFMA2 / FMUL2 / FADD2: two pixels per issue
-// slot).  Stage parameters are NOT fetched per pixel: a tiny preparation kernel writes the chain's
-// derived coefficients into a __constant__ block once per launch and the kernels read them through the
+// Everything here works on a PAIR of neighbouring pixels held as float2 per channel, so a multiply / add /
+// fma of the chain can be one Blackwell packed instruction (FFMA2 / FMUL2 / FADD2: two pixels per issue
+// slot); the sites where two scalar instructions are cheaper are listed under "cheapest fp32 form per site".
+// Stage parameters are NOT fetched per pixel: a tiny preparation kernel writes the chain's derived
+// coefficients into a __constant__ block once per launch and the kernels read them through the
 // constant bank -> uniform registers (`FFMA2 R, R.F32x2, UR.F32, R`: the scalar is broadcast to both
 // halves by the instruction, so coefficients cost neither vector registers nor splat moves).
 //
@@ -100,6 +101,54 @@ __device__ __forceinline__ float2 sat2(float2 a) { return make_float2(__saturate
 __device__ __forceinline__ float2 sel2(bool px, bool py, float2 a) { return make_float2(px ? a.x : 0.f, py ? a.y : 0.f); }
 __device__ __forceinline__ float2 zero2() { return make_float2(0.f, 0.f); }
 
+// ---- cheapest fp32 form per site of the backward-carrying kernels -------------------------------------------------
+// A packed FFMA2 holds the FMA pipe for two cycles, and with vector register pairs as operands it costs more than the two
+// scalar FFMA it replaces (profiles/r3_fma_rates.txt, cycles per warp instruction: FFMA2 R,R,R 4.3 against FFMA R,R,R 1.6;
+// FFMA2 with a uniform coefficient pair 2.9 against FFMA with a coefficient 0.9-1.1).  So the sites below use scalar
+// instructions in the backward-carrying kernels of chains with the 3x10 polynomial (the FMA-bound ones; template flag SC
+// where a helper also serves other chains); each -DRISP_FUSED_PACKED_* switch restores the packed form of one site
+// (per-site step times on the B200: profiles/r3_ablation.txt -- every site is faster scalar).  The gamma -> tone curve
+// step is memory-bound and keeps the packed forms: with them scalar it took 0.1600 instead of 0.1555 ms per 48 MP.
+//   * folded accumulators: both pixels of a pair go into ONE sum, acc.x = fma(u.y, v.y, fma(u.x, v.x, acc.x)); acc.y stays
+//     the constant 0 (no register), and the epilogue's acc.x + acc.y reduces it unchanged -- the summation order is still
+//     fixed, gradients stay bit-reproducible run to run.  Half the accumulator registers: the 37-parameter step kernel
+//     fits 168 registers, three one-warp CTAs per SM sub-partition instead of two.
+#ifndef RISP_FUSED_PACKED_POLY_FWD
+constexpr bool kScalarPolyFwd = true;    // polynomial rows of the channel-major step: FFMA R,UR,R
+#else
+constexpr bool kScalarPolyFwd = false;
+#endif
+#ifndef RISP_FUSED_PACKED_S_ACC
+constexpr bool kFoldS = true;            // polynomial gradient sums S[c][i] += e_c phi_i
+#else
+constexpr bool kFoldS = false;
+#endif
+#ifndef RISP_FUSED_PACKED_GTM_ACC
+constexpr bool kFoldGtm = true;          // tone-curve hinge sums A_k
+#else
+constexpr bool kFoldGtm = false;
+#endif
+#ifndef RISP_FUSED_PACKED_GAMMA_ACC
+constexpr bool kFoldGamma = true;        // gamma exponent sum
+#else
+constexpr bool kFoldGamma = false;
+#endif
+#ifndef RISP_FUSED_PACKED_LOSS
+constexpr bool kScalarLoss = true;       // loss residual y - t and its sum
+#else
+constexpr bool kScalarLoss = false;
+#endif
+template <bool FOLD>
+__device__ __forceinline__ void acc_fma(float2& acc, float2 u, float2 v) {     // acc += u * v
+  if constexpr (FOLD) acc.x = fmaf(u.y, v.y, fmaf(u.x, v.x, acc.x));
+  else acc = fma2(u, v, acc);
+}
+template <bool FOLD>
+__device__ __forceinline__ void acc_add(float2& acc, float2 u) {               // acc += u
+  if constexpr (FOLD) acc.x = (acc.x + u.x) + u.y;
+  else acc = add2(acc, u);
+}
+
 // ---- stage state kept from the forward sweep for the backward sweep --------------------------------------------
 struct GammaSaved { P2 x, l2, y; };
 struct PolySaved { float2 phi[9]; P2 u, y; };     // phi = b2 g2 r2 bg br gr b g r  (coefficient order of WbQuadratic)
@@ -135,10 +184,10 @@ __device__ __forceinline__ P2 gamma_fwd(const P2& x, float gm, GammaSaved& sv) {
 // d <- dL/dx (WITHOUT the factor gm when DEFER: the caller multiplies the upstream accumulators once at the end);
 // acc += d*y*lg2(xc)  (ln 2 applied in the epilogue).  rcp(x) may be inf/NaN where the mask is 0: selected away.
 // NOMASK: the caller applies the clamp mask itself (merged with the mask of the stage in front), so v is returned as is.
-template <bool IN01, bool NEED_DX, bool DEFER, bool NOMASK = false, bool RFORM = false>
+template <bool IN01, bool NEED_DX, bool DEFER, bool NOMASK = false, bool RFORM = false, bool SC = true>
 __device__ __forceinline__ float2 gamma_bwd2(float2 x, float2 y, float2 l2, float2 d, float gm, float2& acc, float2 r = float2()) {
   const float2 t = mul2(d, y);
-  acc = fma2(t, l2, acc);
+  acc_fma<kFoldGamma && SC>(acc, t, l2);
   if (!NEED_DX) return zero2();
   float2 v = RFORM ? mul2(d, r) : mul2(t, make_float2(rcp_ftz(x.x), rcp_ftz(x.y)));
   if (!DEFER) v = mul2s(v, gm);
@@ -200,8 +249,8 @@ __device__ __forceinline__ P2 poly_bwd(const PolySaved& sv, const P2& d, const f
 #pragma unroll
   for (int c = 0; c < 3; ++c) {
 #pragma unroll
-    for (int i = 0; i < 9; ++i) acc[c * 10 + i] = fma2(e[c], sv.phi[i], acc[c * 10 + i]);
-    acc[c * 10 + 9] = add2(acc[c * 10 + 9], e[c]);
+    for (int i = 0; i < 9; ++i) acc_fma<kFoldS>(acc[c * 10 + i], e[c], sv.phi[i]);
+    acc_add<kFoldS>(acc[c * 10 + 9], e[c]);
   }
   P2 o;
   if (NEED_DX) {
@@ -308,12 +357,12 @@ __device__ __forceinline__ P2 gtm_fwd(const P2& x, const float* c, GtmSaved& sv,
 }
 // accumulates A_0 = sum d x, A_k = sum d max(x - x_k, 0); the knot gradients are the second differences
 // 4 (A_{j-1} - 2 A_j + A_{j+1}) (hat basis = second difference of hinges; A_4 = 0 on [0,1]), formed in the epilogue.
-template <bool NEED_DX>
+template <bool NEED_DX, bool SC = true>
 __device__ __forceinline__ float2 gtm_bwd2(float2 x, const float2 (&sv)[3], float2 d, const float* c, float2* acc) {
-  acc[0] = fma2(d, x, acc[0]);
+  acc_fma<kFoldGtm && SC>(acc[0], d, x);
  if constexpr (kGtmTable) {
 #pragma unroll
-  for (int k = 0; k < 3; ++k) acc[k + 1] = fma2(d, gtm_hinge<true>(x, x, 0.25f * (float)(k + 1)), acc[k + 1]);
+  for (int k = 0; k < 3; ++k) acc_fma<kFoldGtm && SC>(acc[k + 1], d, gtm_hinge<true>(x, x, 0.25f * (float)(k + 1)));
   if (!NEED_DX) return zero2();
   return mul2(d, sv[0]);
  } else {
@@ -322,7 +371,7 @@ __device__ __forceinline__ float2 gtm_bwd2(float2 x, const float2 (&sv)[3], floa
 #pragma unroll
   for (int k = 0; k < 3; ++k) {
     const float2 st = make_float2(hd[k].x >= 0.f ? 1.f : 0.f, hd[k].y >= 0.f ? 1.f : 0.f);
-    acc[k + 1] = fma2(d, gtm_hinge<false>(x, hd[k], 0.f), acc[k + 1]);
+    acc_fma<kFoldGtm && SC>(acc[k + 1], d, gtm_hinge<false>(x, hd[k], 0.f));
     if (NEED_DX) slope = fma2s(c[k + 1], st, slope);
   }
   if (!NEED_DX) return zero2();

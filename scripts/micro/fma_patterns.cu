@@ -1,6 +1,6 @@
 // The two FMA-heavy phases of the fused step kernel as packed (FFMA2) and as scalar (FFMA) code: cycles per pixel pair
-// and scheduler with 4 warps per scheduler.  (a) gradient accumulation acc[c][i] += e_c * phi_i (all vector registers),
-// (b) polynomial forward u_c = sum_i q[c][i] * phi_i with the coefficients in uniform registers.
+// and scheduler with 4 warps per scheduler.  (a) gradient accumulation acc[c][i] += e_c * phi_i (all vector registers):
+// one sum per pixel column (packed or scalar) or both pixels of the pair folded into one sum, (b) polynomial forward u_c = sum_i q[c][i] * phi_i with the coefficients in uniform registers.
 #include <cstdio>
 #include <cuda_runtime.h>
 #define ITERS 4096
@@ -72,6 +72,12 @@ __global__ void __launch_bounds__(512, 1) pat_kernel(Coef cf, float* out, long l
           sacc[2 * (c * 9 + i)] = fmaf(se[2 * c], sphi[2 * i], sacc[2 * (c * 9 + i)]);
           sacc[2 * (c * 9 + i) + 1] = fmaf(se[2 * c + 1], sphi[2 * i + 1], sacc[2 * (c * 9 + i) + 1]);
         }
+    } else if (V == 5) {   // folded accumulate: 54 FFMA per pair into 27 sums, acc = fma(e.y, phi.y, fma(e.x, phi.x, acc))
+#pragma unroll
+      for (int c = 0; c < 3; ++c)
+#pragma unroll
+        for (int i = 0; i < 9; ++i)
+          sacc[c * 9 + i] = fmaf(se[2 * c + 1], sphi[2 * i + 1], fmaf(se[2 * c], sphi[2 * i], sacc[c * 9 + i]));
     }
   }
   const long long t1 = clock64();
@@ -101,6 +107,7 @@ int main() {
   cudaMalloc(&out, 148 * 512 * 4); cudaMalloc(&cyc, 148 * 8);
   run<0>("accumulate 3x9, packed (27 FFMA2 r,r,r)", out, cyc);
   run<1>("accumulate 3x9, scalar (54 FFMA r,r,r)", out, cyc);
+  run<5>("accumulate 3x9, folded (54 FFMA r,r,r, 27 sums)", out, cyc);
   run<4>("accumulate 3x9, 1 channel packed + 2 scalar", out, cyc);
   run<2>("polynomial forward, packed (27 FFMA2 r,u,r)", out, cyc);
   run<3>("polynomial forward, scalar (54 FFMA r,u,r)", out, cyc);

@@ -3,6 +3,7 @@
 #include <cstdio>
 #include <cuda_runtime.h>
 typedef unsigned long long u64;
+__constant__ float c_coef[4] = {1.0001f, 0.9999f, 1.0002f, 0.9998f};
 #define REP 8
 #define ITERS 2048
 template <int V>
@@ -11,6 +12,7 @@ __global__ void __launch_bounds__(1024, 1) rate_kernel(float s, float t, u64* ou
   u64 p[REP], q[REP];
   const float x0 = 1.f + threadIdx.x * 1e-6f;
   const u64 ss = ((u64)__float_as_uint(s) << 32) | __float_as_uint(s);
+  const float su = c_coef[(int)t & 3];
 #pragma unroll
   for (int i = 0; i < REP; ++i) {
     a[i] = x0 + i; b[i] = 0.999f + i * 1e-7f + threadIdx.x * 1e-9f;
@@ -40,6 +42,9 @@ __global__ void __launch_bounds__(1024, 1) rate_kernel(float s, float t, u64* ou
       if (V == 13) { asm volatile("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(p[i]) : "l"(q[i]), "l"(q[(i + 1) % REP]));
                      asm volatile("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(q[i]) : "l"(p[i]), "l"(ss));
                      asm volatile("max.f32 %0, %0, %1;" : "+f"(a[i]) : "f"(b[i])); }
+      // a coefficient from the constant bank: the step kernel reads it as FFMA R,R,UR,R; in this short loop ptxas keeps it in
+      // a vector register instead, read through the operand reuse cache (no register-bank read either way)
+      if (V == 14) a[i] = fmaf(a[i], su, b[i]);
     }
   }
   const long long t1 = clock64();
@@ -66,6 +71,7 @@ int main() {
   cudaMalloc(&out, 148 * 1024 * 8); cudaMalloc(&cyc, 148 * 8);
   run<0>("FFMA  R,R,R", 1, out, cyc);
   run<1>("FFMA  R,imm,R", 1, out, cyc);
+  run<14>("FFMA  R,coefficient (R.reuse),R", 1, out, cyc);
   run<2>("FFMA2 R,R,R", 1, out, cyc);
   run<3>("FFMA2 R,uniform pair,R", 1, out, cyc);
   run<4>("FMUL2 R,R", 1, out, cyc);
