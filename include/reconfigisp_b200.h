@@ -168,6 +168,23 @@ int risp_pipeline_bwd(const float* raw, const float* dy, float* dparams, int N, 
                       risp_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------
+ * Evaluation metric of the reference (test.py, test_split.py: tensor2bgr -> psnr per image).  Both images are quantised as
+ * tensor2bgr does, q(v) = trunc(clip(fl32(v*255), 0, 255)) (NaN -> 0, the codes of risp_to_u8_hwc), and
+ *   sse_out[n] = sum_{c,h,w} (q(y) - q(gt))^2        DEVICE long long[N], exact
+ * PSNR_n = 20 log10(255 / sqrt(sse_n / (C*H*W))) is formed on the host (inf when sse_n == 0).
+ * ------------------------------------------------------------------------------------- */
+/* any fp32 (N,C,H,W) pair, any H and W; one read of each */
+int risp_sse_u8(const float* y, const float* gt, long long* sse_out, int N, int C, int H, int W, risp_stream_t stream);
+/* The same sum for y = risp_pipeline_fwd(raw, ...) without writing y (16 B/px: raw + gt).  Same arguments and the same
+ * dispatch as risp_pipeline_fwd, so the codes are that entry point's codes.  u8_out (nullable, 4-byte aligned) receives the
+ * 8-bit image as (N,H,W,3) BGR bytes, the image test.py writes with cv2.imwrite. */
+size_t risp_pipeline_eval_workspace(int N, int H, int W);
+int risp_pipeline_eval(const float* raw, const float* gt, unsigned char* u8_out, long long* sse_out, int N, int H, int W,
+                       int dm_kind, float dm_clip_hi, const int* ops, const int* param_off, const int* iarg, int S,
+                       const float* params, int param_stride, void* workspace, size_t workspace_bytes,
+                       risp_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------
  * Per-image statistics (grayworld tools_origin.py:35-41, SRCNNRes global features
  * srcnn_res_arch.py:36-40, whiteworld :655-662, conditional-module histogram :120-129).
  * ------------------------------------------------------------------------------------- */

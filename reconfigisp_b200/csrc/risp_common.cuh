@@ -85,6 +85,25 @@ __device__ __forceinline__ float warp_max(float v) {
   return v;
 }
 __device__ __forceinline__ float sat01(float v) { return __saturatef(v); }   // one .SAT instruction (NaN -> 0)
+// 8-bit display code of tensor2bgr (utils/util.py:118-135): trunc(clip(fl32(v*255), 0, 255)), NaN -> 0, the codes of
+// risp_to_u8_hwc.  Same value as fl32(sat(v)*255) (sat first or clip after the rounded product: both give 0 / 255 outside
+// [0,1] and the same product inside), truncated without F2I: adding 2^23 rounding toward zero leaves trunc(x) in the low
+// mantissa bits for 0 <= x < 2^23.  FMUL + FADD.RZ on the FMA pipe instead of a conversion on the quarter-rate XU pipe, which
+// the gamma's lg2 / ex2 already load (the difference of two codes cancels the exponent bits).
+__device__ __forceinline__ int u8_code(float v) {
+  return __float_as_int(__fadd_rz(__fmul_rn(__saturatef(v), 255.f), 8388608.f)) - 0x4B000000;
+}
+// squared code differences of 4 pixels of one channel: <= 4 * 255^2, exact in 32 bits
+__device__ __forceinline__ uint32_t sq_codes4(float4 y, float4 t) {
+  const int d0 = u8_code(y.x) - u8_code(t.x), d1 = u8_code(y.y) - u8_code(t.y);
+  const int d2 = u8_code(y.z) - u8_code(t.z), d3 = u8_code(y.w) - u8_code(t.w);
+  return (uint32_t)(d0 * d0 + d1 * d1 + d2 * d2 + d3 * d3);
+}
+__device__ __forceinline__ unsigned long long warp_sum_u64(unsigned long long v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
 // torch.clamp backward mask is inclusive on both ends
 __device__ __forceinline__ float in01(float v) { return (v >= 0.f && v <= 1.f) ? 1.f : 0.f; }
 #endif
@@ -114,5 +133,9 @@ size_t finalize_rows_workspace(int R, int NS);
 int finalize_rows(const float* partial, void* scratch_ws, float* out, float* loss_out, int R, int B, int NS, int P,
                   const short* dst, const short* slot, int n, float scale, float loss_scale, int loss_slot, bool sum_rows,
                   cudaStream_t st);
+
+// Integer sums of the evaluation kernels: out[r] = sum_b partial[r*B + b] (risp_metric.cu).  Exact, so any order gives the
+// same bits.
+int finalize_sse(const unsigned long long* partial, long long* out, int R, int B, cudaStream_t st);
 
 }  // namespace risp

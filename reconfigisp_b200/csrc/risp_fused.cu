@@ -23,7 +23,8 @@ namespace fused {
 
 __constant__ float g_cpar[kCSlots][kCRows][kCRowFloats];
 
-enum { MODE_FWD = 0, MODE_STEP = 1, MODE_BWD = 2, MODE_STEP_L1 = 3 };   // STEP: MSE loss; STEP_L1: L1 loss (isp_model.py:44-49)
+// STEP: MSE loss; STEP_L1: L1 loss (isp_model.py:44-49); EVAL: inference arithmetic + squared 8-bit code differences to the GT
+enum { MODE_FWD = 0, MODE_STEP = 1, MODE_BWD = 2, MODE_STEP_L1 = 3, MODE_EVAL = 4 };
 constexpr int kWarps = 1;     // one warp per CTA: everything but the lane index is CTA-uniform (uniform datapath, no R2UR)
 constexpr int kStrip = 128;
 
@@ -39,6 +40,8 @@ struct FusedArgs {
   float clip_hi;
   int slot;
   int dbg;              // RISP_FUSED_DEBUG builds: 1 = no stores, 2 = no loads (bandwidth experiments)
+  unsigned char* u8;    // EVAL: (N,H,W,3) 8-bit codes of y, nullable
+  unsigned long long* sse;   // EVAL: [N][cpf*kWarps] sums of squared code differences
 };
 
 // ---- preparation: derived constants of every parameter row ---------------------------------------------------------
@@ -458,7 +461,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
   constexpr EffChain E = Eff<SIG>::e;
   constexpr int HL = (DM == RISP_DM_MALVAR) ? 2 : 1;
   constexpr int WR = 2 * HL + 1, WC = 4 + 2 * HL;
-  constexpr int NACC = (MODE == MODE_FWD || E.nacc == 0) ? 1 : E.nacc;
+  constexpr int NACC = (MODE == MODE_FWD || MODE == MODE_EVAL || E.nacc == 0) ? 1 : E.nacc;
   constexpr int NCST = E.ncst > 0 ? E.ncst : 1;
   static_assert(E.ncst <= kCRowFloats, "the chain's derived constants must fit one row of the constant slot");
   constexpr bool PKDM = E.n > 0 && (E.op[0] == RISP_OP_POLY10 || E.op[0] == FOP_POLYG || E.op[0] == RISP_OP_GAIN);
@@ -489,7 +492,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
 #pragma unroll
     for (int s = 0; s < D; ++s) mbar_init(bars + 8 * s, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    if constexpr (kGtmTable && MODE != MODE_FWD) {
+    if constexpr (kGtmTable && MODE != MODE_FWD && MODE != MODE_EVAL) {
 #pragma unroll
       for (int k = 0; k < E.n; ++k)
         if (E.op[k] == RISP_OP_GTM) gtm_table_fill(tbl + k * kGtmTableBytes, cp + E.coff[k]);
@@ -500,6 +503,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
 
   float2 acc[NACC];
   float2 loss = zero2();
+  unsigned long long sse = 0;     // EVAL: this lane's sum of squared code differences (64 bits: exact for any geometry)
 #pragma unroll
   for (int i = 0; i < NACC; ++i) acc[i] = zero2();
 
@@ -579,9 +583,27 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
         P2 lo, hi;
         demosaic4<DM, HL, 0, ODD, WR, PKDM>(w, a.clip_hi, lo, hi);
         P2 ylo, yhi;
-        if constexpr (MODE == MODE_FWD) {
+        if constexpr (MODE == MODE_EVAL) {
+          // the inference arithmetic (Fwd, not Run): the codes are those of risp_pipeline_fwd's image, byte for byte
           ylo = Fwd<SIG, 0>::go(lo, cp, slow, tbl);
           yhi = Fwd<SIG, 0>::go(hi, cp, slow, tbl);
+          const float4 yB = make_float4(ylo.b.x, ylo.b.y, yhi.b.x, yhi.b.y), yG = make_float4(ylo.g.x, ylo.g.y, yhi.g.x, yhi.g.y),
+                       yR = make_float4(ylo.r.x, ylo.r.y, yhi.r.x, yhi.r.y);
+          // lanes beyond the right edge compute garbage from zero-filled raw (a zero pixel is not zero after the chain): masked
+          if (active) {
+            const uint32_t s = sq_codes4(yB, lds4(gta + lane * 16)) + sq_codes4(yG, lds4(gta + RC::GTPLANEB + lane * 16)) +
+                               sq_codes4(yR, lds4(gta + 2 * RC::GTPLANEB + lane * 16));
+            sse += s;
+            if (a.u8) {      // (H,W,3) BGR bytes of the lane's 4 pixels: 12 contiguous bytes, 4-byte aligned (c0 % 4 == 0)
+              const uint32_t b0 = u8_code(yB.x), b1 = u8_code(yB.y), b2 = u8_code(yB.z), b3 = u8_code(yB.w);
+              const uint32_t g0 = u8_code(yG.x), g1 = u8_code(yG.y), g2 = u8_code(yG.z), g3 = u8_code(yG.w);
+              const uint32_t r0 = u8_code(yR.x), r1 = u8_code(yR.y), r2 = u8_code(yR.z), r3 = u8_code(yR.w);
+              uint32_t* po = reinterpret_cast<uint32_t*>(a.u8 + (((long long)n * H + r) * W + c0) * 3);
+              po[0] = b0 | (g0 << 8) | (r0 << 16) | (b1 << 24);
+              po[1] = g1 | (r1 << 8) | (b2 << 16) | (g2 << 24);
+              po[2] = r2 | (b3 << 8) | (g3 << 16) | (r3 << 24);
+            }
+          }
         } else {
           float4 tg[3];
   #pragma unroll
@@ -592,7 +614,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
           Run<SIG, 0, MODE>::go(lo, tlo, cp, acc, loss, ylo, slow, lane_w, tbl);
           Run<SIG, 0, MODE>::go(hi, thi, cp, acc, loss, yhi, slow, lane_w, tbl);
         }
-        if ((MODE == MODE_FWD || yb) && active) {
+        if (MODE != MODE_EVAL && (MODE == MODE_FWD || yb) && active) {
           float* po = yb + (size_t)r * W + c0;
           st_stream4(po, make_float4(ylo.b.x, ylo.b.y, yhi.b.x, yhi.b.y));
           st_stream4(po + plane, make_float4(ylo.g.x, ylo.g.y, yhi.g.x, yhi.g.y));
@@ -746,7 +768,10 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
     gcount += (unsigned)nrec;
   }
 
-  if constexpr (MODE != MODE_FWD) {
+  if constexpr (MODE == MODE_EVAL) {
+    const unsigned long long tot = warp_sum_u64(sse);
+    if (lane == 0) a.sse[(long long)n * a.cpf + j0] = tot;
+  } else if constexpr (MODE != MODE_FWD) {
     // ---- epilogue: one partial row per warp, slot layout of risp_common.cuh ------------------------------------------
     float tot[NACC];
 #pragma unroll
@@ -917,7 +942,7 @@ template <int MODE>
 static int dispatch(const FusedArgs& a, const ChainDesc& d, unsigned sig, int N, int dm_kind, cudaStream_t st, Geometry* gout) {
 #define RISP_F_SIG(DMK, SG) if (sig == (SG)) return launch_one<DMK, MODE, (SG)>(a, d, N, st, gout);
 #define RISP_F_DM(DMK) RISP_F_SIG(DMK, RISP_SIG_A) RISP_F_SIG(DMK, RISP_SIG_B) RISP_F_SIG(DMK, RISP_SIG_C) RISP_F_SIG(DMK, RISP_SIG_D) \
-  if constexpr (MODE == MODE_FWD) { RISP_F_SIG(DMK, RISP_SIG_SKIP) }
+  if constexpr (MODE == MODE_FWD || MODE == MODE_EVAL) { RISP_F_SIG(DMK, RISP_SIG_SKIP) }
   switch (dm_kind) {
     case RISP_DM_NEAREST: RISP_F_DM(RISP_DM_NEAREST) break;
     case RISP_DM_BILINEAR: RISP_F_DM(RISP_DM_BILINEAR) break;
@@ -947,6 +972,28 @@ int fused_partial_rows_per_frame(int N, int H, int W) {
   int cpf = slots / N < 1 ? 1 : slots / N;
   (void)H; (void)W;
   return cpf * fused::kWarps;
+}
+
+// evaluation mode: inference arithmetic, squared 8-bit code differences to gt -> partial[N][*rows_per_frame], optional 8-bit
+// HWC image.  Returns RISP_OK, an error, or 1 when the chain is not handled.
+int fused_eval_launch(const float* raw, const float* gt, unsigned char* u8, unsigned long long* partial, const float* params,
+                      int pstride, int N, int H, int W, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st,
+                      int* rows_per_frame) {
+  using namespace fused;
+  if (!fused_handles(d, N, pstride, H, W)) return 1;
+  float* cbase = cpar_device_ptr();
+  RISP_REQUIRE(cbase, RISP_E_CUDA, "fused pipeline: cannot resolve the constant parameter block");
+  const int slot = slot_of(st);
+  fused_prep_kernel<<<pstride ? N : 1, 32, 0, st>>>(params, pstride, d, cbase + (size_t)slot * kCRows * kCRowFloats);
+  int rc = check_launch("fused_prep_kernel");
+  if (rc != RISP_OK) return rc;
+  FusedArgs a{raw, gt, nullptr, nullptr, params, pstride, H, W, 0, 0, 0, 0, clip_hi, slot, 0, u8, partial};
+  const unsigned sig = chain_signature(d);
+  Geometry g;
+  rc = dispatch<MODE_EVAL>(a, d, sig, N, dm_kind, st, &g);
+  if (rc != RISP_OK) return rc;
+  *rows_per_frame = g.cpf * kWarps;
+  return dispatch<MODE_EVAL>(a, d, sig, N, dm_kind, st, nullptr);
 }
 
 // mode: 0 forward, 1 MSE step, 2 backward with upstream dy, 3 L1 step.  Returns RISP_OK, an error, or 1 when the chain is not handled.

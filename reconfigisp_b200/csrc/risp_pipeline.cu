@@ -118,13 +118,17 @@ __device__ __forceinline__ void demosaic4(const float (&w)[2 * HL + 1][4 + 2 * H
   }
 }
 
-enum { MODE_FWD = 0, MODE_STEP = 1 };
+// EVAL: the forward of MODE_FWD, then the squared 8-bit code differences to the GT (per-image PSNR numerator); writes no y
+enum { MODE_FWD = 0, MODE_STEP = 1, MODE_EVAL = 2 };
 
 // packed-fp32 / constant-bank kernels for the pre-instantiated signatures (risp_fused.cu)
 bool fused_handles(const ChainDesc& d, int N, int param_stride, int H, int W);
 int fused_partial_rows_per_frame(int N, int H, int W);
 int fused_launch(int mode, const float* raw, const float* gt, float* y, float* partial, const float* params, int pstride,
                  int N, int H, int W, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st, int* rows_per_frame);
+int fused_eval_launch(const float* raw, const float* gt, unsigned char* u8, unsigned long long* partial, const float* params,
+                      int pstride, int N, int H, int W, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st,
+                      int* rows_per_frame);
 
 struct PipeArgs {
   const float* raw;   // (N,1,H,W)
@@ -136,6 +140,8 @@ struct PipeArgs {
   int H, W, rows_per_chunk;
   float clip_hi;
   int gt_is_dy;       // MODE_STEP: `gt` holds dL/dy (container-level backward) instead of the target
+  unsigned char* u8;  // MODE_EVAL: (N,H,W,3) 8-bit codes of y, nullable
+  unsigned long long* sse;   // MODE_EVAL: [N][warps_per_image] sums of squared code differences
 };
 
 #ifndef RISP_STEP_MINB
@@ -147,12 +153,16 @@ struct PipeArgs {
 #ifndef RISP_FWD_MINB
 #define RISP_FWD_MINB 4
 #endif
+#ifndef RISP_EVAL_MINB
+#define RISP_EVAL_MINB 3   // the forward's registers plus the GT row in flight: 4 CTAs (128 registers) spill
+#endif
 #ifndef RISP_FWD_PREFETCH
 #define RISP_FWD_PREFETCH 1   // raw rows in flight per warp in the forward-only kernel.  Measured on B200 (12 MP x 4,
 #endif                        // bilinear + 4 stages): depth 2 = 0.242 ms vs depth 1 = 0.234 ms -- not latency-bound
 
 template <int DM, int MODE, unsigned SIG, bool BIGG>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, (MODE == 1 /*MODE_STEP*/) ? ((SIG == 0) ? 1 : RISP_STEP_MINB) : RISP_FWD_MINB)
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, (MODE == 1 /*MODE_STEP*/) ? ((SIG == 0) ? 1 : RISP_STEP_MINB)
+                                                    : (MODE == 2 /*MODE_EVAL*/) ? RISP_EVAL_MINB : RISP_FWD_MINB)
 pipeline_kernel(PipeArgs a, ChainDesc d) {
   using SG = Sig<SIG>;
   constexpr int SMAX = SG::S;
@@ -171,12 +181,13 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
   const float* __restrict__ img = a.raw + (long long)n * plane;
   const float* __restrict__ prow_inv = a.params + (long long)n * a.pstride;
   const float* __restrict__ prow = prow_inv;
-  const float* __restrict__ gtb = (MODE == MODE_STEP) ? a.gt + (long long)n * 3 * plane : nullptr;
+  const float* __restrict__ gtb = (MODE != MODE_FWD) ? a.gt + (long long)n * 3 * plane : nullptr;
   float* __restrict__ yb = a.y ? a.y + (long long)n * 3 * plane : nullptr;
 
   float accS[SMAX][RISP_SMALL_ACC];
   float2 accB[RISP_BIG_ACC];
   float loss = 0.f;
+  unsigned long long sse = 0;     // MODE_EVAL: this lane's sum of squared code differences
   if (MODE == MODE_STEP) {
 #pragma unroll
     for (int s = 0; s < SMAX; ++s)
@@ -206,6 +217,15 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
     for (int r = ra; r < rb; ++r) {
       row_finish<HL>(w[WR - 1], q, W, c0, active, lane);
       const float4 tB = gB, tG = gG, tR = gR;
+      float4 eB, eG, eR;         // MODE_EVAL: GT of this row
+      if constexpr (MODE == MODE_EVAL) {
+        // requested before the demosaic and the chain it waits behind (a row-ahead prefetch as in MODE_STEP keeps two GT
+        // rows live and spills)
+        if (active) {
+          const long long o = (long long)r * W + c0;
+          eB = ld_stream4(gtb + o); eG = ld_stream4(gtb + plane + o); eR = ld_stream4(gtb + 2 * plane + o);
+        }
+      }
       if (kDeep) {
         q = q2;                                                     // row r+1 (already in flight) becomes current
         if (r + 2 < rb) row_issue<HL>(q2, img, reflect101(r + 2 + HL, H), W, c0, active, lane);
@@ -218,7 +238,25 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
       }
       Px<4> px;
       demosaic4<DM, HL>(w, (r & 1) != 0, a.clip_hi, px);
-      if (MODE == MODE_FWD) {
+      if constexpr (MODE == MODE_EVAL) {
+#pragma unroll
+        for (int s = 0; s < SMAX; ++s)
+          if (SG::live(d, s)) stage_fwd(SG::op(d, s), SG::iarg(d, s), prow + d.off[s], px);
+        if (active) {
+          const float4 yB = make_float4(px.b[0], px.b[1], px.b[2], px.b[3]), yG = make_float4(px.g[0], px.g[1], px.g[2], px.g[3]),
+                       yR = make_float4(px.r[0], px.r[1], px.r[2], px.r[3]);
+          sse += sq_codes4(yB, eB) + sq_codes4(yG, eG) + sq_codes4(yR, eR);
+          if (a.u8) {        // (H,W,3) BGR bytes of the lane's 4 pixels: 12 contiguous bytes, 4-byte aligned (c0 % 4 == 0)
+            uint32_t b[4], g[4], rr[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) { b[k] = u8_code(px.b[k]); g[k] = u8_code(px.g[k]); rr[k] = u8_code(px.r[k]); }
+            uint32_t* po = reinterpret_cast<uint32_t*>(a.u8 + (((long long)n * H + r) * W + c0) * 3);
+            po[0] = b[0] | (g[0] << 8) | (rr[0] << 16) | (b[1] << 24);
+            po[1] = g[1] | (rr[1] << 8) | (b[2] << 16) | (g[2] << 24);
+            po[2] = rr[2] | (b[3] << 8) | (g[3] << 16) | (rr[3] << 24);
+          }
+        }
+      } else if (MODE == MODE_FWD) {
 #pragma unroll
         for (int s = 0; s < SMAX; ++s)
           if (SG::live(d, s)) stage_fwd(SG::op(d, s), SG::iarg(d, s), prow + d.off[s], px);
@@ -305,6 +343,12 @@ constexpr int kPairUnroll = RISP_PAIR_UNROLL;
     float v = warp_sum(loss);
     if (lane == 0) { out[RISP_SLOT_LOSS] = v; out[RISP_SLOT_LOSS + 1] = 0.f; }
   }
+  if constexpr (MODE == MODE_EVAL) {    // every warp writes its row, also one whose strip lies outside the frame
+    const int warps_per_image = gridDim.y * gridDim.x * kWarpsPerBlock;
+    const int widx = (blockIdx.y * gridDim.x + blockIdx.x) * kWarpsPerBlock + wid;
+    const unsigned long long v = warp_sum_u64(sse);
+    if (lane == 0) a.sse[(long long)n * warps_per_image + widx] = v;
+  }
 }
 
 struct PipeGeom { int strips_x, chunks, rows_per_chunk, warps_per_image; };
@@ -336,16 +380,20 @@ static int launch_pipeline(const PipeArgs& a, const ChainDesc& d, int N, int dm_
   dim3 grid(g.strips_x, g.chunks, N), block(kWarpsPerBlock * 32);
   const unsigned sig = chain_signature(d);
   bool done = false;
+  // the evaluation mode has the generic instantiation only: the same stage_fwd arithmetic, 3 kernels instead of 15
 #define RISP_PIPE_SIG(DMK, SG)                                                       \
-  if (!done && sig == (SG)) {                                                        \
-    pipeline_kernel<DMK, MODE, (SG), false><<<grid, block, 0, st>>>(b, d);           \
-    done = true;                                                                     \
+  if constexpr (MODE != MODE_EVAL) {                                                 \
+    if (!done && sig == (SG)) {                                                      \
+      pipeline_kernel<DMK, MODE, (SG), false><<<grid, block, 0, st>>>(b, d);         \
+      done = true;                                                                   \
+    }                                                                                \
   }
 #define RISP_PIPE(DMK)                                                               \
   do {                                                                               \
     RISP_PIPE_SIG(DMK, RISP_SIG_A) RISP_PIPE_SIG(DMK, RISP_SIG_B) RISP_PIPE_SIG(DMK, RISP_SIG_C) RISP_PIPE_SIG(DMK, RISP_SIG_D) \
     if (!done) {                                                                     \
-      if (big) pipeline_kernel<DMK, MODE, 0u, true><<<grid, block, 0, st>>>(b, d);   \
+      if constexpr (MODE == MODE_EVAL) pipeline_kernel<DMK, MODE, 0u, false><<<grid, block, 0, st>>>(b, d); \
+      else if (big) pipeline_kernel<DMK, MODE, 0u, true><<<grid, block, 0, st>>>(b, d); \
       else pipeline_kernel<DMK, MODE, 0u, false><<<grid, block, 0, st>>>(b, d);      \
     }                                                                                \
   } while (0)
@@ -404,6 +452,57 @@ extern "C" int risp_pipeline_fwd(const float* raw, float* y, int N, int H, int W
 extern "C" int risp_demosaic_fwd(const float* raw, float* bgr, int N, int H, int W, int kind, float clip_hi,
                                  risp_stream_t stream) {
   return risp_pipeline_fwd(raw, bgr, N, H, W, kind, clip_hi, nullptr, nullptr, nullptr, 0, nullptr, 0, stream);
+}
+
+extern "C" size_t risp_pipeline_eval_workspace(int N, int H, int W) {
+  if (N <= 0 || H <= 0 || W <= 0) return 0;
+  size_t rows = (size_t)pipe_geometry(N, H, W).warps_per_image;
+  const size_t frows = (size_t)fused_partial_rows_per_frame(N, H, W);
+  if (frows > rows) rows = frows;
+  return (size_t)N * rows * sizeof(unsigned long long);
+}
+
+// Per-image sum of squared 8-bit code differences between the pipeline's output and gt, without writing the image: the same
+// dispatch as risp_pipeline_fwd (packed kernel when it takes the chain, else the interpreter), so the codes are that entry
+// point's codes under either setting of RISP_FUSED.
+extern "C" int risp_pipeline_eval(const float* raw, const float* gt, unsigned char* u8_out, long long* sse_out, int N, int H,
+                                  int W, int dm_kind, float dm_clip_hi, const int* ops, const int* param_off, const int* iarg,
+                                  int S, const float* params, int param_stride, void* workspace, size_t workspace_bytes,
+                                  risp_stream_t stream) {
+  const char* who = "risp_pipeline_eval";
+  int rc = check_frame(who, raw, N, H, W);
+  if (rc != RISP_OK) return rc;
+  RISP_REQUIRE(gt && sse_out, RISP_E_INVALID, "%s: gt and sse_out must be non-null", who);
+  RISP_REQUIRE(aligned16(gt), RISP_E_ALIGN, "%s: gt must be 16-byte aligned", who);
+  RISP_REQUIRE((reinterpret_cast<uintptr_t>(sse_out) & 7u) == 0, RISP_E_ALIGN, "%s: sse_out must be 8-byte aligned", who);
+  RISP_REQUIRE((reinterpret_cast<uintptr_t>(u8_out) & 3u) == 0, RISP_E_ALIGN, "%s: u8_out must be 4-byte aligned", who);
+  RISP_REQUIRE(dm_kind == RISP_DM_NEAREST || dm_kind == RISP_DM_BILINEAR || dm_kind == RISP_DM_MALVAR, RISP_E_INVALID,
+               "%s: unknown demosaic kind %d", who, dm_kind);
+  ChainDesc d;
+  int P = 0;
+  rc = make_chain(&d, ops, param_off, iarg, S, &P);
+  if (rc != RISP_OK) return rc;
+  RISP_REQUIRE(P == 0 || params, RISP_E_INVALID, "%s: chain needs %d parameters but params is null", who, P);
+  RISP_REQUIRE(param_stride == 0 || param_stride >= P, RISP_E_INVALID, "%s: param_stride %d < %d", who, param_stride, P);
+  RISP_REQUIRE(workspace, RISP_E_INVALID, "%s: workspace is null", who);
+  const size_t need = risp_pipeline_eval_workspace(N, H, W);
+  RISP_REQUIRE(workspace_bytes >= need, RISP_E_WORKSPACE, "%s: workspace %zu < %zu", who, workspace_bytes, need);
+  cudaStream_t st = as_stream(stream);
+  unsigned long long* partial = static_cast<unsigned long long*>(workspace);
+  int rows = 0;
+  rc = 1;
+  if (use_fused()) {
+    ChainDesc df = d;
+    if (S == 0) { df.S = 1; df.op[0] = RISP_OP_SKIP; df.off[0] = 0; df.iarg[0] = 0; }     // demosaic only
+    rc = fused_eval_launch(raw, gt, u8_out, partial, params, param_stride, N, H, W, dm_kind, dm_clip_hi, df, st, &rows);
+  }
+  if (rc == 1) {
+    PipeArgs a{raw, gt, nullptr, nullptr, params, param_stride, H, W, 0, dm_clip_hi, 0, u8_out, partial};
+    rc = launch_pipeline<MODE_EVAL>(a, d, N, dm_kind, false, st);
+    rows = pipe_geometry(N, H, W).warps_per_image;
+  }
+  if (rc != RISP_OK) return rc;
+  return finalize_sse(partial, sse_out, N, rows, st);
 }
 
 extern "C" size_t risp_pipeline_step_workspace(int N, int H, int W, int P) {

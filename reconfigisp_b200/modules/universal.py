@@ -189,11 +189,12 @@ class _Universal(nn.Module):
                 cols.append(kp.reshape(1, -1))
         return torch.cat(cols, dim=1) if cols else None
 
-    def _run_fused(self, x):
+    def _run_fused(self, x, stop=None):
+        """The planned segments [0, stop) (all of them by default)."""
         if self._plan is None:
             self._plan = self._make_plan()
         N = x.size(0)
-        for kind, idx, keep, chain in self._plan:
+        for kind, idx, keep, chain in self._plan[:stop]:
             if kind == 'module':
                 x = self.all_modules[idx](x, self._stage_params(idx, N))
             elif kind == 'chain':
@@ -220,6 +221,33 @@ class _Universal(nn.Module):
     @property
     def trainable_parameters(self):
         return self.all_params
+
+    # -- evaluation (test.py: tensor2bgr -> psnr per image) ----------------------------------------------------
+    def evaluate(self, x, gt, u8=False):
+        """Score the pipeline's output on x against gt the way the reference's test scripts do -> (sse, u8_or_None):
+        sse = int64 (N,) sums of squared 8-bit code differences on the device (`metrics.psnr_from_sse(sse, 3*H*W)` gives
+        the per-image PSNR), u8 = the (N,H,W,3) 8-bit output images when asked for.  When the last segment of the plan is a
+        fused head on a frame with even H and W % 4 == 0, that segment runs in the pipeline kernels' evaluation mode and
+        its image is never written; otherwise the forward runs and `ops.sse_u8` scores it.  Runs under no_grad; parameters
+        and `intermediate_results` are left as they are."""
+        with torch.no_grad():
+            if self.fuse:
+                if self._plan is None:
+                    self._plan = self._make_plan()
+                last = len(self._plan)
+                while last > 0 and self._plan[last - 1][0] == 'chain' and not self._plan[last - 1][2]:
+                    last -= 1                                   # trailing skip-only segments change nothing
+                if last > 0 and self._plan[last - 1][0] == 'head':
+                    _, idx, keep, chain = self._plan[last - 1]
+                    h = self._run_fused(x, last - 1)
+                    if h.shape[2] % 2 == 0 and h.shape[3] % 4 == 0:
+                        return ops.pipeline_eval(h, gt, self.all_modules[idx].demosaic_kind, chain,
+                                                 self._segment_table(keep, x.size(0)), u8=u8)
+                y = self._run_fused(x)
+            else:
+                y = self._run_sequential(x)[0]
+            sse = ops.sse_u8(y, gt)
+            return sse, (torch.stack([ops.to_u8_hwc(y[n]) for n in range(y.shape[0])]) if u8 else None)
 
     # -- the whole proxy-tuning step in one pass (isp_model.py:128-142) ----------------------------------------
     def fused_mse_step_plan(self):

@@ -613,6 +613,41 @@ def pipeline_fwd(raw, dm_kind, chain, params=None, clip_hi=1.0):
     return y
 
 
+def sse_u8(y, gt):
+    """Per-image sum of squared differences of the 8-bit codes tensor2bgr makes of y and gt (utils/util.py:118-135:
+    trunc(clip(x*255, 0, 255))) -> int64 (N,) CUDA tensor, exact.  y, gt: fp32 (N,C,H,W) or (C,H,W), any H and W.
+    Nothing waits for the device: `metrics.psnr_from_sse` turns the sums into PSNR."""
+    y, gt = y.detach(), gt.detach()
+    if y.dim() == 3:
+        y, gt = y.unsqueeze(0), gt.unsqueeze(0)
+    y, gt = _img(y), _img(gt)
+    if y.shape != gt.shape:
+        raise ValueError('sse_u8: shapes differ, %s and %s' % (tuple(y.shape), tuple(gt.shape)))
+    N, C, H, W = y.shape
+    sse = torch.zeros((N,), device=y.device, dtype=torch.int64)
+    if y.numel() == 0:
+        return sse
+    L.call('risp_sse_u8', L.ptr(y), L.ptr(gt), L.ptr(sse), N, C, H, W, L.stream())
+    return sse
+
+
+def pipeline_eval(raw, gt, dm_kind, chain, params=None, clip_hi=1.0, u8=False):
+    """Evaluate the fused pipeline against gt without writing its image: -> (sse, u8_or_None).  sse is `sse_u8` of
+    `pipeline_fwd(raw, dm_kind, chain, params, clip_hi)` and gt, int64 (N,); with u8=True the 8-bit image of the output
+    comes along as (N,H,W,3) BGR uint8 (`to_u8_hwc` of each image).  16 B/px: raw and gt are read once."""
+    raw, gt = _img(raw.detach(), 1), _img(gt.detach(), 3)
+    N, _, H, W = raw.shape
+    if gt.shape != (N, 3, H, W):
+        raise ValueError('pipeline_eval: gt must be (%d,3,%d,%d), got %s' % (N, H, W, tuple(gt.shape)))
+    tab, stride = _param_table(params.detach(), N, chain.P) if chain.P else (None, 0)
+    sse = torch.empty((N,), device=raw.device, dtype=torch.int64)
+    out8 = torch.empty((N, H, W, 3), device=raw.device, dtype=torch.uint8) if u8 else None
+    ws = L.workspace(L.size('risp_pipeline_eval_workspace', N, H, W), raw.device)
+    L.call('risp_pipeline_eval', L.ptr(raw), L.ptr(gt), L.ptr(out8), L.ptr(sse), N, H, W, DM[dm_kind], float(clip_hi),
+           *chain.desc(), L.ptr(tab), stride, L.ptr(ws), ws.numel() * 4, L.stream())
+    return sse, out8
+
+
 class PipelineStep:
     """Pre-allocated state for repeated proxy-tuning steps on frames of one geometry."""
 
