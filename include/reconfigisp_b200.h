@@ -184,6 +184,19 @@ int risp_pipeline_eval(const float* raw, const float* gt, unsigned char* u8_out,
                        const float* params, int param_stride, void* workspace, size_t workspace_bytes,
                        risp_stream_t stream);
 
+/* Per-image SSIM of the same 8-bit codes (skimage 0.16 compare_ssim(a, b, multichannel=True) with its defaults: uniform 7x7
+ * window, sample covariance, K1 = 0.01, K2 = 0.03, data_range 255, a border of 3 pixels cropped).  For every channel and
+ * interior pixel (h in [3, H-3), w in [3, W-3)) the 7x7 integer sums Sa, Sb, Saa, Sbb, Sab of the codes give
+ *   P1 = 2 Sa Sb, Q1 = Sa^2 + Sb^2, P2 = 2 (49 Sab - Sa Sb), Q2 = 49 (Saa + Sbb) - Sa^2 - Sb^2     exact in int32
+ *   S  = (P1 + c1)(P2 + c2) / ((Q1 + c1)(Q2 + c2)),  c1 = 49^2 (0.01*255)^2,  c2 = 49*48 (0.03*255)^2    fp32, rounded
+ *   ssim_sum_out[n] = sum_{c,h,w} rint(S * 2^32)         DEVICE long long[N], exact: the same bits on any grid
+ * SSIM_n = ssim_sum_out[n] / (2^32 C (H-6)(W-6)) is formed on the host.  Identical images give exactly 1 per pixel, and
+ * swapping the operands gives the same bits.  y is fp32 (N,C,H,W) or the 8-bit (N,H,W,C) image of risp_to_u8_hwc /
+ * risp_pipeline_eval; gt is fp32 (N,C,H,W).  H, W >= 7 and C (H-6)(W-6) < 2^31.  One read of each operand. */
+enum risp_image_layout { RISP_IMG_F32_NCHW = 0, RISP_IMG_U8_NHWC = 1 };
+int risp_ssim_u8(const void* y, int y_layout, const float* gt, long long* ssim_sum_out, int N, int C, int H, int W,
+                 risp_stream_t stream);
+
 /* ---------------------------------------------------------------------------------------
  * Per-image statistics (grayworld tools_origin.py:35-41, SRCNNRes global features
  * srcnn_res_arch.py:36-40, whiteworld :655-662, conditional-module histogram :120-129).

@@ -222,14 +222,17 @@ class _Universal(nn.Module):
     def trainable_parameters(self):
         return self.all_params
 
-    # -- evaluation (test.py: tensor2bgr -> psnr per image) ----------------------------------------------------
-    def evaluate(self, x, gt, u8=False):
+    # -- evaluation (test.py: tensor2bgr -> psnr per image; get_ssim) ------------------------------------------
+    def evaluate(self, x, gt, u8=False, ssim=False):
         """Score the pipeline's output on x against gt the way the reference's test scripts do -> (sse, u8_or_None):
         sse = int64 (N,) sums of squared 8-bit code differences on the device (`metrics.psnr_from_sse(sse, 3*H*W)` gives
         the per-image PSNR), u8 = the (N,H,W,3) 8-bit output images when asked for.  When the last segment of the plan is a
         fused head on a frame with even H and W % 4 == 0, that segment runs in the pipeline kernels' evaluation mode and
         its image is never written; otherwise the forward runs and `ops.sse_u8` scores it.  Runs under no_grad; parameters
-        and `intermediate_results` are left as they are."""
+        and `intermediate_results` are left as they are.
+        With ssim=True -> (sse, u8_or_None, ssim_sums): ssim_sums = `ops.ssim_u8` of the output and gt, int64 (N,)
+        (`metrics.ssim_from_sums(ssim_sums, 3, H, W)` gives the per-image SSIM).  On the fused-head path SSIM is computed
+        from the evaluation mode's 8-bit image, which is dropped afterwards unless u8 was asked for."""
         with torch.no_grad():
             if self.fuse:
                 if self._plan is None:
@@ -241,13 +244,17 @@ class _Universal(nn.Module):
                     _, idx, keep, chain = self._plan[last - 1]
                     h = self._run_fused(x, last - 1)
                     if h.shape[2] % 2 == 0 and h.shape[3] % 4 == 0:
-                        return ops.pipeline_eval(h, gt, self.all_modules[idx].demosaic_kind, chain,
-                                                 self._segment_table(keep, x.size(0)), u8=u8)
+                        sse, img = ops.pipeline_eval(h, gt, self.all_modules[idx].demosaic_kind, chain,
+                                                     self._segment_table(keep, x.size(0)), u8=u8 or ssim)
+                        if not ssim:
+                            return sse, img
+                        return sse, (img if u8 else None), ops.ssim_u8(img, gt)
                 y = self._run_fused(x)
             else:
                 y = self._run_sequential(x)[0]
             sse = ops.sse_u8(y, gt)
-            return sse, (torch.stack([ops.to_u8_hwc(y[n]) for n in range(y.shape[0])]) if u8 else None)
+            img = torch.stack([ops.to_u8_hwc(y[n]) for n in range(y.shape[0])]) if u8 else None
+            return (sse, img, ops.ssim_u8(y, gt)) if ssim else (sse, img)
 
     # -- the whole proxy-tuning step in one pass (isp_model.py:128-142) ----------------------------------------
     def fused_mse_step_plan(self):

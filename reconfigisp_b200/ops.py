@@ -631,6 +631,38 @@ def sse_u8(y, gt):
     return sse
 
 
+def ssim_u8(y, gt):
+    """Per-image SSIM of the 8-bit images of y and gt (skimage `compare_ssim(a, b, multichannel=True)` on the tensor2bgr
+    codes: uniform 7x7 window, border of 3 cropped) as exact int64 (N,) CUDA sums of rint(S * 2^32) over the C (H-6)(W-6)
+    interior values; `metrics.ssim_from_sums` turns them into SSIM.  Nothing waits for the device.
+    y: fp32 (N,C,H,W) / (C,H,W), or the uint8 (N,H,W,C) / (H,W,C) image of `to_u8_hwc`, `pipeline_eval(u8=True)` or
+    `patch2whole_u8`; gt: fp32 (N,C,H,W) / (C,H,W).  H and W must be at least 7."""
+    y, gt = y.detach(), gt.detach()
+    if gt.dim() == 3:
+        gt = gt.unsqueeze(0)
+    if y.dim() == 3:
+        y = y.unsqueeze(0)
+    gt = _img(gt)
+    N, C, H, W = gt.shape
+    if y.dtype == torch.uint8:
+        if not y.is_cuda:
+            raise RuntimeError('reconfigisp_b200 ops run on CUDA tensors only (no CPU fallback); got a %s tensor' % y.device)
+        if tuple(y.shape) != (N, H, W, C):
+            raise ValueError('ssim_u8: the 8-bit y must be (N,H,W,C) = %s, got %s' % ((N, H, W, C), tuple(y.shape)))
+        y, layout = y.contiguous(), L.ENUMS['RISP_IMG_U8_NHWC']
+    else:
+        y, layout = _img(y), L.ENUMS['RISP_IMG_F32_NCHW']
+        if y.shape != gt.shape:
+            raise ValueError('ssim_u8: shapes differ, %s and %s' % (tuple(y.shape), tuple(gt.shape)))
+    if H < 7 or W < 7:
+        raise ValueError('ssim_u8: the 7x7 window needs H and W >= 7, got %d x %d' % (H, W))
+    out = torch.empty((N,), device=gt.device, dtype=torch.int64)
+    if N == 0:
+        return out
+    L.call('risp_ssim_u8', L.ptr(y), layout, L.ptr(gt), L.ptr(out), N, C, H, W, L.stream())
+    return out
+
+
 def pipeline_eval(raw, gt, dm_kind, chain, params=None, clip_hi=1.0, u8=False):
     """Evaluate the fused pipeline against gt without writing its image: -> (sse, u8_or_None).  sse is `sse_u8` of
     `pipeline_fwd(raw, dm_kind, chain, params, clip_hi)` and gt, int64 (N,); with u8=True the 8-bit image of the output

@@ -309,13 +309,14 @@ class IspModel:
         self._output = self.netG(self.img)
         return self._output, self.netG.intermediate_results
 
-    def evaluate(self, u8=False):
-        """Score the fed batch like the reference's test script (tensor2bgr -> psnr per image) -> (sse, u8_or_None), see
-        `_Universal.evaluate`; `metrics.psnr_from_sse(sse, 3*H*W)` gives the PSNR.  Reads the batch like a step does (waits
-        for its copy, marks it used for the double-buffered feed) and leaves the optimizer, the gradients and the captured
-        step graphs alone."""
+    def evaluate(self, u8=False, ssim=False):
+        """Score the fed batch like the reference's test script (tensor2bgr -> psnr per image) -> (sse, u8_or_None), or with
+        ssim=True (sse, u8_or_None, ssim_sums), see `_Universal.evaluate`; `metrics.psnr_from_sse(sse, 3*H*W)` gives the
+        PSNR and `metrics.ssim_from_sums(ssim_sums, 3, H, W)` the SSIM.  Reads the batch like a step does (waits for its
+        copy, marks it used for the double-buffered feed) and leaves the optimizer, the gradients and the captured step
+        graphs alone."""
         self._sync_feed()
-        res = self.netG.evaluate(self.img, self.gt, u8=u8)
+        res = self.netG.evaluate(self.img, self.gt, u8=u8, ssim=ssim)
         self._mark_used()
         return res
 
