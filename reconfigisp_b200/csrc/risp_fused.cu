@@ -15,6 +15,8 @@
 #include "risp_fused.cuh"
 
 #include <cuda.h>
+#include <array>
+#include <map>
 #include <mutex>
 #include <stdlib.h>
 
@@ -42,6 +44,9 @@ struct FusedArgs {
   int dbg;              // RISP_FUSED_DEBUG builds: 1 = no stores, 2 = no loads (bandwidth experiments)
   unsigned char* u8;    // EVAL: (N,H,W,3) 8-bit codes of y, nullable
   unsigned long long* sse;   // EVAL: [N][cpf*kWarps] sums of squared code differences
+  // narrow items (backward-carrying kernels): the last strip of a frame, nw = 32 or 64 columns wide (0: none), marched by
+  // 128/nw lane groups on as many row pairs at once; the strip_blocks full strips lie to its left
+  int nw, nrows_per_chunk, nchunks;
 };
 
 // ---- preparation: derived constants of every parameter row ---------------------------------------------------------
@@ -455,9 +460,12 @@ __device__ __forceinline__ bool chain_slow(const float* __restrict__ cp) {
 #define RISP_FUSED_FWD_MAXROWS 256
 #endif
 
-template <int DM, int MODE, unsigned SIG>
+// NARROW: the kernel also runs narrow items (a.nw != 0); a separate instantiation, so that the kernels of frames without
+// them keep their register allocation
+template <int DM, int MODE, unsigned SIG, bool NARROW>
 __global__ void __launch_bounds__(kWarps * 32, (MODE == MODE_FWD) ? RISP_FUSED_FWD_MINB : RISP_FUSED_STEP_MINB)
-fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_raw, const __grid_constant__ CUtensorMap tm_gt) {
+fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_raw, const __grid_constant__ CUtensorMap tm_gt,
+             const __grid_constant__ CUtensorMap tm_rawn, const __grid_constant__ CUtensorMap tm_gtn) {
   constexpr EffChain E = Eff<SIG>::e;
   constexpr int HL = (DM == RISP_DM_MALVAR) ? 2 : 1;
   constexpr int WR = 2 * HL + 1, WC = 4 + 2 * HL;
@@ -506,6 +514,83 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
   unsigned long long sse = 0;     // EVAL: this lane's sum of squared code differences (64 bits: exact for any geometry)
 #pragma unroll
   for (int i = 0; i < NACC; ++i) acc[i] = zero2();
+
+  // where a lane's 4 pixels sit in the records of the current item (backward-carrying kernels)
+  struct LanePos {
+    uint32_t own, oL0, oL1, oR0, oR1;   // raw-row byte offsets: own columns; halo columns c0-HL, c0-1, c0+4, c0+5
+    uint32_t gt;                        // GT-row byte offset of the own columns
+    int c0;                             // first column
+    int dr;                             // row of the lane's pixels relative to the row the warp computes
+    bool active;                        // a pixel of this item: inside the frame and the item's rows
+    float lane_w;                       // active ? 1 : 0
+  };
+  // ---- backward-carrying kernels (issue-bound): a private window per row read with plain LDS ----
+  // one row: read the window (wa(j): shared-memory address of its raw row j) and the GT row, demosaic, chain, store.
+  // NARROW: the lane's row may belong to another item while its GT is real data: such a lane's target is zeroed so that it
+  // adds exactly nothing.
+  auto do_row = [&](auto odd_tag, auto slow_tag, auto narrow_tag, int r, auto wa, uint32_t gta, const LanePos& L) {
+    constexpr bool ODD = decltype(odd_tag)::value;
+    constexpr bool slow = decltype(slow_tag)::value;     // shadows the run-time flag: the chain's branches on it fold away
+    constexpr bool NARROW = decltype(narrow_tag)::value;
+    float w[WR][WC];
+#pragma unroll
+    for (int j = 0; j < WR; ++j) {
+      const uint32_t rj = wa(j);
+      const float4 v = lds4(rj + L.own);
+      if constexpr (HL == 1) {
+        w[j][0] = lds1(rj + L.oL0); w[j][1] = v.x; w[j][2] = v.y; w[j][3] = v.z; w[j][4] = v.w; w[j][5] = lds1(rj + L.oR0);
+      } else {
+        w[j][0] = lds1(rj + L.oL0); w[j][1] = lds1(rj + L.oL1);
+        w[j][2] = v.x; w[j][3] = v.y; w[j][4] = v.z; w[j][5] = v.w;
+        w[j][6] = lds1(rj + L.oR0); w[j][7] = lds1(rj + L.oR1);
+      }
+    }
+    P2 lo, hi;
+    demosaic4<DM, HL, 0, ODD, WR, PKDM>(w, a.clip_hi, lo, hi);
+    P2 ylo, yhi;
+    if constexpr (MODE == MODE_EVAL) {
+      // the inference arithmetic (Fwd, not Run): the codes are those of risp_pipeline_fwd's image, byte for byte
+      ylo = Fwd<SIG, 0>::go(lo, cp, slow, tbl);
+      yhi = Fwd<SIG, 0>::go(hi, cp, slow, tbl);
+      const float4 yB = make_float4(ylo.b.x, ylo.b.y, yhi.b.x, yhi.b.y), yG = make_float4(ylo.g.x, ylo.g.y, yhi.g.x, yhi.g.y),
+                   yR = make_float4(ylo.r.x, ylo.r.y, yhi.r.x, yhi.r.y);
+      // lanes beyond the right edge compute garbage from zero-filled raw (a zero pixel is not zero after the chain): masked
+      if (L.active) {
+        const uint32_t s = sq_codes4(yB, lds4(gta + L.gt)) + sq_codes4(yG, lds4(gta + RC::GTPLANEB + L.gt)) +
+                           sq_codes4(yR, lds4(gta + 2 * RC::GTPLANEB + L.gt));
+        sse += s;
+        if (a.u8) {      // (H,W,3) BGR bytes of the lane's 4 pixels: 12 contiguous bytes, 4-byte aligned (c0 % 4 == 0)
+          const uint32_t b0 = u8_code(yB.x), b1 = u8_code(yB.y), b2 = u8_code(yB.z), b3 = u8_code(yB.w);
+          const uint32_t g0 = u8_code(yG.x), g1 = u8_code(yG.y), g2 = u8_code(yG.z), g3 = u8_code(yG.w);
+          const uint32_t r0 = u8_code(yR.x), r1 = u8_code(yR.y), r2 = u8_code(yR.z), r3 = u8_code(yR.w);
+          uint32_t* po = reinterpret_cast<uint32_t*>(a.u8 + (((long long)n * H + r + L.dr) * W + L.c0) * 3);
+          po[0] = b0 | (g0 << 8) | (r0 << 16) | (b1 << 24);
+          po[1] = g1 | (r1 << 8) | (b2 << 16) | (g2 << 24);
+          po[2] = r2 | (b3 << 8) | (g3 << 16) | (r3 << 24);
+        }
+      }
+    } else {
+      float4 tg[3];
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        tg[c] = lds4(gta + c * RC::GTPLANEB + L.gt);
+        if constexpr (NARROW) {
+          if (!L.active) tg[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+      }
+      P2 tlo, thi;
+      tlo.b = make_float2(tg[0].x, tg[0].y); tlo.g = make_float2(tg[1].x, tg[1].y); tlo.r = make_float2(tg[2].x, tg[2].y);
+      thi.b = make_float2(tg[0].z, tg[0].w); thi.g = make_float2(tg[1].z, tg[1].w); thi.r = make_float2(tg[2].z, tg[2].w);
+      Run<SIG, 0, MODE>::go(lo, tlo, cp, acc, loss, ylo, slow, L.lane_w, tbl);
+      Run<SIG, 0, MODE>::go(hi, thi, cp, acc, loss, yhi, slow, L.lane_w, tbl);
+    }
+    if (MODE != MODE_EVAL && yb && L.active) {
+      float* po = yb + (size_t)(r + L.dr) * W + L.c0;
+      st_stream4(po, make_float4(ylo.b.x, ylo.b.y, yhi.b.x, yhi.b.y));
+      st_stream4(po + plane, make_float4(ylo.g.x, ylo.g.y, yhi.g.x, yhi.g.y));
+      st_stream4(po + 2 * plane, make_float4(ylo.r.x, ylo.r.y, yhi.r.x, yhi.r.y));
+    }
+  };
 
   const int items = a.chunks * a.strip_blocks;
   for (int item = j0; item < items; item += a.cpf) {
@@ -563,64 +648,8 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
     const uint32_t oR1 = own + (last ? 4 : 20);                          // column c0+5    (reflect: W+1 -> W-3)
 
     if constexpr (MODE != MODE_FWD) {
-      // ---- backward-carrying kernels (issue-bound): 2-row records, a private window per row read with plain LDS ----
-      // one row: read the window and the GT row, demosaic, chain, store
-      auto do_row = [&](auto odd_tag, auto slow_tag, int r, const uint32_t* wa, uint32_t gta) {
-        constexpr bool ODD = decltype(odd_tag)::value;
-        constexpr bool slow = decltype(slow_tag)::value;     // shadows the run-time flag: the chain's branches on it fold away
-        float w[WR][WC];
-  #pragma unroll
-        for (int j = 0; j < WR; ++j) {
-          const float4 v = lds4(wa[j] + own);
-          if constexpr (HL == 1) {
-            w[j][0] = lds1(wa[j] + oL0); w[j][1] = v.x; w[j][2] = v.y; w[j][3] = v.z; w[j][4] = v.w; w[j][5] = lds1(wa[j] + oR0);
-          } else {
-            w[j][0] = lds1(wa[j] + oL0); w[j][1] = lds1(wa[j] + oL1);
-            w[j][2] = v.x; w[j][3] = v.y; w[j][4] = v.z; w[j][5] = v.w;
-            w[j][6] = lds1(wa[j] + oR0); w[j][7] = lds1(wa[j] + oR1);
-          }
-        }
-        P2 lo, hi;
-        demosaic4<DM, HL, 0, ODD, WR, PKDM>(w, a.clip_hi, lo, hi);
-        P2 ylo, yhi;
-        if constexpr (MODE == MODE_EVAL) {
-          // the inference arithmetic (Fwd, not Run): the codes are those of risp_pipeline_fwd's image, byte for byte
-          ylo = Fwd<SIG, 0>::go(lo, cp, slow, tbl);
-          yhi = Fwd<SIG, 0>::go(hi, cp, slow, tbl);
-          const float4 yB = make_float4(ylo.b.x, ylo.b.y, yhi.b.x, yhi.b.y), yG = make_float4(ylo.g.x, ylo.g.y, yhi.g.x, yhi.g.y),
-                       yR = make_float4(ylo.r.x, ylo.r.y, yhi.r.x, yhi.r.y);
-          // lanes beyond the right edge compute garbage from zero-filled raw (a zero pixel is not zero after the chain): masked
-          if (active) {
-            const uint32_t s = sq_codes4(yB, lds4(gta + lane * 16)) + sq_codes4(yG, lds4(gta + RC::GTPLANEB + lane * 16)) +
-                               sq_codes4(yR, lds4(gta + 2 * RC::GTPLANEB + lane * 16));
-            sse += s;
-            if (a.u8) {      // (H,W,3) BGR bytes of the lane's 4 pixels: 12 contiguous bytes, 4-byte aligned (c0 % 4 == 0)
-              const uint32_t b0 = u8_code(yB.x), b1 = u8_code(yB.y), b2 = u8_code(yB.z), b3 = u8_code(yB.w);
-              const uint32_t g0 = u8_code(yG.x), g1 = u8_code(yG.y), g2 = u8_code(yG.z), g3 = u8_code(yG.w);
-              const uint32_t r0 = u8_code(yR.x), r1 = u8_code(yR.y), r2 = u8_code(yR.z), r3 = u8_code(yR.w);
-              uint32_t* po = reinterpret_cast<uint32_t*>(a.u8 + (((long long)n * H + r) * W + c0) * 3);
-              po[0] = b0 | (g0 << 8) | (r0 << 16) | (b1 << 24);
-              po[1] = g1 | (r1 << 8) | (b2 << 16) | (g2 << 24);
-              po[2] = r2 | (b3 << 8) | (g3 << 16) | (r3 << 24);
-            }
-          }
-        } else {
-          float4 tg[3];
-  #pragma unroll
-          for (int c = 0; c < 3; ++c) tg[c] = lds4(gta + c * RC::GTPLANEB + lane * 16);
-          P2 tlo, thi;
-          tlo.b = make_float2(tg[0].x, tg[0].y); tlo.g = make_float2(tg[1].x, tg[1].y); tlo.r = make_float2(tg[2].x, tg[2].y);
-          thi.b = make_float2(tg[0].z, tg[0].w); thi.g = make_float2(tg[1].z, tg[1].w); thi.r = make_float2(tg[2].z, tg[2].w);
-          Run<SIG, 0, MODE>::go(lo, tlo, cp, acc, loss, ylo, slow, lane_w, tbl);
-          Run<SIG, 0, MODE>::go(hi, thi, cp, acc, loss, yhi, slow, lane_w, tbl);
-        }
-        if (MODE != MODE_EVAL && (MODE == MODE_FWD || yb) && active) {
-          float* po = yb + (size_t)r * W + c0;
-          st_stream4(po, make_float4(ylo.b.x, ylo.b.y, yhi.b.x, yhi.b.y));
-          st_stream4(po + plane, make_float4(ylo.g.x, ylo.g.y, yhi.g.x, yhi.g.y));
-          st_stream4(po + 2 * plane, make_float4(ylo.r.x, ylo.r.y, yhi.r.x, yhi.r.y));
-        }
-      };
+      // ---- backward-carrying kernels: 2-row records ----
+      const LanePos L{own, oL0, oL1, oR0, oR1, (uint32_t)lane * 16u, c0, 0, active, lane_w};
 
       // iteration m computes rows r = ra + 2(m-1) (even) and r+1 (odd) from records m-1, m, m+1.
       // The loop exists twice, with the tone curve's slow flag (a knot outside [0,1]: final clamp active) as a compile-time
@@ -646,8 +675,8 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
   #pragma unroll
           for (int j = 0; j < WR; ++j) { we[j] = row_addr(r - HL + j); wo[j] = row_addr(r + 1 - HL + j); }
         }
-        do_row(std::false_type{}, slow_tag, r, we, recB + RC::RAWB);
-        do_row(std::true_type{}, slow_tag, r + 1, wo, recB + RC::RAWB + kStrip * 4);
+        do_row(std::false_type{}, slow_tag, std::false_type{}, r, [&](int j) { return we[j]; }, recB + RC::RAWB, L);
+        do_row(std::true_type{}, slow_tag, std::false_type{}, r + 1, [&](int j) { return wo[j]; }, recB + RC::RAWB + kStrip * 4, L);
         __syncwarp();                              // every lane has read record m-1: its slot may be refilled
         if (m - 1 + D < nrec) {
           if (elect_one()) issue(m - 1 + D);
@@ -768,6 +797,85 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
     gcount += (unsigned)nrec;
   }
 
+  if constexpr (MODE != MODE_FWD && NARROW) {
+    // ---- narrow items: the frame's last strip when it is nw = 32 or 64 columns wide (or less) ------------------------
+    // A full-width warp would issue its whole row loop for 8 or 16 useful lanes.  Here the warp splits into G = 128/nw
+    // groups of nw/4 lanes; a record holds 2G rows ((nw + kPad) x 2G raw box, nw x 2G x 3 GT box: no more bytes than a
+    // full record) and group g computes rows 2g, 2g+1 of it, so every lane still runs an even and then an odd row.  The
+    // window rows are per lane (reflect-101 folded in as in row_addr).  A CTA's narrow items come after its full ones:
+    // item t goes to CTA cpf-1 - t % cpf, the CTAs with the fewest full items.
+    const int nw = a.nw;
+    const int sh = (nw == 32) ? 3 : 2;              // log2 of the rows per record (2G)
+    const int RRn = 1 << sh;
+    const int grp = lane >> (6 - sh), li = lane & ((1 << (6 - sh)) - 1);
+    const int c0s = a.strip_blocks * kStrip, c0 = c0s + 4 * li;
+    const uint32_t rowb = (uint32_t)(nw + kPad) * 4u;
+    const bool incol = c0 < W, first = (c0 == 0), last = incol && (c0 + 4 >= W);
+    LanePos L;
+    L.own = (uint32_t)(kPad + 4 * li) * 4u;
+    L.oL0 = L.own + (first ? (HL == 1 ? 4 : 8) : -4 * HL);
+    L.oL1 = L.own + (first ? 4 : -4);
+    // a lane with c0 + 4 < W is never the last of its group (W <= c0s + nw).  Lanes past the frame read inside their row
+    // as well: past the last row of a 64-wide box lie pad bytes that no copy writes (stale data, possibly NaN)
+    const bool fold = last || !incol;
+    L.oR0 = L.own + (fold ? 8 : 16);
+    L.oR1 = L.own + (fold ? 4 : 20);
+    L.c0 = c0;
+    L.dr = 2 * grp;
+    const uint32_t gt_even = (uint32_t)(2 * grp * nw + 4 * li) * 4u;
+    for (int t = a.cpf - 1 - j0; t < a.nchunks; t += a.cpf) {
+      const int ra = t * a.nrows_per_chunk;
+      const int rb = min(H, ra + a.nrows_per_chunk);
+      const int rbase = ra - RRn;                   // record k holds rows rbase + RRn*k .. + RRn-1
+      const int nrec = (rb - ra + RRn - 1) / RRn + 2;
+      auto issue = [&](int k) {
+        const unsigned g = gcount + (unsigned)k;
+        const uint32_t rec = ring + (g & (D - 1)) * RC::RECB, bar = bars + (g & (D - 1)) * 8;
+        const bool has_gt = (k >= 1) && (k < nrec - 1);
+        mbar_expect_tx(bar, (uint32_t)RRn * rowb + (has_gt ? (uint32_t)RC::GTB : 0u));
+        tma_load_3d(rec, &tm_rawn, c0s - kPad, rbase + RRn * k, n, bar);
+        if (has_gt) tma_load_3d(rec + RC::RAWB, &tm_gtn, c0s, rbase + RRn * k, 3 * n, bar);
+      };
+      auto wait_rec = [&](int k) {
+        const unsigned g = gcount + (unsigned)k;
+        mbar_wait(bars + (g & (D - 1)) * 8, (g / D) & 1u);
+      };
+      auto row_addr = [&](int q) -> uint32_t {      // per lane
+        const int rel = reflect101(q, H) - rbase;
+        const unsigned g = gcount + (unsigned)(rel >> sh);
+        return ring + (g & (D - 1)) * RC::RECB + (uint32_t)(rel & (RRn - 1)) * rowb;
+      };
+      if (elect_one()) {
+        for (int k = 0; k < D && k < nrec; ++k) issue(k);
+      }
+      __syncwarp();
+      wait_rec(0);
+      wait_rec(1);
+      auto rows_loop = [&](auto slow_tag) {
+        for (int m = 1; m < nrec - 1; ++m) {
+          const int R = ra + RRn * (m - 1);         // group g computes rows R + 2g, R + 2g + 1
+          // a group past the item's last row is masked.  Its window rows, reflected at the frame's last row, still lie in
+          // the records m-1 .. m+1 (R <= H-2, so a reflected row is >= R - 2G + 1): loaded frame data, finite
+          L.active = incol && R + L.dr < rb;
+          L.lane_w = L.active ? 1.f : 0.f;
+          L.gt = gt_even;
+          wait_rec(m + 1);
+          const uint32_t gta = ring + ((gcount + (unsigned)m) & (D - 1)) * RC::RECB + RC::RAWB;
+          // window rows are computed where they are read: per-lane addresses live across the chain would cost registers
+          do_row(std::false_type{}, slow_tag, std::true_type{}, R, [&](int j) { return row_addr(R + L.dr - HL + j); }, gta, L);
+          L.gt = gt_even + (uint32_t)nw * 4u;
+          do_row(std::true_type{}, slow_tag, std::true_type{}, R + 1, [&](int j) { return row_addr(R + L.dr + 1 - HL + j); }, gta, L);
+          __syncwarp();                              // every lane has read record m-1: its slot may be refilled
+          if (m - 1 + D < nrec) {
+            if (elect_one()) issue(m - 1 + D);
+          }
+        }
+      };
+      if (slow) rows_loop(std::true_type{}); else rows_loop(std::false_type{});
+      gcount += (unsigned)nrec;
+    }
+  }
+
   if constexpr (MODE == MODE_EVAL) {
     const unsigned long long tot = warp_sum_u64(sse);
     if (lane == 0) a.sse[(long long)n * a.cpf + j0] = tot;
@@ -828,13 +936,61 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
 }
 
 // ---- host side ---------------------------------------------------------------------------------------------------------
-struct Geometry { int rows_per_chunk, chunks, strip_blocks, cpf, grid; };
+struct Geometry { int rows_per_chunk, chunks, strip_blocks, cpf, grid, nw, nrows_per_chunk, nchunks; };
 
-static Geometry geometry(int N, int H, int W, int ctas_per_sm, int rr, int max_rows = 256) {
-  Geometry g;
-  g.strip_blocks = (int)cdiv(W, kStrip);     // items are (row chunk, strip): one warp per CTA
+// Critical path of a layout, in row units: a full item of rf rows costs rf + rr + 2 (it also loads a lead-in record and
+// fills the pipeline), a narrow item of rn rows 2 * rn / (2G) + rr + 2.  CTA j runs full items j, j + cpf, .. < F, then
+// narrow items cpf-1-j, 2cpf-1-j, .. < Nn.  Both counts are step functions of j (at F % cpf and cpf - Nn % cpf), so the
+// extremes are on those steps.  Returns the largest cost over all CTAs; *narrow_max: the largest over CTAs with a narrow item.
+static long long layout_cost(long long F, long long cf, long long Nn, long long cn, long long cpf, long long* narrow_max) {
+  const long long js[6] = {0, F % cpf - 1, F % cpf, cpf - Nn % cpf - 1, cpf - Nn % cpf, cpf - 1};
+  long long worst = 0, nworst = 0;
+  for (long long j : js) {
+    if (j < 0 || j >= cpf) continue;
+    const long long nf = F > j ? cdiv(F - j, cpf) : 0, u = cpf - 1 - j, nn = Nn > u ? cdiv(Nn - u, cpf) : 0;
+    const long long c = nf * cf + nn * cn;
+    worst = c > worst ? c : worst;
+    if (nn > 0 && c > nworst) nworst = c;
+  }
+  *narrow_max = nworst;
+  return worst;
+}
+
+static Geometry geometry_uncached(int N, int H, int W, int ctas_per_sm, int rr, int max_rows, bool narrow) {
+  Geometry g{};
+  const int rem = W % kStrip;
+  g.nw = (narrow && rem > 0 && rem <= 64) ? (rem <= 32 ? 32 : 64) : 0;
+  g.strip_blocks = g.nw ? W / kStrip : (int)cdiv(W, kStrip);     // items are (row chunk, strip): one warp per CTA
   const int slots = sm_count() * ctas_per_sm;
   g.cpf = slots / N < 1 ? 1 : slots / N;
+  if (g.nw) {
+    // rows per full and per narrow chunk: least critical path, then the narrow items' CTAs least loaded (the cost of a
+    // narrow row is the least certain), then fewest items
+    const int rrn = 2 * (kStrip / g.nw);
+    long long best = -1, best_n = 0, best_items = 0;
+    for (int rf = rr; rf <= max_rows; rf += rr) {
+      if ((rf > H || g.strip_blocks == 0) && rf > rr) break;
+      const long long F = cdiv(H, rf) * g.strip_blocks, cf = rf + rr + 2;
+      for (int rn = rrn;; rn += rrn) {
+        const long long Nn = cdiv(H, rn), cn = 2 * (rn / rrn) + rr + 2;
+        if (best >= 0 && cn > best) break;          // grows with rn
+        const long long cpf = F + Nn < g.cpf ? F + Nn : g.cpf;
+        long long nmax;
+        const long long c = layout_cost(F, cf, Nn, cn, cpf, &nmax);
+        if (best < 0 || c < best || (c == best && (nmax < best_n || (nmax == best_n && F + Nn < best_items)))) {
+          best = c; best_n = nmax; best_items = F + Nn;
+          g.rows_per_chunk = rf; g.nrows_per_chunk = rn;
+        }
+        if (rn >= H) break;
+      }
+    }
+    g.chunks = g.strip_blocks ? (int)cdiv(H, g.rows_per_chunk) : 0;
+    g.nchunks = (int)cdiv(H, g.nrows_per_chunk);
+    const long long items = (long long)g.chunks * g.strip_blocks + g.nchunks;
+    if (items < g.cpf) g.cpf = (int)items;
+    g.grid = N * g.cpf;
+    return g;
+  }
   // rows per chunk: minimise rounds * (rows + per-item overhead); an item costs ~3 extra rows (window fill, exposed latency)
   long long best = -1;
   int best_rows = rr;
@@ -852,6 +1008,17 @@ static Geometry geometry(int N, int H, int W, int ctas_per_sm, int rr, int max_r
   if (items < g.cpf) g.cpf = (int)items;
   g.grid = N * g.cpf;
   return g;
+}
+
+// the narrow layout's search visits thousands of layouts: it runs once per shape, later launches look the result up
+static Geometry geometry(int N, int H, int W, int ctas_per_sm, int rr, int max_rows, bool narrow) {
+  static std::mutex mu;
+  static std::map<std::array<int, 7>, Geometry> cache;
+  const std::array<int, 7> key{N, H, W, ctas_per_sm, rr, max_rows, narrow ? 1 : 0};
+  std::lock_guard<std::mutex> lk(mu);
+  auto it = cache.find(key);
+  if (it == cache.end()) it = cache.emplace(key, geometry_uncached(N, H, W, ctas_per_sm, rr, max_rows, narrow)).first;
+  return it->second;
 }
 
 static std::mutex g_slot_mu;
@@ -877,12 +1044,12 @@ static float* cpar_device_ptr() {
   return p;
 }
 
-template <int DM, int MODE, unsigned SIG>
+template <int DM, int MODE, unsigned SIG, bool NARROW>
 static int resident_ctas() {
   static int n = 0;
   if (n == 0) {
-    cudaFuncSetAttribute(fused_kernel<DM, MODE, SIG>, cudaFuncAttributeMaxDynamicSharedMemorySize, RingCfg<MODE>::SMEM);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, fused_kernel<DM, MODE, SIG>, kWarps * 32, RingCfg<MODE>::SMEM) != cudaSuccess || n < 1) n = 1;
+    cudaFuncSetAttribute(fused_kernel<DM, MODE, SIG, NARROW>, cudaFuncAttributeMaxDynamicSharedMemorySize, RingCfg<MODE>::SMEM);
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, fused_kernel<DM, MODE, SIG, NARROW>, kWarps * 32, RingCfg<MODE>::SMEM) != cudaSuccess || n < 1) n = 1;
   }
   return n;
 }
@@ -921,11 +1088,15 @@ template <int DM, int MODE, unsigned SIG>
 static int launch_one(FusedArgs a, const ChainDesc& d, int N, cudaStream_t st, Geometry* gout) {
   // RISP_FUSED_FWD_ROWS / RISP_FUSED_STEP_ROWS: cap of the rows per item (experiments on the write order of the inference kernels)
   static const int cap = [] { const char* e = getenv(MODE == MODE_FWD ? "RISP_FUSED_FWD_ROWS" : "RISP_FUSED_STEP_ROWS"); return e ? atoi(e) : 0; }();
-  const Geometry g = geometry(N, a.H, a.W, resident_ctas<DM, MODE, SIG>(), RingCfg<MODE>::RR,
-                              cap >= RingCfg<MODE>::RR ? cap : (MODE == MODE_FWD ? RISP_FUSED_FWD_MAXROWS : 256));
+  // narrow items where the kernel that runs them keeps the occupancy of the one that does not
+  bool narrow = false;
+  if constexpr (MODE != MODE_FWD) narrow = resident_ctas<DM, MODE, SIG, true>() == resident_ctas<DM, MODE, SIG, false>();
+  const Geometry g = geometry(N, a.H, a.W, resident_ctas<DM, MODE, SIG, false>(), RingCfg<MODE>::RR,
+                              cap >= RingCfg<MODE>::RR ? cap : (MODE == MODE_FWD ? RISP_FUSED_FWD_MAXROWS : 256), narrow);
   if (gout) { *gout = g; return RISP_OK; }
   a.rows_per_chunk = g.rows_per_chunk; a.chunks = g.chunks; a.strip_blocks = g.strip_blocks; a.cpf = g.cpf;
-  CUtensorMap tm_raw, tm_gt;
+  a.nw = g.nw; a.nrows_per_chunk = g.nrows_per_chunk; a.nchunks = g.nchunks;
+  CUtensorMap tm_raw, tm_gt, tm_rawn, tm_gtn;
   int rc = make_map(&tm_raw, a.raw, a.W, a.H, N, kStrip + 2 * kPad, RingCfg<MODE>::RR, 1);
   if (rc != RISP_OK) return rc;
   if (MODE != MODE_FWD) {
@@ -934,7 +1105,25 @@ static int launch_one(FusedArgs a, const ChainDesc& d, int N, cudaStream_t st, G
   } else {
     tm_gt = tm_raw;
   }
-  fused_kernel<DM, MODE, SIG><<<dim3(g.cpf, N), kWarps * 32, RingCfg<MODE>::SMEM, st>>>(a, d, tm_raw, tm_gt);
+  if (g.nw) {     // narrow boxes: 4 pad columns on the left only (the strip ends at the frame's right edge), 2G rows
+    const int rrn = 2 * (kStrip / g.nw);
+    static_assert(RingCfg<MODE_STEP>::RAWB >= 36 * 8 * 4 && RingCfg<MODE_STEP>::RAWB >= 68 * 4 * 4 &&
+                  RingCfg<MODE_STEP>::GTB == 3 * 32 * 8 * 4 && RingCfg<MODE_STEP>::GTB == 3 * 64 * 4 * 4,
+                  "a narrow record must fit the ring's record");
+    rc = make_map(&tm_rawn, a.raw, a.W, a.H, N, g.nw + kPad, rrn, 1);
+    if (rc != RISP_OK) return rc;
+    rc = make_map(&tm_gtn, a.gt, a.W, a.H, 3ll * N, g.nw, rrn, 3);
+    if (rc != RISP_OK) return rc;
+  } else {
+    tm_rawn = tm_raw; tm_gtn = tm_gt;
+  }
+  if constexpr (MODE != MODE_FWD) {
+    if (g.nw) {
+      fused_kernel<DM, MODE, SIG, true><<<dim3(g.cpf, N), kWarps * 32, RingCfg<MODE>::SMEM, st>>>(a, d, tm_raw, tm_gt, tm_rawn, tm_gtn);
+      return check_launch("fused_kernel");
+    }
+  }
+  fused_kernel<DM, MODE, SIG, false><<<dim3(g.cpf, N), kWarps * 32, RingCfg<MODE>::SMEM, st>>>(a, d, tm_raw, tm_gt, tm_rawn, tm_gtn);
   return check_launch("fused_kernel");
 }
 

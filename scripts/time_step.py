@@ -3,7 +3,7 @@ Bayer_02_Demosaic_02_sRGB_11_13_01_14 (gain -> 3x10 polynomial -> gamma -> tone 
 (coefficient preparation + step kernel + finaliser).  The library is the one RISP_LIB_PATH names, so builds with
 different compile-time switches can be compared in one session:
 
-    RISP_LIB_PATH=build/abl/<variant>.so python scripts/time_step.py [launches=200] [repeats=5]
+    RISP_LIB_PATH=build/abl/<variant>.so python scripts/time_step.py [launches=200] [repeats=5] [width=4000]
 
 Prints one JSON line: ms per step for each repeat of `launches` back-to-back launches, and their median.
 """
@@ -22,6 +22,7 @@ N, H, W = 4, 3000, 4000
 def main():
     launches = int(sys.argv[1]) if len(sys.argv) > 1 else 200
     repeats = int(sys.argv[2]) if len(sys.argv) > 2 else 5
+    W = int(sys.argv[3]) if len(sys.argv) > 3 else globals()['W']
     g = torch.Generator().manual_seed(3)
     raw = torch.rand(N, 1, H, W, generator=g).cuda()
     gt = torch.rand(N, 3, H, W, generator=g).cuda()
@@ -41,7 +42,7 @@ def main():
         e1.record()
         torch.cuda.synchronize()
         ms.append(e0.elapsed_time(e1) / launches)
-    print(json.dumps({'lib': os.path.relpath(_lib.LIB_PATH), 'launches': launches, 'ms': [round(x, 5) for x in ms],
+    print(json.dumps({'lib': os.path.relpath(_lib.LIB_PATH), 'W': W, 'launches': launches, 'ms': [round(x, 5) for x in ms],
                       'median_ms': round(statistics.median(ms), 5), 'gpu': torch.cuda.get_device_name()}))
 
 
