@@ -17,7 +17,6 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, 'csrc')
 OBJ = os.path.join(ROOT, 'build', os.environ.get('RISP_BUILD_OBJ', 'obj'))
 LIB = os.environ.get('RISP_BUILD_LIB', os.path.join(HERE, 'libreconfigisp_b200.so'))
-EXTRA = os.environ.get('RISP_BUILD_FLAGS', '').split()
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
 FLAGS = ['-O3', '-std=c++17', '-lineinfo', '-gencode', 'arch=compute_100a,code=sm_100a',
          '-Xcompiler', '-fPIC', '-Xptxas', '-v', '--expt-relaxed-constexpr'] + os.environ.get('RISP_BUILD_FLAGS', '').split()

@@ -5,7 +5,7 @@
 // proxy-tuning step isp_model.py:128-142 (forward, MSELoss, backward).  Here: one pass, 16 B/px.
 //
 // Shape of the kernel (see DESIGN.md §4):
-//   * persistent CTAs (one wave: SMs x resident CTAs), each walking a static list of (row chunk, 512-column block)
+//   * persistent CTAs (one wave: SMs x resident CTAs), each walking a static list of (row chunk, 128-column strip)
 //     items of ONE frame -> accumulators live in registers for the whole kernel, one reduction per warp, and the
 //     summation order is fixed (bit-reproducible gradients);
 //   * a warp owns a 128-column strip and marches down the rows with the demosaic window in registers (horizontal halo
@@ -27,23 +27,23 @@ __constant__ float g_cpar[kCSlots][kCRows][kCRowFloats];
 
 // STEP: MSE loss; STEP_L1: L1 loss (isp_model.py:44-49); EVAL: inference arithmetic + squared 8-bit code differences to the GT
 enum { MODE_FWD = 0, MODE_STEP = 1, MODE_BWD = 2, MODE_STEP_L1 = 3, MODE_EVAL = 4 };
-constexpr int kWarps = 1;     // one warp per CTA: everything but the lane index is CTA-uniform (uniform datapath, no R2UR)
+// A CTA is one warp (32 threads), so everything but the lane index is CTA-uniform (uniform datapath, no R2UR).  The warp
+// owns a strip of kStrip columns.
 constexpr int kStrip = 128;
 
 struct FusedArgs {
   const float* raw;     // (N,1,H,W)
   const float* gt;      // (N,3,H,W): target (STEP) or dL/dy (BWD)
   float* y;             // (N,3,H,W), nullable except in FWD
-  float* partial;       // [N][cpf*kWarps][RISP_NSLOT]
+  float* partial;       // [N][cpf][RISP_NSLOT]
   const float* params;  // raw parameter rows (epilogue of the folded gain)
   int pstride;
   int H, W;
   int rows_per_chunk, chunks, strip_blocks, cpf;   // cpf = CTAs per frame
   float clip_hi;
   int slot;
-  int dbg;              // RISP_FUSED_DEBUG builds: 1 = no stores, 2 = no loads (bandwidth experiments)
   unsigned char* u8;    // EVAL: (N,H,W,3) 8-bit codes of y, nullable
-  unsigned long long* sse;   // EVAL: [N][cpf*kWarps] sums of squared code differences
+  unsigned long long* sse;   // EVAL: [N][cpf] sums of squared code differences
   // narrow items (backward-carrying kernels): the last strip of a frame, nw = 32 or 64 columns wide (0: none), marched by
   // 128/nw lane groups on as many row pairs at once; the strip_blocks full strips lie to its left
   int nw, nrows_per_chunk, nchunks;
@@ -59,7 +59,7 @@ __global__ void fused_prep_kernel(const float* __restrict__ params, int pstride,
     float* o = c + e.coff[k];
     const float* q = p + d.off[e.src[k]];
     switch (e.op[k]) {
-      case RISP_OP_GAMMA: o[0] = q[0]; o[1] = q[0] - 1.f; break;     // gm, gm - 1 (RFORM)
+      case RISP_OP_GAMMA: o[0] = q[0]; break;     // gm (the block stays 2 floats wide: fop_csize)
       case RISP_OP_GAIN: o[0] = q[0]; o[1] = q[1]; o[2] = q[2]; o[3] = 0.f; break;
       case RISP_OP_POLY10:
       case FOP_POLYG: {
@@ -83,8 +83,6 @@ __global__ void fused_prep_kernel(const float* __restrict__ params, int pstride,
         const float y1 = q[0], y2 = q[1], y3 = q[2];
         const float s0 = (y1 - 0.f) * 4.f, s1 = (y2 - y1) * 4.f, s2 = (y3 - y2) * 4.f, s3 = (1.f - y3) * 4.f;
         o[0] = s0; o[1] = s1 - s0; o[2] = s2 - s1; o[3] = s3 - s2;
-        const float s3acc = ((s0 + o[1]) + o[2]) + o[3];     // the slope the kernel accumulates on the last segment
-        o[4] = 1.f - s3acc;
         const bool in_range = (y1 >= 0.f && y1 <= 1.f) && (y2 >= 0.f && y2 <= 1.f) && (y3 >= 0.f && y3 <= 1.f);
         o[5] = in_range ? 0.f : 1.f;
         o[6] = 0.f; o[7] = 0.f;
@@ -145,15 +143,6 @@ __device__ __forceinline__ void sts4(uint32_t addr, float4 v) {
   asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
 }
 
-#ifndef RISP_FUSED_FWD_D
-#define RISP_FUSED_FWD_D 4
-#endif
-#ifndef RISP_FUSED_FWD_RR
-#define RISP_FUSED_FWD_RR 4
-#endif
-#ifndef RISP_FUSED_STEP_D
-#define RISP_FUSED_STEP_D 4
-#endif
 // tensor-map TMA: one instruction moves a (columns x rows x planes) box; out-of-bounds elements arrive as zeros
 __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* tm, int x, int y, int z, uint32_t mbar) {
   asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
@@ -163,19 +152,19 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* tm,
 constexpr int kPad = 4;            // floats of halo pad on each side of the raw strip
 template <int MODE>
 struct RingCfg {
-  static constexpr int D = (MODE == 0 /*MODE_FWD*/) ? RISP_FUSED_FWD_D : RISP_FUSED_STEP_D;   // records per warp (power of 2)
+  static constexpr int D = 4;                                            // records per warp (power of 2)
   // rows per record = rows per TMA box.  A TMA instruction costs the SM's copy engine ~150 cycles whatever its size
   // (measured: 1 KB boxes deliver 1.9 TB/s chip-wide), so the inference kernel, which has nothing but the copies to wait
   // for, uses 4-row boxes; the backward-carrying kernels are issue-bound and keep the smaller ring
-  static constexpr int RR = (MODE == 0 /*MODE_FWD*/) ? RISP_FUSED_FWD_RR : 2;
+  static constexpr int RR = (MODE == MODE_FWD) ? 4 : 2;
   static constexpr int RAWROWB = (kStrip + 2 * kPad) * 4;                // 544 B: one raw row of the box
   static constexpr int RAWB = (RR * RAWROWB + 127) / 128 * 128;          // RR rows, padded to a 128-B multiple
   static constexpr int GTPLANEB = RR * kStrip * 4;
-  static constexpr int GTB = (MODE == 0 /*MODE_FWD*/) ? 0 : 3 * GTPLANEB;  // [plane][row][128]
+  static constexpr int GTB = (MODE == MODE_FWD) ? 0 : 3 * GTPLANEB;  // [plane][row][128]
   static constexpr int RECB = RAWB + GTB;                                // multiple of 128
   static constexpr int WARPB = D * RECB;
-  static constexpr int TBLOFF = (kWarps * WARPB + kWarps * D * 8 + 63) / 64 * 64;   // tone-curve tables (one per stage slot)
-  static constexpr int SMEM = TBLOFF + ((MODE == 0 /*MODE_FWD*/) ? 0 : RISP_MAX_STAGES * kGtmTableBytes) + 128;  // records + mbarriers + tables + alignment slack
+  static constexpr int TBLOFF = (WARPB + D * 8 + 63) / 64 * 64;       // tone-curve tables (one per stage slot)
+  static constexpr int SMEM = TBLOFF + ((MODE == MODE_FWD) ? 0 : RISP_MAX_STAGES * kGtmTableBytes) + 128;  // records + mbarriers + tables + alignment slack
 };
 
 __device__ __forceinline__ int reflect101(int r, int H) { return r < 0 ? -r : (r >= H ? 2 * H - 2 - r : r); }
@@ -186,7 +175,6 @@ template <int DM, int HL, int RO, bool ODD, int WRT, bool PK>
 __device__ __forceinline__ void demosaic4(const float (&w)[WRT][4 + 2 * HL], float clip_hi, P2& lo, P2& hi) {
   float B[4], G[4], R[4];
   constexpr int M = RO + HL;     // window row of the pixel's own raw row
-#ifndef RISP_FUSED_NO_PACKED_DM
   if constexpr (DM == RISP_DM_BILINEAR && PK) {   // PK: the chain starts with packed arithmetic on the pairs (gain / polynomial)
     // The 0.5 / 0.25 / 1 weights are applied by ONE packed multiply per output pair (constant pair from the uniform
     // datapath): a pair like (raw, 0.5*sum) then leaves the demosaic as the result of an arithmetic instruction.  A pair
@@ -215,53 +203,51 @@ __device__ __forceinline__ void demosaic4(const float (&w)[WRT][4 + 2 * HL], flo
     const float2 sr = ODD ? make_float2(0.5f, 0.25f) : make_float2(1.f, 0.5f);
     lo.b = __fmul2_rn(make_float2(B[0], B[1]), sb); lo.g = __fmul2_rn(make_float2(G[0], G[1]), sg); lo.r = __fmul2_rn(make_float2(R[0], R[1]), sr);
     hi.b = __fmul2_rn(make_float2(B[2], B[3]), sb); hi.g = __fmul2_rn(make_float2(G[2], G[3]), sg); hi.r = __fmul2_rn(make_float2(R[2], R[3]), sr);
-    (void)clip_hi;
-    return;
-  }
-#endif
+  } else {
 #pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    const int x = HL + k;
-    const bool xo = (k & 1);
-    const float c = w[M][x];
-    if constexpr (DM == RISP_DM_NEAREST) {
-      if (!ODD) { R[k] = xo ? w[M][x - 1] : c; G[k] = xo ? c : w[M][x + 1]; B[k] = xo ? w[M + 1][x] : w[M + 1][x + 1]; }
-      else      { R[k] = xo ? w[M - 1][x - 1] : w[M - 1][x]; G[k] = xo ? w[M][x - 1] : c; B[k] = xo ? c : w[M][x + 1]; }
-    } else if constexpr (DM == RISP_DM_BILINEAR) {
-      const bool at_g = (ODD != xo);
-      if (at_g) {
-        const float hor = 0.5f * (w[M][x - 1] + w[M][x + 1]);
-        const float ver = 0.5f * (w[M - 1][x] + w[M + 1][x]);
-        G[k] = c;
-        if (!ODD) { R[k] = hor; B[k] = ver; } else { R[k] = ver; B[k] = hor; }
-      } else {
-        const float cross = (w[M - 1][x] + w[M + 1][x]) + (w[M][x - 1] + w[M][x + 1]);
-        const float diag = (w[M - 1][x - 1] + w[M - 1][x + 1]) + (w[M + 1][x - 1] + w[M + 1][x + 1]);
-        G[k] = 0.25f * cross;
-        if (!ODD) { R[k] = c; B[k] = 0.25f * diag; } else { R[k] = 0.25f * diag; B[k] = c; }
+    for (int k = 0; k < 4; ++k) {
+      const int x = HL + k;
+      const bool xo = (k & 1);
+      const float c = w[M][x];
+      if constexpr (DM == RISP_DM_NEAREST) {
+        if (!ODD) { R[k] = xo ? w[M][x - 1] : c; G[k] = xo ? c : w[M][x + 1]; B[k] = xo ? w[M + 1][x] : w[M + 1][x + 1]; }
+        else      { R[k] = xo ? w[M - 1][x - 1] : w[M - 1][x]; G[k] = xo ? w[M][x - 1] : c; B[k] = xo ? c : w[M][x + 1]; }
+      } else if constexpr (DM == RISP_DM_BILINEAR) {
+        const bool at_g = (ODD != xo);
+        if (at_g) {
+          const float hor = 0.5f * (w[M][x - 1] + w[M][x + 1]);
+          const float ver = 0.5f * (w[M - 1][x] + w[M + 1][x]);
+          G[k] = c;
+          if (!ODD) { R[k] = hor; B[k] = ver; } else { R[k] = ver; B[k] = hor; }
+        } else {
+          const float cross = (w[M - 1][x] + w[M + 1][x]) + (w[M][x - 1] + w[M][x + 1]);
+          const float diag = (w[M - 1][x - 1] + w[M - 1][x + 1]) + (w[M + 1][x - 1] + w[M + 1][x + 1]);
+          G[k] = 0.25f * cross;
+          if (!ODD) { R[k] = c; B[k] = 0.25f * diag; } else { R[k] = 0.25f * diag; B[k] = c; }
+        }
+      } else {  // Malvar-He-Cutler 5x5
+        const float n1 = w[M - 1][x], s1 = w[M + 1][x], e1 = w[M][x + 1], w1 = w[M][x - 1];
+        const float n2 = w[M - 2][x], s2 = w[M + 2][x], e2 = w[M][x + 2], w2 = w[M][x - 2];
+        const float dg = (w[M - 1][x - 1] + w[M - 1][x + 1]) + (w[M + 1][x - 1] + w[M + 1][x + 1]);
+        float rr, gg, bb;
+        const bool at_g = (ODD != xo);
+        if (at_g) {
+          const float f_row = 0.125f * (5.f * c + 4.f * (e1 + w1) - dg - (e2 + w2) + 0.5f * (n2 + s2));
+          const float f_col = 0.125f * (5.f * c + 4.f * (n1 + s1) - dg - (n2 + s2) + 0.5f * (e2 + w2));
+          gg = c;
+          if (!ODD) { rr = f_row; bb = f_col; } else { rr = f_col; bb = f_row; }
+        } else {
+          const float f_g = 0.125f * (4.f * c + 2.f * ((n1 + s1) + (e1 + w1)) - ((n2 + s2) + (e2 + w2)));
+          const float f_dg = 0.125f * (6.f * c + 2.f * dg - 1.5f * ((n2 + s2) + (e2 + w2)));
+          gg = f_g;
+          if (!ODD) { rr = c; bb = f_dg; } else { rr = f_dg; bb = c; }
+        }
+        R[k] = fminf(fmaxf(rr, 0.f), clip_hi); G[k] = fminf(fmaxf(gg, 0.f), clip_hi); B[k] = fminf(fmaxf(bb, 0.f), clip_hi);
       }
-    } else {  // Malvar-He-Cutler 5x5
-      const float n1 = w[M - 1][x], s1 = w[M + 1][x], e1 = w[M][x + 1], w1 = w[M][x - 1];
-      const float n2 = w[M - 2][x], s2 = w[M + 2][x], e2 = w[M][x + 2], w2 = w[M][x - 2];
-      const float dg = (w[M - 1][x - 1] + w[M - 1][x + 1]) + (w[M + 1][x - 1] + w[M + 1][x + 1]);
-      float rr, gg, bb;
-      const bool at_g = (ODD != xo);
-      if (at_g) {
-        const float f_row = 0.125f * (5.f * c + 4.f * (e1 + w1) - dg - (e2 + w2) + 0.5f * (n2 + s2));
-        const float f_col = 0.125f * (5.f * c + 4.f * (n1 + s1) - dg - (n2 + s2) + 0.5f * (e2 + w2));
-        gg = c;
-        if (!ODD) { rr = f_row; bb = f_col; } else { rr = f_col; bb = f_row; }
-      } else {
-        const float f_g = 0.125f * (4.f * c + 2.f * ((n1 + s1) + (e1 + w1)) - ((n2 + s2) + (e2 + w2)));
-        const float f_dg = 0.125f * (6.f * c + 2.f * dg - 1.5f * ((n2 + s2) + (e2 + w2)));
-        gg = f_g;
-        if (!ODD) { rr = c; bb = f_dg; } else { rr = f_dg; bb = c; }
-      }
-      R[k] = fminf(fmaxf(rr, 0.f), clip_hi); G[k] = fminf(fmaxf(gg, 0.f), clip_hi); B[k] = fminf(fmaxf(bb, 0.f), clip_hi);
     }
+    lo.b = make_float2(B[0], B[1]); lo.g = make_float2(G[0], G[1]); lo.r = make_float2(R[0], R[1]);
+    hi.b = make_float2(B[2], B[3]); hi.g = make_float2(G[2], G[3]); hi.r = make_float2(R[2], R[3]);
   }
-  lo.b = make_float2(B[0], B[1]); lo.g = make_float2(G[0], G[1]); lo.r = make_float2(R[0], R[1]);
-  hi.b = make_float2(B[2], B[3]); hi.g = make_float2(G[2], G[3]); hi.r = make_float2(R[2], R[3]);
 }
 
 // ---- the chain on one pixel pair: forward, loss, backward (compile-time recursion over the effective stages) ----------
@@ -287,13 +273,13 @@ struct Tail {
       if constexpr (MODE == MODE_BWD) return tgt;
       // d loss / d y up to the constant 2/numel (applied by the finaliser).  lane_w = 1 for lanes inside the frame (1*x - t is
       // exactly x - t) and 0 for the lanes of the last strip that hang over the right edge (their t is 0): no divergent branch
-      const float2 dd = (kScalarLoss && SC) ? make_float2(fmaf(lane_w, x.x, -tgt.x), fmaf(lane_w, x.y, -tgt.y))
-                                    : __ffma2_rn(make_float2(lane_w, lane_w), x, make_float2(-tgt.x, -tgt.y));
+      const float2 dd = SC ? make_float2(fmaf(lane_w, x.x, -tgt.x), fmaf(lane_w, x.y, -tgt.y))
+                           : __ffma2_rn(make_float2(lane_w, lane_w), x, make_float2(-tgt.x, -tgt.y));
       if constexpr (MODE == MODE_STEP_L1) {      // nn.L1Loss: sum |y - t| ; gradient sign(y - t) (0 at equality), 1/numel later
-        acc_add<kScalarLoss && SC>(loss, make_float2(fabsf(dd.x), fabsf(dd.y)));
+        acc_add<SC>(loss, make_float2(fabsf(dd.x), fabsf(dd.y)));
         return make_float2((dd.x > 0.f ? 1.f : 0.f) - (dd.x < 0.f ? 1.f : 0.f), (dd.y > 0.f ? 1.f : 0.f) - (dd.y < 0.f ? 1.f : 0.f));
       }
-      acc_fma<kScalarLoss && SC>(loss, dd, dd);
+      acc_fma<SC>(loss, dd, dd);
       return dd;
     } else {
       constexpr int OP = E.op[K];
@@ -304,16 +290,11 @@ struct Tail {
       if constexpr (OP == RISP_OP_SKIP) {
         return Tail<SIG, K + 1, MODE, C>::go(x, tgt, cp, acc, loss, yout, slow, lane_w, tbl);
       } else if constexpr (OP == RISP_OP_GAMMA) {
-        float2 l2, r = zero2();
+        float2 l2;
         const float gm = c[0];
-#ifdef RISP_FUSED_RFORM      // measured: 2 % slower (the product y = r xc lengthens the dependent chain; the XU pipe is not the limiter)
-        constexpr bool RFORM = NEED_DX && MODE != MODE_FWD;
-#else
-        constexpr bool RFORM = false;
-#endif
-        const float2 y = gamma_fwd2<IN01, RFORM>(x, gm, l2, c[1], &r);
+        const float2 y = gamma_fwd2<IN01>(x, gm, l2);
         const float2 d = Tail<SIG, K + 1, MODE, C>::go(y, tgt, cp, acc, loss, yout, slow, lane_w, tbl);
-        return gamma_bwd2<IN01, NEED_DX, true, NOMASK, RFORM, SC>(x, y, l2, d, gm, a[0], r);
+        return gamma_bwd2<IN01, NEED_DX, true, NOMASK, SC>(x, y, l2, d, gm, a[0]);
       } else if constexpr (OP == RISP_OP_GAIN) {
         const float2 y = mul2s(x, c[C]);
         const float2 d = Tail<SIG, K + 1, MODE, C>::go(y, tgt, cp, acc, loss, yout, slow, lane_w, tbl);
@@ -321,11 +302,11 @@ struct Tail {
         return NEED_DX ? mul2s(d, c[C]) : zero2();
       } else {
         static_assert(OP == RISP_OP_GTM && IN01, "packed path: unsupported per-channel op");
-        float2 hd[3], m = zero2();
-        const float2 y = gtm_fwd2<kGtmTable>(x, c, hd, slow, m, tbl + K * kGtmTableBytes);
+        float2 slope, m = zero2();
+        const float2 y = gtm_fwd2<true>(x, c, slope, slow, m, tbl + K * kGtmTableBytes);
         float2 d = Tail<SIG, K + 1, MODE, C>::go(y, tgt, cp, acc, loss, yout, slow, lane_w, tbl);
         if (slow) d = mul2(d, m);
-        return gtm_bwd2<NEED_DX, SC>(x, hd, d, c, a);
+        return gtm_bwd2<NEED_DX, SC>(x, slope, d, a);
       }
     }
   }
@@ -354,11 +335,6 @@ struct Run {
         const P2 y = gamma_fwd<IN01>(x, gm, sv);
         const P2 d = Run<SIG, K + 1, MODE>::go(y, tgt, cp, acc, loss, yout, slow, lane_w, tbl);
         return gamma_bwd<IN01, NEED_DX, true>(sv, d, gm, a[0]);
-      } else if constexpr (OP == RISP_OP_GAIN) {
-        GainSaved sv;
-        const P2 y = gain_fwd(x, c, sv);
-        const P2 d = Run<SIG, K + 1, MODE>::go(y, tgt, cp, acc, loss, yout, slow, lane_w, tbl);
-        return gain_bwd<NEED_DX>(sv, d, c, a);
       } else if constexpr ((OP == RISP_OP_POLY10 || OP == FOP_POLYG) && !NEED_DX && per_channel_from<SIG>(K + 1)) {
         // channel-major: the monomials are the only cross-channel state; each output channel then runs its polynomial
         // row, its whole tail, the loss and the way back, and accumulates e_c * phi straight away
@@ -368,24 +344,13 @@ struct Run {
         phi[6] = x.b; phi[7] = x.g; phi[8] = x.r;
         auto channel = [&](auto ctag, float2 tg, float2& yo) {
           constexpr int C = decltype(ctag)::value;
-          float2 u;
-          if constexpr (kScalarPolyFwd) {
-            u = make_float2(fmaf(c[C * 10], phi[0].x, c[C * 10 + 9]), fmaf(c[C * 10], phi[0].y, c[C * 10 + 9]));
+          float2 u = make_float2(fmaf(c[C * 10], phi[0].x, c[C * 10 + 9]), fmaf(c[C * 10], phi[0].y, c[C * 10 + 9]));
 #pragma unroll
-            for (int i = 1; i < 9; ++i) u = make_float2(fmaf(c[C * 10 + i], phi[i].x, u.x), fmaf(c[C * 10 + i], phi[i].y, u.y));
-          } else {
-            u = fma2ss(c[C * 10], phi[0], c[C * 10 + 9]);
-#pragma unroll
-            for (int i = 1; i < 9; ++i) u = fma2s(c[C * 10 + i], phi[i], u);
-          }
+          for (int i = 1; i < 9; ++i) u = make_float2(fmaf(c[C * 10 + i], phi[i].x, u.x), fmaf(c[C * 10 + i], phi[i].y, u.y));
           const float2 y = sat2(u);
-#ifndef RISP_FUSED_NO_MERGED_MASK
           // a gamma directly behind the polynomial masks its gradient with [y >= eps]; together with the clamp mask
           // [0 <= u <= 1] that is [eps <= u <= 1] <=> max(sat(u), eps) == u: one compare on the value gamma computes anyway
           constexpr bool GNEXT = (K + 1 < E.n) && (E.op[K + 1 < E.n ? K + 1 : K] == RISP_OP_GAMMA);
-#else
-          constexpr bool GNEXT = false;
-#endif
           const float2 d = Tail<SIG, K + 1, MODE, C, GNEXT>::go(y, tg, cp, acc, loss, yo, slow, lane_w, tbl);
           float2 e;
           if constexpr (GNEXT) {
@@ -395,25 +360,21 @@ struct Run {
             e = sel2(u.x == y.x, u.y == y.y, d);     // clamp mask, inclusive: u in [0,1] <=> sat(u) == u
           }
 #pragma unroll
-          for (int i = 0; i < 9; ++i) acc_fma<kFoldS>(a[C * 10 + i], e, phi[i]);
-          acc_add<kFoldS>(a[C * 10 + 9], e);
+          for (int i = 0; i < 9; ++i) acc_fma<true>(a[C * 10 + i], e, phi[i]);
+          acc_add<true>(a[C * 10 + 9], e);
         };
         channel(std::integral_constant<int, 0>{}, tgt.b, yout.b);
         channel(std::integral_constant<int, 1>{}, tgt.g, yout.g);
         channel(std::integral_constant<int, 2>{}, tgt.r, yout.r);
         P2 z; z.b = zero2(); z.g = zero2(); z.r = zero2();
         return z;
-      } else if constexpr (OP == RISP_OP_POLY10 || OP == FOP_POLYG) {
+      } else {
+        // a gain or tone curve in front of a cross-channel stage: no instantiated signature has one (Tail runs them)
+        static_assert(OP == RISP_OP_POLY10 || OP == FOP_POLYG, "packed path: unsupported effective op");
         PolySaved sv;
         const P2 y = poly_fwd(x, c, sv);
         const P2 d = Run<SIG, K + 1, MODE>::go(y, tgt, cp, acc, loss, yout, slow, lane_w, tbl);
         return poly_bwd<NEED_DX>(sv, d, c, a);
-      } else {
-        static_assert(OP == RISP_OP_GTM && IN01, "packed path: unsupported effective op");
-        GtmSaved sv;
-        const P2 y = gtm_fwd<kGtmTable>(x, c, sv, slow, tbl + K * kGtmTableBytes);
-        const P2 d = Run<SIG, K + 1, MODE>::go(y, tgt, cp, acc, loss, yout, slow, lane_w, tbl);
-        return gtm_bwd<NEED_DX>(sv, d, c, a, slow);
       }
     }
   }
@@ -422,7 +383,7 @@ struct Run {
 template <unsigned SIG, int K>
 struct Fwd {
   static constexpr EffChain E = Eff<SIG>::e;
-  static __device__ __forceinline__ P2 go(const P2& x, const float* __restrict__ cp, bool slow, uint32_t tbl) {
+  static __device__ __forceinline__ P2 go(const P2& x, const float* __restrict__ cp, bool slow) {
     if constexpr (K == E.n) {
       return x;
     } else {
@@ -432,10 +393,10 @@ struct Fwd {
       P2 y;
       if constexpr (OP == RISP_OP_SKIP) { y = x; }
       else if constexpr (OP == RISP_OP_GAMMA) { GammaSaved sv; y = gamma_fwd<IN01>(x, c[0], sv); }
-      else if constexpr (OP == RISP_OP_GAIN) { GainSaved sv; y = gain_fwd(x, c, sv); }
+      else if constexpr (OP == RISP_OP_GAIN) { y = gain_fwd(x, c); }
       else if constexpr (OP == RISP_OP_POLY10 || OP == FOP_POLYG) { PolySaved sv; y = poly_fwd(x, c, sv); }
-      else { GtmSaved sv; y = gtm_fwd<false>(x, c, sv, slow, 0u); }
-      return Fwd<SIG, K + 1>::go(y, cp, slow, tbl);
+      else { y = gtm_fwd(x, c, slow); }
+      return Fwd<SIG, K + 1>::go(y, cp, slow);
     }
   }
 };
@@ -450,20 +411,14 @@ __device__ __forceinline__ bool chain_slow(const float* __restrict__ cp) {
   return slow;
 }
 
-#ifndef RISP_FUSED_STEP_MINB
-#define RISP_FUSED_STEP_MINB 8
-#endif
-#ifndef RISP_FUSED_FWD_MINB
-#define RISP_FUSED_FWD_MINB 16
-#endif
-#ifndef RISP_FUSED_FWD_MAXROWS
-#define RISP_FUSED_FWD_MAXROWS 256
-#endif
+constexpr int kStepMinBlocks = 8;    // resident CTAs per SM the kernels are compiled for (register cap)
+constexpr int kFwdMinBlocks = 16;
+constexpr int kMaxRows = 256;        // rows per item at most
 
 // NARROW: the kernel also runs narrow items (a.nw != 0); a separate instantiation, so that the kernels of frames without
 // them keep their register allocation
 template <int DM, int MODE, unsigned SIG, bool NARROW>
-__global__ void __launch_bounds__(kWarps * 32, (MODE == MODE_FWD) ? RISP_FUSED_FWD_MINB : RISP_FUSED_STEP_MINB)
+__global__ void __launch_bounds__(32, (MODE == MODE_FWD) ? kFwdMinBlocks : kStepMinBlocks)
 fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_raw, const __grid_constant__ CUtensorMap tm_gt,
              const __grid_constant__ CUtensorMap tm_rawn, const __grid_constant__ CUtensorMap tm_gtn) {
   constexpr EffChain E = Eff<SIG>::e;
@@ -500,7 +455,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
 #pragma unroll
     for (int s = 0; s < D; ++s) mbar_init(bars + 8 * s, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    if constexpr (kGtmTable && MODE != MODE_FWD && MODE != MODE_EVAL) {
+    if constexpr (MODE != MODE_FWD && MODE != MODE_EVAL) {
 #pragma unroll
       for (int k = 0; k < E.n; ++k)
         if (E.op[k] == RISP_OP_GTM) gtm_table_fill(tbl + k * kGtmTableBytes, cp + E.coff[k]);
@@ -526,12 +481,11 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
   };
   // ---- backward-carrying kernels (issue-bound): a private window per row read with plain LDS ----
   // one row: read the window (wa(j): shared-memory address of its raw row j) and the GT row, demosaic, chain, store.
-  // NARROW: the lane's row may belong to another item while its GT is real data: such a lane's target is zeroed so that it
-  // adds exactly nothing.
+  // Narrow items: the lane's row may belong to another item while its GT is real data: such a lane's target is zeroed so
+  // that it adds exactly nothing.
   auto do_row = [&](auto odd_tag, auto slow_tag, auto narrow_tag, int r, auto wa, uint32_t gta, const LanePos& L) {
     constexpr bool ODD = decltype(odd_tag)::value;
     constexpr bool slow = decltype(slow_tag)::value;     // shadows the run-time flag: the chain's branches on it fold away
-    constexpr bool NARROW = decltype(narrow_tag)::value;
     float w[WR][WC];
 #pragma unroll
     for (int j = 0; j < WR; ++j) {
@@ -550,8 +504,8 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
     P2 ylo, yhi;
     if constexpr (MODE == MODE_EVAL) {
       // the inference arithmetic (Fwd, not Run): the codes are those of risp_pipeline_fwd's image, byte for byte
-      ylo = Fwd<SIG, 0>::go(lo, cp, slow, tbl);
-      yhi = Fwd<SIG, 0>::go(hi, cp, slow, tbl);
+      ylo = Fwd<SIG, 0>::go(lo, cp, slow);
+      yhi = Fwd<SIG, 0>::go(hi, cp, slow);
       const float4 yB = make_float4(ylo.b.x, ylo.b.y, yhi.b.x, yhi.b.y), yG = make_float4(ylo.g.x, ylo.g.y, yhi.g.x, yhi.g.y),
                    yR = make_float4(ylo.r.x, ylo.r.y, yhi.r.x, yhi.r.y);
       // lanes beyond the right edge compute garbage from zero-filled raw (a zero pixel is not zero after the chain): masked
@@ -570,11 +524,12 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
         }
       }
     } else {
+      constexpr bool narrow_item = decltype(narrow_tag)::value;
       float4 tg[3];
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
         tg[c] = lds4(gta + c * RC::GTPLANEB + L.gt);
-        if constexpr (NARROW) {
+        if constexpr (narrow_item) {
           if (!L.active) tg[c] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
       }
@@ -607,9 +562,6 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
     const int nrec = (rb - ra + RR - 1) / RR + 2;
 
     auto issue = [&](int k) {        // one elected lane: the two TMA boxes of record k
-#ifdef RISP_FUSED_DEBUG
-      if (a.dbg & 2) return;
-#endif
       const unsigned g = gcount + (unsigned)k;
       const uint32_t rec = ring + (g & (D - 1)) * RC::RECB, bar = bars + (g & (D - 1)) * 8;
       const bool has_gt = (MODE != MODE_FWD) && (k >= 1) && (k < nrec - 1);
@@ -618,9 +570,6 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
       if (has_gt) tma_load_3d(rec + RC::RAWB, &tm_gt, c0s, rbase + RR * k, 3 * n, bar);
     };
     auto wait_rec = [&](int k) {
-#ifdef RISP_FUSED_DEBUG
-      if (a.dbg & 2) return;
-#endif
       const unsigned g = gcount + (unsigned)k;
       mbar_wait(bars + (g & (D - 1)) * 8, (g / D) & 1u);
     };
@@ -690,16 +639,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
       auto load_row = [&](float* dst, uint32_t ra_) {            // one raw row of the window: columns c0-HL .. c0+3+HL
         const unsigned full = 0xffffffffu;
         const float4 v = lds4(ra_ + own);
-        if constexpr (MODE != MODE_FWD) {
-          // issue-bound kernels: every lane reads its halo columns from the record (a 4-way bank conflict costs nothing here,
-          // two shuffles and two selects per row do)
-          if constexpr (HL == 1) {
-            dst[0] = lds1(ra_ + oL0); dst[1] = v.x; dst[2] = v.y; dst[3] = v.z; dst[4] = v.w; dst[5] = lds1(ra_ + oR0);
-          } else {
-            dst[0] = lds1(ra_ + oL0); dst[1] = lds1(ra_ + oL1); dst[2] = v.x; dst[3] = v.y; dst[4] = v.z; dst[5] = v.w;
-            dst[6] = lds1(ra_ + oR0); dst[7] = lds1(ra_ + oR1);
-          }
-        } else if constexpr (HL == 1) {
+        if constexpr (HL == 1) {
           float l = __shfl_up_sync(full, v.w, 1), r = __shfl_down_sync(full, v.x, 1);
           if (endL) l = lds1(ra_ + oL0);
           if (endR) r = lds1(ra_ + oR0);
@@ -713,39 +653,14 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
         }
       };
 
-      // one row from the register window w[RO .. RO+WR): demosaic, chain (+ loss and backward), store
-      auto do_row = [&](auto ro_tag, auto odd_tag, int r, uint32_t gta, const uint32_t* wa) {
+      // one row from the register window w[RO .. RO+WR): demosaic, chain, store
+      auto do_row = [&](auto ro_tag, auto odd_tag, int r) {
         constexpr int RO = decltype(ro_tag)::value;
         constexpr bool ODD = decltype(odd_tag)::value;
         P2 lo, hi;
-        if constexpr (MODE == MODE_FWD) {
-          demosaic4<DM, HL, RO, ODD, WR + 1, PKDM>(w, a.clip_hi, lo, hi);
-        } else {                                     // register-heavy modes: a private window, dead before the chain starts
-          float wl[WR][WC];
-  #pragma unroll
-          for (int j = 0; j < WR; ++j) load_row(wl[j], wa[j]);
-          demosaic4<DM, HL, 0, ODD, WR, PKDM>(wl, a.clip_hi, lo, hi);
-        }
-        P2 ylo, yhi;
-        if constexpr (MODE == MODE_FWD) {
-          ylo = Fwd<SIG, 0>::go(lo, cp, slow, tbl);
-          yhi = Fwd<SIG, 0>::go(hi, cp, slow, tbl);
-        } else {
-          float4 tg[3];
-  #pragma unroll
-          for (int c = 0; c < 3; ++c) tg[c] = lds4(gta + c * RC::GTPLANEB + lane * 16);
-          P2 tlo, thi;
-          tlo.b = make_float2(tg[0].x, tg[0].y); tlo.g = make_float2(tg[1].x, tg[1].y); tlo.r = make_float2(tg[2].x, tg[2].y);
-          thi.b = make_float2(tg[0].z, tg[0].w); thi.g = make_float2(tg[1].z, tg[1].w); thi.r = make_float2(tg[2].z, tg[2].w);
-          Run<SIG, 0, MODE>::go(lo, tlo, cp, acc, loss, ylo, slow, lane_w, tbl);
-          Run<SIG, 0, MODE>::go(hi, thi, cp, acc, loss, yhi, slow, lane_w, tbl);
-        }
-  #ifdef RISP_FUSED_DEBUG
-        const bool st_ok = !(a.dbg & 1) || ylo.b.x == 12345.678f;
-  #else
-        constexpr bool st_ok = true;
-  #endif
-        if ((MODE == MODE_FWD || yb) && active && st_ok) {
+        demosaic4<DM, HL, RO, ODD, WR + 1, PKDM>(w, a.clip_hi, lo, hi);
+        const P2 ylo = Fwd<SIG, 0>::go(lo, cp, slow), yhi = Fwd<SIG, 0>::go(hi, cp, slow);
+        if (active) {
           float* po = yb + (size_t)r * W + c0;
           st_stream4(po, make_float4(ylo.b.x, ylo.b.y, yhi.b.x, yhi.b.y));
           st_stream4(po + plane, make_float4(ylo.g.x, ylo.g.y, yhi.g.x, yhi.g.y));
@@ -776,16 +691,11 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
   #pragma unroll
               for (int j = 0; j < WR + 1; ++j) wa[j] = row_addr(r - HL + j);
             }
-            if constexpr (MODE == MODE_FWD) {          // the WR+1 rows are read once and serve both output rows
+            // the WR+1 rows are read once and serve both output rows
   #pragma unroll
-              for (int j = 0; j < WR + 1; ++j) load_row(w[j], wa[j]);
-              do_row(std::integral_constant<int, 0>{}, std::false_type{}, r, 0u, wa);
-              do_row(std::integral_constant<int, 1>{}, std::true_type{}, r + 1, 0u, wa);
-            } else {                                   // register-heavy modes: one window at a time
-              const uint32_t gta = recB + RC::RAWB + (uint32_t)(2 * p) * kStrip * 4;
-              do_row(std::integral_constant<int, 0>{}, std::false_type{}, r, gta, wa);
-              do_row(std::integral_constant<int, 0>{}, std::true_type{}, r + 1, gta + kStrip * 4, wa + 1);
-            }
+            for (int j = 0; j < WR + 1; ++j) load_row(w[j], wa[j]);
+            do_row(std::integral_constant<int, 0>{}, std::false_type{}, r);
+            do_row(std::integral_constant<int, 1>{}, std::true_type{}, r + 1);
           }
         }
         __syncwarp();                              // every lane has read record m-1: its slot may be refilled
@@ -1049,7 +959,7 @@ static int resident_ctas() {
   static int n = 0;
   if (n == 0) {
     cudaFuncSetAttribute(fused_kernel<DM, MODE, SIG, NARROW>, cudaFuncAttributeMaxDynamicSharedMemorySize, RingCfg<MODE>::SMEM);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, fused_kernel<DM, MODE, SIG, NARROW>, kWarps * 32, RingCfg<MODE>::SMEM) != cudaSuccess || n < 1) n = 1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, fused_kernel<DM, MODE, SIG, NARROW>, 32, RingCfg<MODE>::SMEM) != cudaSuccess || n < 1) n = 1;
   }
   return n;
 }
@@ -1085,15 +995,15 @@ static int make_map(CUtensorMap* tm, const float* base, int W, int H, long long 
 }
 
 template <int DM, int MODE, unsigned SIG>
-static int launch_one(FusedArgs a, const ChainDesc& d, int N, cudaStream_t st, Geometry* gout) {
-  // RISP_FUSED_FWD_ROWS / RISP_FUSED_STEP_ROWS: cap of the rows per item (experiments on the write order of the inference kernels)
-  static const int cap = [] { const char* e = getenv(MODE == MODE_FWD ? "RISP_FUSED_FWD_ROWS" : "RISP_FUSED_STEP_ROWS"); return e ? atoi(e) : 0; }();
+static int launch_one(FusedArgs a, const ChainDesc& d, int N, cudaStream_t st, int* rows_per_frame) {
+  // RISP_FUSED_STEP_ROWS: cap of the rows per item of the backward-carrying and evaluation kernels (many short items)
+  static const int cap = [] { const char* e = MODE == MODE_FWD ? nullptr : getenv("RISP_FUSED_STEP_ROWS"); return e ? atoi(e) : 0; }();
   // narrow items where the kernel that runs them keeps the occupancy of the one that does not
   bool narrow = false;
   if constexpr (MODE != MODE_FWD) narrow = resident_ctas<DM, MODE, SIG, true>() == resident_ctas<DM, MODE, SIG, false>();
   const Geometry g = geometry(N, a.H, a.W, resident_ctas<DM, MODE, SIG, false>(), RingCfg<MODE>::RR,
-                              cap >= RingCfg<MODE>::RR ? cap : (MODE == MODE_FWD ? RISP_FUSED_FWD_MAXROWS : 256), narrow);
-  if (gout) { *gout = g; return RISP_OK; }
+                              cap >= RingCfg<MODE>::RR ? cap : kMaxRows, narrow);
+  if (rows_per_frame) *rows_per_frame = g.cpf;
   a.rows_per_chunk = g.rows_per_chunk; a.chunks = g.chunks; a.strip_blocks = g.strip_blocks; a.cpf = g.cpf;
   a.nw = g.nw; a.nrows_per_chunk = g.nrows_per_chunk; a.nchunks = g.nchunks;
   CUtensorMap tm_raw, tm_gt, tm_rawn, tm_gtn;
@@ -1119,17 +1029,18 @@ static int launch_one(FusedArgs a, const ChainDesc& d, int N, cudaStream_t st, G
   }
   if constexpr (MODE != MODE_FWD) {
     if (g.nw) {
-      fused_kernel<DM, MODE, SIG, true><<<dim3(g.cpf, N), kWarps * 32, RingCfg<MODE>::SMEM, st>>>(a, d, tm_raw, tm_gt, tm_rawn, tm_gtn);
+      fused_kernel<DM, MODE, SIG, true><<<dim3(g.cpf, N), 32, RingCfg<MODE>::SMEM, st>>>(a, d, tm_raw, tm_gt, tm_rawn, tm_gtn);
       return check_launch("fused_kernel");
     }
   }
-  fused_kernel<DM, MODE, SIG, false><<<dim3(g.cpf, N), kWarps * 32, RingCfg<MODE>::SMEM, st>>>(a, d, tm_raw, tm_gt, tm_rawn, tm_gtn);
+  fused_kernel<DM, MODE, SIG, false><<<dim3(g.cpf, N), 32, RingCfg<MODE>::SMEM, st>>>(a, d, tm_raw, tm_gt, tm_rawn, tm_gtn);
   return check_launch("fused_kernel");
 }
 
 template <int MODE>
-static int dispatch(const FusedArgs& a, const ChainDesc& d, unsigned sig, int N, int dm_kind, cudaStream_t st, Geometry* gout) {
-#define RISP_F_SIG(DMK, SG) if (sig == (SG)) return launch_one<DMK, MODE, (SG)>(a, d, N, st, gout);
+static int dispatch(const FusedArgs& a, const ChainDesc& d, int N, int dm_kind, cudaStream_t st, int* rows_per_frame) {
+  const unsigned sig = chain_signature(d);
+#define RISP_F_SIG(DMK, SG) if (sig == (SG)) return launch_one<DMK, MODE, (SG)>(a, d, N, st, rows_per_frame);
 #define RISP_F_DM(DMK) RISP_F_SIG(DMK, RISP_SIG_A) RISP_F_SIG(DMK, RISP_SIG_B) RISP_F_SIG(DMK, RISP_SIG_C) RISP_F_SIG(DMK, RISP_SIG_D) \
   if constexpr (MODE == MODE_FWD || MODE == MODE_EVAL) { RISP_F_SIG(DMK, RISP_SIG_SKIP) }
   switch (dm_kind) {
@@ -1141,6 +1052,15 @@ static int dispatch(const FusedArgs& a, const ChainDesc& d, unsigned sig, int N,
 #undef RISP_F_DM
 #undef RISP_F_SIG
   return 1;   // not handled
+}
+
+// derived constants of every parameter row into the stream's constant slot, ahead of the kernel that reads them
+static int prep_constants(const float* params, int pstride, int N, const ChainDesc& d, cudaStream_t st, int* slot) {
+  float* cbase = cpar_device_ptr();
+  RISP_REQUIRE(cbase, RISP_E_CUDA, "fused pipeline: cannot resolve the constant parameter block");
+  *slot = slot_of(st);
+  fused_prep_kernel<<<pstride ? N : 1, 32, 0, st>>>(params, pstride, d, cbase + (size_t)*slot * kCRows * kCRowFloats);
+  return check_launch("fused_prep_kernel");
 }
 
 }  // namespace fused
@@ -1155,12 +1075,10 @@ bool fused_handles(const ChainDesc& d, int N, int param_stride, int H, int W) {
 }
 
 // partial rows the step / backward kernels write: [N][rows_per_frame][RISP_NSLOT]
-int fused_partial_rows_per_frame(int N, int H, int W) {
+int fused_partial_rows_per_frame(int N) {
   // the largest grid any instantiation may use: 32 resident CTAs per SM is the hardware bound
   int slots = sm_count() * 32;
-  int cpf = slots / N < 1 ? 1 : slots / N;
-  (void)H; (void)W;
-  return cpf * fused::kWarps;
+  return slots / N < 1 ? 1 : slots / N;
 }
 
 // evaluation mode: inference arithmetic, squared 8-bit code differences to gt -> partial[N][*rows_per_frame], optional 8-bit
@@ -1170,47 +1088,29 @@ int fused_eval_launch(const float* raw, const float* gt, unsigned char* u8, unsi
                       int* rows_per_frame) {
   using namespace fused;
   if (!fused_handles(d, N, pstride, H, W)) return 1;
-  float* cbase = cpar_device_ptr();
-  RISP_REQUIRE(cbase, RISP_E_CUDA, "fused pipeline: cannot resolve the constant parameter block");
-  const int slot = slot_of(st);
-  fused_prep_kernel<<<pstride ? N : 1, 32, 0, st>>>(params, pstride, d, cbase + (size_t)slot * kCRows * kCRowFloats);
-  int rc = check_launch("fused_prep_kernel");
+  int slot;
+  const int rc = prep_constants(params, pstride, N, d, st, &slot);
   if (rc != RISP_OK) return rc;
-  FusedArgs a{raw, gt, nullptr, nullptr, params, pstride, H, W, 0, 0, 0, 0, clip_hi, slot, 0, u8, partial};
-  const unsigned sig = chain_signature(d);
-  Geometry g;
-  rc = dispatch<MODE_EVAL>(a, d, sig, N, dm_kind, st, &g);
-  if (rc != RISP_OK) return rc;
-  *rows_per_frame = g.cpf * kWarps;
-  return dispatch<MODE_EVAL>(a, d, sig, N, dm_kind, st, nullptr);
+  const FusedArgs a{raw, gt, nullptr, nullptr, params, pstride, H, W, 0, 0, 0, 0, clip_hi, slot, u8, partial};
+  return dispatch<MODE_EVAL>(a, d, N, dm_kind, st, rows_per_frame);
 }
 
 // mode: 0 forward, 1 MSE step, 2 backward with upstream dy, 3 L1 step.  Returns RISP_OK, an error, or 1 when the chain is not handled.
-// *rows_per_frame receives the number of partial rows per frame actually written (modes 1, 2).
+// *rows_per_frame (nullable) receives the number of partial rows per frame actually written (modes 1-3).
 int fused_launch(int mode, const float* raw, const float* gt, float* y, float* partial, const float* params, int pstride,
                  int N, int H, int W, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st, int* rows_per_frame) {
   using namespace fused;
   if (!fused_handles(d, N, pstride, H, W)) return 1;
-  float* cbase = cpar_device_ptr();
-  RISP_REQUIRE(cbase, RISP_E_CUDA, "fused pipeline: cannot resolve the constant parameter block");
-  const int slot = slot_of(st);
-  const int rows = pstride ? N : 1;
-  fused_prep_kernel<<<rows, 32, 0, st>>>(params, pstride, d, cbase + (size_t)slot * kCRows * kCRowFloats);
-  int rc = check_launch("fused_prep_kernel");
+  int slot;
+  const int rc = prep_constants(params, pstride, N, d, st, &slot);
   if (rc != RISP_OK) return rc;
-  static const int dbg = getenv("RISP_FUSED_DBG") ? atoi(getenv("RISP_FUSED_DBG")) : 0;
-  FusedArgs a{raw, gt, y, partial, params, pstride, H, W, 0, 0, 0, 0, clip_hi, slot, dbg};
-  const unsigned sig = chain_signature(d);
-  Geometry g;
-  if (mode == 0) return dispatch<MODE_FWD>(a, d, sig, N, dm_kind, st, nullptr);
-  auto go = [&](Geometry* gp) {
-    return (mode == 1) ? dispatch<MODE_STEP>(a, d, sig, N, dm_kind, st, gp)
-         : (mode == 3) ? dispatch<MODE_STEP_L1>(a, d, sig, N, dm_kind, st, gp) : dispatch<MODE_BWD>(a, d, sig, N, dm_kind, st, gp);
-  };
-  rc = go(&g);
-  if (rc != RISP_OK) return rc;
-  if (rows_per_frame) *rows_per_frame = g.cpf * kWarps;
-  return go(nullptr);
+  const FusedArgs a{raw, gt, y, partial, params, pstride, H, W, 0, 0, 0, 0, clip_hi, slot};
+  switch (mode) {
+    case 0: return dispatch<MODE_FWD>(a, d, N, dm_kind, st, rows_per_frame);
+    case 1: return dispatch<MODE_STEP>(a, d, N, dm_kind, st, rows_per_frame);
+    case 3: return dispatch<MODE_STEP_L1>(a, d, N, dm_kind, st, rows_per_frame);
+    default: return dispatch<MODE_BWD>(a, d, N, dm_kind, st, rows_per_frame);
+  }
 }
 
 }  // namespace risp

@@ -106,38 +106,15 @@ __device__ __forceinline__ float2 zero2() { return make_float2(0.f, 0.f); }
 // scalar FFMA it replaces (profiles/r3_fma_rates.txt, cycles per warp instruction: FFMA2 R,R,R 4.3 against FFMA R,R,R 1.6;
 // FFMA2 with a uniform coefficient pair 2.9 against FFMA with a coefficient 0.9-1.1).  So the sites below use scalar
 // instructions in the backward-carrying kernels of chains with the 3x10 polynomial (the FMA-bound ones; template flag SC
-// where a helper also serves other chains); each -DRISP_FUSED_PACKED_* switch restores the packed form of one site
-// (per-site step times on the B200: profiles/r3_ablation.txt -- every site is faster scalar).  The gamma -> tone curve
-// step is memory-bound and keeps the packed forms: with them scalar it took 0.1600 instead of 0.1555 ms per 48 MP.
+// where a helper also serves other chains): the polynomial rows of the channel-major step (FFMA R,UR,R), the loss residual
+// y - t and its sum, and the folded accumulators below (polynomial gradient sums, tone-curve hinge sums, gamma exponent
+// sum).  Per-site step times on the B200 with each site packed instead: profiles/r3_ablation.txt -- every site is faster
+// scalar.  The gamma -> tone curve step is memory-bound and keeps the packed forms: with them scalar it took 0.1600 instead
+// of 0.1555 ms per 48 MP.
 //   * folded accumulators: both pixels of a pair go into ONE sum, acc.x = fma(u.y, v.y, fma(u.x, v.x, acc.x)); acc.y stays
 //     the constant 0 (no register), and the epilogue's acc.x + acc.y reduces it unchanged -- the summation order is still
 //     fixed, gradients stay bit-reproducible run to run.  Half the accumulator registers: the 37-parameter step kernel
 //     fits 168 registers, three one-warp CTAs per SM sub-partition instead of two.
-#ifndef RISP_FUSED_PACKED_POLY_FWD
-constexpr bool kScalarPolyFwd = true;    // polynomial rows of the channel-major step: FFMA R,UR,R
-#else
-constexpr bool kScalarPolyFwd = false;
-#endif
-#ifndef RISP_FUSED_PACKED_S_ACC
-constexpr bool kFoldS = true;            // polynomial gradient sums S[c][i] += e_c phi_i
-#else
-constexpr bool kFoldS = false;
-#endif
-#ifndef RISP_FUSED_PACKED_GTM_ACC
-constexpr bool kFoldGtm = true;          // tone-curve hinge sums A_k
-#else
-constexpr bool kFoldGtm = false;
-#endif
-#ifndef RISP_FUSED_PACKED_GAMMA_ACC
-constexpr bool kFoldGamma = true;        // gamma exponent sum
-#else
-constexpr bool kFoldGamma = false;
-#endif
-#ifndef RISP_FUSED_PACKED_LOSS
-constexpr bool kScalarLoss = true;       // loss residual y - t and its sum
-#else
-constexpr bool kScalarLoss = false;
-#endif
 template <bool FOLD>
 __device__ __forceinline__ void acc_fma(float2& acc, float2 u, float2 v) {     // acc += u * v
   if constexpr (FOLD) acc.x = fmaf(u.y, v.y, fmaf(u.x, v.x, acc.x));
@@ -152,27 +129,16 @@ __device__ __forceinline__ void acc_add(float2& acc, float2 u) {               /
 // ---- stage state kept from the forward sweep for the backward sweep --------------------------------------------
 struct GammaSaved { P2 x, l2, y; };
 struct PolySaved { float2 phi[9]; P2 u, y; };     // phi = b2 g2 r2 bg br gr b g r  (coefficient order of WbQuadratic)
-struct GainSaved { P2 x; };
-struct GtmSaved { P2 x; float2 hd[3][3]; P2 m; };  // hd[c][k] = x_c - x_{k+1};  m = final-clamp mask (slow path only)
 
 // ---- gamma: y = clamp(x, eps, 1)^gm ------------------------------------------------------------------------------
-// RFORM (the stage's input gradient is needed): y = xc * r with r = xc^(gm-1) = ex2((gm-1) lg2 xc).  The backward sweep then
-// has d y / d x = gm r without the reciprocal of the plain form (t / x): 2 MUFU per pixel and channel instead of 3.  Opt-in
-// (-DRISP_FUSED_RFORM): on the B200 the step kernel got 2 % SLOWER with it (0.294 -> 0.300 ms per 48 MP).
-template <bool IN01, bool RFORM = false>
-__device__ __forceinline__ float2 gamma_fwd2(float2 x, float gm, float2& l2, float gm1 = 0.f, float2* r = nullptr) {
+template <bool IN01>
+__device__ __forceinline__ float2 gamma_fwd2(float2 x, float gm, float2& l2) {
   float2 xc;
   xc.x = IN01 ? fmaxf(x.x, RISP_GAMMA_EPS) : fminf(fmaxf(x.x, RISP_GAMMA_EPS), 1.f);
   xc.y = IN01 ? fmaxf(x.y, RISP_GAMMA_EPS) : fminf(fmaxf(x.y, RISP_GAMMA_EPS), 1.f);
   l2 = make_float2(lg2_ftz(xc.x), lg2_ftz(xc.y));
-  if constexpr (RFORM) {
-    const float2 t = mul2s(l2, gm1);
-    *r = make_float2(ex2_ftz(t.x), ex2_ftz(t.y));
-    return mul2(*r, xc);
-  } else {
-    const float2 t = mul2s(l2, gm);
-    return make_float2(ex2_ftz(t.x), ex2_ftz(t.y));
-  }
+  const float2 t = mul2s(l2, gm);
+  return make_float2(ex2_ftz(t.x), ex2_ftz(t.y));
 }
 template <bool IN01>
 __device__ __forceinline__ P2 gamma_fwd(const P2& x, float gm, GammaSaved& sv) {
@@ -184,12 +150,12 @@ __device__ __forceinline__ P2 gamma_fwd(const P2& x, float gm, GammaSaved& sv) {
 // d <- dL/dx (WITHOUT the factor gm when DEFER: the caller multiplies the upstream accumulators once at the end);
 // acc += d*y*lg2(xc)  (ln 2 applied in the epilogue).  rcp(x) may be inf/NaN where the mask is 0: selected away.
 // NOMASK: the caller applies the clamp mask itself (merged with the mask of the stage in front), so v is returned as is.
-template <bool IN01, bool NEED_DX, bool DEFER, bool NOMASK = false, bool RFORM = false, bool SC = true>
-__device__ __forceinline__ float2 gamma_bwd2(float2 x, float2 y, float2 l2, float2 d, float gm, float2& acc, float2 r = float2()) {
+template <bool IN01, bool NEED_DX, bool DEFER, bool NOMASK = false, bool SC = true>
+__device__ __forceinline__ float2 gamma_bwd2(float2 x, float2 y, float2 l2, float2 d, float gm, float2& acc) {
   const float2 t = mul2(d, y);
-  acc_fma<kFoldGamma && SC>(acc, t, l2);
+  acc_fma<SC>(acc, t, l2);
   if (!NEED_DX) return zero2();
-  float2 v = RFORM ? mul2(d, r) : mul2(t, make_float2(rcp_ftz(x.x), rcp_ftz(x.y)));
+  float2 v = mul2(t, make_float2(rcp_ftz(x.x), rcp_ftz(x.y)));
   if (!DEFER) v = mul2s(v, gm);
   if (NOMASK) return v;
   const bool mx = IN01 ? (x.x >= RISP_GAMMA_EPS) : (x.x >= RISP_GAMMA_EPS && x.x <= 1.f);
@@ -205,20 +171,11 @@ __device__ __forceinline__ P2 gamma_bwd(const GammaSaved& sv, const P2& d, float
   return o;
 }
 
-// ---- diagonal gain ---------------------------------------------------------------------------------------------------
-__device__ __forceinline__ P2 gain_fwd(const P2& x, const float* g, GainSaved& sv) {
-  sv.x = x;
+// ---- diagonal gain (the backward-carrying kernels run it per channel in risp_fused.cu's Tail) --------------------------
+__device__ __forceinline__ P2 gain_fwd(const P2& x, const float* g) {
   P2 y;
   y.b = mul2s(x.b, g[0]); y.g = mul2s(x.g, g[1]); y.r = mul2s(x.r, g[2]);
   return y;
-}
-template <bool NEED_DX>
-__device__ __forceinline__ P2 gain_bwd(const GainSaved& sv, const P2& d, const float* g, float2* acc) {
-  acc[0] = fma2(d.b, sv.x.b, acc[0]); acc[1] = fma2(d.g, sv.x.g, acc[1]); acc[2] = fma2(d.r, sv.x.r, acc[2]);
-  P2 o;
-  if (NEED_DX) { o.b = mul2s(d.b, g[0]); o.g = mul2s(d.g, g[1]); o.r = mul2s(d.r, g[2]); }
-  else { o.b = zero2(); o.g = zero2(); o.r = zero2(); }
-  return o;
 }
 
 // ---- 3x10 polynomial: u_c = sum_i q[c][i] phi_i, y = clamp(u, 0, 1) ----------------------------------------------------
@@ -249,8 +206,8 @@ __device__ __forceinline__ P2 poly_bwd(const PolySaved& sv, const P2& d, const f
 #pragma unroll
   for (int c = 0; c < 3; ++c) {
 #pragma unroll
-    for (int i = 0; i < 9; ++i) acc_fma<kFoldS>(acc[c * 10 + i], e[c], sv.phi[i]);
-    acc_add<kFoldS>(acc[c * 10 + 9], e[c]);
+    for (int i = 0; i < 9; ++i) acc_fma<true>(acc[c * 10 + i], e[c], sv.phi[i]);
+    acc_add<true>(acc[c * 10 + 9], e[c]);
   }
   P2 o;
   if (NEED_DX) {
@@ -272,21 +229,16 @@ __device__ __forceinline__ P2 poly_bwd(const PolySaved& sv, const P2& d, const f
 // ---- 4-segment tone curve, input in [0,1] ------------------------------------------------------------------------
 // Reference: tools_origin.py:429-435, out = (x - x_k) * slope_k + y_k on the half-open segment [x_k, x_k+1), x_k = k/4;
 // x == 1 lies in no segment: the pass-through pixel (out = 1, slope 1, no knot gradient).
-// constant block: s0, ds1, ds2, ds3, (1 - s3), slow flag, -, -, a_0..a_3, s_0..s_3   (a_k = y_k - x_k s_k)
+// constant block: s0, ds1, ds2, ds3, -, slow flag, -, -, a_0..a_3, s_0..s_3   (a_k = y_k - x_k s_k)
 //
-// Table form (default): the segment of a pixel is looked up instead of being rebuilt from three hinges and four step
-// masks.  FFMA.RZ(x, 4, 2^20) leaves floor(4x) in bits 3..5 of the sum (ulp 1/8), LOP3 turns that into the address of an
-// 8-byte entry (a_k, s_k) of a 64-byte table in shared memory (entry 4: x == 1 -> pass-through; entry 7: NaN -> NaN),
+// Table form (backward-carrying kernels): the segment of a pixel is looked up instead of being rebuilt from three hinges and
+// four step masks.  FFMA.RZ(x, 4, 2^20) leaves floor(4x) in bits 3..5 of the sum (ulp 1/8), LOP3 turns that into the address
+// of an 8-byte entry (a_k, s_k) of a 64-byte table in shared memory (entry 4: x == 1 -> pass-through; entry 7: NaN -> NaN),
 // one LDS.64 fetches it:  out = s_k x + a_k,  d out / d x = s_k.  3 + 1 instructions per pixel and channel instead of
 // 1.5 FADD2 + 3 FMNMX + 2 FFMA2 (forward) and 4 FSET + 2 FFMA2 (slope).  The knot gradients still come from the hinge sums
-// A_0 = sum d x, A_k = sum d max(x - x_k, 0), the hinge being ONE saturating add (x - x_k < 1: the upper clamp never acts).
+// A_0 = sum d x, A_k = sum d max(x - x_k, 0).
 // The inference kernels keep the hinge form: they are bound by the memory system, and the dependent LDS in the middle of
 // every pixel's chain costs them 4 % (measured); the backward-carrying kernels are bound by instruction issue.
-#ifndef RISP_FUSED_NO_GTM_TABLE
-constexpr bool kGtmTable = true;
-#else
-constexpr bool kGtmTable = false;
-#endif
 constexpr int kGtmTableBytes = 64;
 __device__ __forceinline__ float2 gtm_lookup(float x, uint32_t tbl) {     // tbl: 64-byte aligned shared address
   const uint32_t bits = __float_as_uint(__fmaf_rz(x, 4.f, 1048576.f));
@@ -303,17 +255,16 @@ __device__ __forceinline__ void gtm_table_fill(uint32_t tbl, const float* c) {
     asm volatile("st.shared.v2.f32 [%0], {%1,%2};" ::"r"(tbl + 8u * k), "f"(a), "f"(s) : "memory");
   }
 }
-template <bool TABLE>
-__device__ __forceinline__ float2 gtm_hinge(float2 x, float2 hd, float xk) {
-  if constexpr (TABLE) return make_float2(__saturatef(x.x - xk), __saturatef(x.y - xk));
-  else return make_float2(fmaxf(hd.x, 0.f), fmaxf(hd.y, 0.f));
+// max(x - x_k, 0) as ONE saturating add (x - x_k < 1: the upper clamp never acts)
+__device__ __forceinline__ float2 gtm_hinge(float2 x, float xk) {
+  return make_float2(__saturatef(x.x - xk), __saturatef(x.y - xk));
 }
-// sv: state for the backward sweep -- table form: sv[0] = slope of the pixel's segment; hinge form: sv[k] = x - x_{k+1}
+// slope: table form only -- the slope of the pixel's segment, for the backward sweep
 template <bool TABLE>
-__device__ __forceinline__ float2 gtm_fwd2(float2 x, const float* c, float2 (&sv)[3], bool slow, float2& mask, uint32_t tbl) {
+__device__ __forceinline__ float2 gtm_fwd2(float2 x, const float* c, float2& slope, bool slow, float2& mask, uint32_t tbl) {
  if constexpr (TABLE) {
   const float2 e0 = gtm_lookup(x.x, tbl), e1 = gtm_lookup(x.y, tbl);
-  sv[0] = make_float2(e0.y, e1.y);
+  slope = make_float2(e0.y, e1.y);
   float2 y;
   if (!slow) {
     y.x = __saturatef(fmaf(e0.y, x.x, e0.x)); y.y = __saturatef(fmaf(e1.y, x.y, e1.x));
@@ -324,18 +275,10 @@ __device__ __forceinline__ float2 gtm_fwd2(float2 x, const float* c, float2 (&sv
   }
  return y;
  } else {
-  float2 (&hd)[3] = sv;
-  hd[0] = add2s(x, -0.25f); hd[1] = add2s(x, -0.5f); hd[2] = add2s(x, -0.75f);
   float2 f = mul2s(x, c[0]);
-  // hinge as ONE saturating add (x - x_k < 1): -DRISP_FUSED_FWD_MAXHINGE restores the packed add + FMNMX form
-#ifndef RISP_FUSED_FWD_MAXHINGE
-  constexpr bool SATH = true;
-#else
-  constexpr bool SATH = false;
-#endif
-  f = fma2s(c[1], gtm_hinge<SATH>(x, hd[0], 0.25f), f);
-  f = fma2s(c[2], gtm_hinge<SATH>(x, hd[1], 0.5f), f);
-  const float2 h3 = gtm_hinge<SATH>(x, hd[2], 0.75f);
+  f = fma2s(c[1], gtm_hinge(x, 0.25f), f);
+  f = fma2s(c[2], gtm_hinge(x, 0.5f), f);
+  const float2 h3 = gtm_hinge(x, 0.75f);
   float2 y;
   if (!slow) {
     y.x = __saturatef(fmaf(c[3], h3.x, f.x)); y.y = __saturatef(fmaf(c[3], h3.y, f.y));
@@ -347,46 +290,24 @@ __device__ __forceinline__ float2 gtm_fwd2(float2 x, const float* c, float2 (&sv
   return y;
  }
 }
-template <bool TABLE>
-__device__ __forceinline__ P2 gtm_fwd(const P2& x, const float* c, GtmSaved& sv, bool slow, uint32_t tbl) {
-  sv.x = x;
+// inference kernels: hinge form, nothing kept for a backward sweep
+__device__ __forceinline__ P2 gtm_fwd(const P2& x, const float* c, bool slow) {
+  float2 slope, mask;
   P2 y;
-  y.b = gtm_fwd2<TABLE>(x.b, c, sv.hd[0], slow, sv.m.b, tbl); y.g = gtm_fwd2<TABLE>(x.g, c, sv.hd[1], slow, sv.m.g, tbl);
-  y.r = gtm_fwd2<TABLE>(x.r, c, sv.hd[2], slow, sv.m.r, tbl);
+  y.b = gtm_fwd2<false>(x.b, c, slope, slow, mask, 0u); y.g = gtm_fwd2<false>(x.g, c, slope, slow, mask, 0u);
+  y.r = gtm_fwd2<false>(x.r, c, slope, slow, mask, 0u);
   return y;
 }
 // accumulates A_0 = sum d x, A_k = sum d max(x - x_k, 0); the knot gradients are the second differences
 // 4 (A_{j-1} - 2 A_j + A_{j+1}) (hat basis = second difference of hinges; A_4 = 0 on [0,1]), formed in the epilogue.
+// slope: from the table form of gtm_fwd2
 template <bool NEED_DX, bool SC = true>
-__device__ __forceinline__ float2 gtm_bwd2(float2 x, const float2 (&sv)[3], float2 d, const float* c, float2* acc) {
-  acc_fma<kFoldGtm && SC>(acc[0], d, x);
- if constexpr (kGtmTable) {
+__device__ __forceinline__ float2 gtm_bwd2(float2 x, float2 slope, float2 d, float2* acc) {
+  acc_fma<SC>(acc[0], d, x);
 #pragma unroll
-  for (int k = 0; k < 3; ++k) acc_fma<kFoldGtm && SC>(acc[k + 1], d, gtm_hinge<true>(x, x, 0.25f * (float)(k + 1)));
+  for (int k = 0; k < 3; ++k) acc_fma<SC>(acc[k + 1], d, gtm_hinge(x, 0.25f * (float)(k + 1)));
   if (!NEED_DX) return zero2();
-  return mul2(d, sv[0]);
- } else {
-  const float2 (&hd)[3] = sv;
-  float2 slope = make_float2(c[0], c[0]);
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    const float2 st = make_float2(hd[k].x >= 0.f ? 1.f : 0.f, hd[k].y >= 0.f ? 1.f : 0.f);
-    acc_fma<kFoldGtm && SC>(acc[k + 1], d, gtm_hinge<false>(x, hd[k], 0.f));
-    if (NEED_DX) slope = fma2s(c[k + 1], st, slope);
-  }
-  if (!NEED_DX) return zero2();
-  slope = fma2s(c[4], make_float2(x.x >= 1.f ? 1.f : 0.f, x.y >= 1.f ? 1.f : 0.f), slope);   // x == 1: slope -> 1
   return mul2(d, slope);
- }
-}
-template <bool NEED_DX>
-__device__ __forceinline__ P2 gtm_bwd(const GtmSaved& sv, const P2& d0, const float* c, float2* acc, bool slow) {
-  P2 d = d0;
-  if (slow) { d.b = mul2(d.b, sv.m.b); d.g = mul2(d.g, sv.m.g); d.r = mul2(d.r, sv.m.r); }
-  P2 o;
-  o.b = gtm_bwd2<NEED_DX>(sv.x.b, sv.hd[0], d.b, c, acc); o.g = gtm_bwd2<NEED_DX>(sv.x.g, sv.hd[1], d.g, c, acc);
-  o.r = gtm_bwd2<NEED_DX>(sv.x.r, sv.hd[2], d.r, c, acc);
-  return o;
 }
 #endif  // __CUDACC__
 

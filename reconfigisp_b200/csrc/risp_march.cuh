@@ -65,10 +65,8 @@ __device__ __forceinline__ void row_finish(float (&dst)[4 + 2 * HL], const Row<H
 }
 
 // F: struct with  __device__ void operator()(const float (&w)[NP][2*HL+1][4+2*HL], float (&out)[NP][4], int zp) const
-#ifndef RISP_MARCH_DEPTH
-#define RISP_MARCH_DEPTH 3
-#endif
-template <int HL, int NP, int BORDER, class F, int D = RISP_MARCH_DEPTH>
+constexpr int kMarchDepth = 3;
+template <int HL, int NP, int BORDER, class F, int D = kMarchDepth>
 __global__ void __launch_bounds__(kWarps * 32)
 march_kernel(const float* __restrict__ x, float* __restrict__ y, int H, int W, int rows_per_chunk, F f) {
   constexpr int WR = 2 * HL + 1, WC = 4 + 2 * HL;

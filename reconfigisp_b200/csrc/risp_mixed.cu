@@ -84,10 +84,7 @@ __device__ __forceinline__ float4 ld_stream4_if(const float* p, bool on) {
   return v;
 }
 constexpr int kExtBatch = 3;     // materialised candidates loaded together (3 planes x 128 bit each = 36 registers)
-#ifndef RISP_MIX_FWD_BATCH
-#define RISP_MIX_FWD_BATCH 4
-#endif
-constexpr int kExtBatchFwd = RISP_MIX_FWD_BATCH;  // measured: 1 CTA/SM with 4 candidates in flight beats 2 CTAs with 2 (0.58 vs 0.44 of HBM peak)
+constexpr int kExtBatchFwd = 4;  // measured: 1 CTA/SM with 4 candidates in flight beats 2 CTAs with 2 (0.58 vs 0.44 of HBM peak)
 
 // load / store one pixel group of a C-plane image (C = 1 or 3; missing planes read as 0)
 template <int VEC>
@@ -129,11 +126,8 @@ __device__ __forceinline__ void mix_store(const Px<MixNpx<VEC>::value>& px, floa
   }
 }
 
-#ifndef RISP_MIX_FWD_MINB
-#define RISP_MIX_FWD_MINB 1
-#endif
 template <int VEC, unsigned SIG>
-__global__ void __launch_bounds__(kT, RISP_MIX_FWD_MINB)
+__global__ void __launch_bounds__(kT, 1)
 mixed_fwd_kernel(const float* __restrict__ x, float* __restrict__ y, long long HW, int C, MixDesc d,
                  const float* __restrict__ params, int pstride, const float* __restrict__ w) {
   constexpr int NPX = MixNpx<VEC>::value;

@@ -123,7 +123,7 @@ enum { MODE_FWD = 0, MODE_STEP = 1, MODE_EVAL = 2 };
 
 // packed-fp32 / constant-bank kernels for the pre-instantiated signatures (risp_fused.cu)
 bool fused_handles(const ChainDesc& d, int N, int param_stride, int H, int W);
-int fused_partial_rows_per_frame(int N, int H, int W);
+int fused_partial_rows_per_frame(int N);
 int fused_launch(int mode, const float* raw, const float* gt, float* y, float* partial, const float* params, int pstride,
                  int N, int H, int W, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st, int* rows_per_frame);
 int fused_eval_launch(const float* raw, const float* gt, unsigned char* u8, unsigned long long* partial, const float* params,
@@ -144,25 +144,17 @@ struct PipeArgs {
   unsigned long long* sse;   // MODE_EVAL: [N][warps_per_image] sums of squared code differences
 };
 
-#ifndef RISP_STEP_MINB
-#define RISP_STEP_MINB 2   // resident CTAs per SM the backward-carrying kernels are compiled for (register cap)
-#endif
-#ifndef RISP_PAIR_UNROLL
-#define RISP_PAIR_UNROLL 2
-#endif
-#ifndef RISP_FWD_MINB
-#define RISP_FWD_MINB 4
-#endif
-#ifndef RISP_EVAL_MINB
-#define RISP_EVAL_MINB 3   // the forward's registers plus the GT row in flight: 4 CTAs (128 registers) spill
-#endif
-#ifndef RISP_FWD_PREFETCH
-#define RISP_FWD_PREFETCH 1   // raw rows in flight per warp in the forward-only kernel.  Measured on B200 (12 MP x 4,
-#endif                        // bilinear + 4 stages): depth 2 = 0.242 ms vs depth 1 = 0.234 ms -- not latency-bound
+// resident CTAs per SM the kernels are compiled for (register cap)
+constexpr int kStepMinBlocks = 2;   // backward-carrying kernels of the pre-instantiated signatures (the generic one: 1)
+constexpr int kFwdMinBlocks = 4;
+constexpr int kEvalMinBlocks = 3;   // the forward's registers plus the GT row in flight: 4 CTAs (128 registers) spill
+constexpr int kPairUnroll = 2;
+// One raw row in flight per warp in the forward-only kernel: measured on B200 (12 MP x 4, bilinear + 4 stages), two rows
+// took 0.242 ms against 0.234 ms for one -- the kernel is not latency-bound.
 
 template <int DM, int MODE, unsigned SIG, bool BIGG>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, (MODE == 1 /*MODE_STEP*/) ? ((SIG == 0) ? 1 : RISP_STEP_MINB)
-                                                    : (MODE == 2 /*MODE_EVAL*/) ? RISP_EVAL_MINB : RISP_FWD_MINB)
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, (MODE == MODE_STEP) ? ((SIG == 0) ? 1 : kStepMinBlocks)
+                                                    : (MODE == MODE_EVAL) ? kEvalMinBlocks : kFwdMinBlocks)
 pipeline_kernel(PipeArgs a, ChainDesc d) {
   using SG = Sig<SIG>;
   constexpr int SMAX = SG::S;
@@ -179,8 +171,7 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
   const int rb = min(H, ra + a.rows_per_chunk);
   const long long plane = (long long)H * W;
   const float* __restrict__ img = a.raw + (long long)n * plane;
-  const float* __restrict__ prow_inv = a.params + (long long)n * a.pstride;
-  const float* __restrict__ prow = prow_inv;
+  const float* __restrict__ prow = a.params + (long long)n * a.pstride;
   const float* __restrict__ gtb = (MODE != MODE_FWD) ? a.gt + (long long)n * 3 * plane : nullptr;
   float* __restrict__ yb = a.y ? a.y + (long long)n * 3 * plane : nullptr;
 
@@ -206,9 +197,6 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
       row_finish<HL>(w[j], q, W, c0, active, lane);
     }
     row_issue<HL>(q, img, reflect101(ra + HL, H), W, c0, active, lane);
-    constexpr bool kDeep = (MODE == MODE_FWD) && (RISP_FWD_PREFETCH >= 2);
-    RawRow<HL> q2;
-    if (kDeep && ra + 1 < rb) row_issue<HL>(q2, img, reflect101(ra + 1 + HL, H), W, c0, active, lane);
     float4 gB = make_float4(0.f, 0.f, 0.f, 0.f), gG = gB, gR = gB;   // GT of the row being computed, fetched one row ahead
     if (MODE == MODE_STEP && active) {
       const long long o = (long long)ra * W + c0;
@@ -226,10 +214,7 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
           eB = ld_stream4(gtb + o); eG = ld_stream4(gtb + plane + o); eR = ld_stream4(gtb + 2 * plane + o);
         }
       }
-      if (kDeep) {
-        q = q2;                                                     // row r+1 (already in flight) becomes current
-        if (r + 2 < rb) row_issue<HL>(q2, img, reflect101(r + 2 + HL, H), W, c0, active, lane);
-      } else if (r + 1 < rb) {
+      if (r + 1 < rb) {
         row_issue<HL>(q, img, reflect101(r + 1 + HL, H), W, c0, active, lane);
         if (MODE == MODE_STEP && active) {
           const long long o = (long long)(r + 1) * W + c0;
@@ -266,7 +251,6 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
         // occupancy of this kernel).  The pair is selected with a warp-uniform predicate, not an index.
         const float gtB[4] = {tB.x, tB.y, tB.z, tB.w}, gtG[4] = {tG.x, tG.y, tG.z, tG.w},
                     gtR[4] = {tR.x, tR.y, tR.z, tR.w};
-constexpr int kPairUnroll = RISP_PAIR_UNROLL;
 #pragma unroll kPairUnroll
         for (int h = 0; h < 2; ++h) {
           const bool hi = (h != 0);
@@ -457,7 +441,7 @@ extern "C" int risp_demosaic_fwd(const float* raw, float* bgr, int N, int H, int
 extern "C" size_t risp_pipeline_eval_workspace(int N, int H, int W) {
   if (N <= 0 || H <= 0 || W <= 0) return 0;
   size_t rows = (size_t)pipe_geometry(N, H, W).warps_per_image;
-  const size_t frows = (size_t)fused_partial_rows_per_frame(N, H, W);
+  const size_t frows = (size_t)fused_partial_rows_per_frame(N);
   if (frows > rows) rows = frows;
   return (size_t)N * rows * sizeof(unsigned long long);
 }
@@ -510,7 +494,7 @@ extern "C" size_t risp_pipeline_step_workspace(int N, int H, int W, int P) {
   if (N <= 0 || H <= 0 || W <= 0) return 0;
   PipeGeom g = pipe_geometry(N, H, W);
   size_t rows = (size_t)g.warps_per_image;
-  const size_t frows = (size_t)fused_partial_rows_per_frame(N, H, W);
+  const size_t frows = (size_t)fused_partial_rows_per_frame(N);
   if (frows > rows) rows = frows;
   return (size_t)N * rows * RISP_NSLOT * sizeof(float) + finalize_rows_workspace(N, RISP_NSLOT);
 }

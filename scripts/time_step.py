@@ -1,7 +1,7 @@
 """CUDA-event time of the fused step alone on bench.py's tuning workload: 4 x 12 MP, bilinear demosaic, the chain of
 Bayer_02_Demosaic_02_sRGB_11_13_01_14 (gain -> 3x10 polynomial -> gamma -> tone curve), through ops.PipelineStep
-(coefficient preparation + step kernel + finaliser).  The library is the one RISP_LIB_PATH names, so builds with
-different compile-time switches can be compared in one session:
+(coefficient preparation + step kernel + finaliser).  The library is the one RISP_LIB_PATH names, so different builds,
+e.g. the parent commit's, can be compared in one session:
 
     RISP_LIB_PATH=build/abl/<variant>.so python scripts/time_step.py [launches=200] [repeats=5] [width=4000]
 
