@@ -120,6 +120,39 @@ def gtm_manual(x, params, n_seg=4):
     return torch.clamp(out, 0.0, 1.0)
 
 
+def gain_clip(x, gain):
+    """EXTENSION.  y_c = clamp(x_c * gain_c, 0, 1), gain (N,3)."""
+    return torch.clamp(wb_manual(x, gain), 0.0, 1.0)
+
+
+def pixel_chain(x, stages, p):
+    """A fused per-pixel chain (the stage list of `ops.Chain`) with KERNEL-level parameter rows p (N,P) or (1,P), packed
+    in stage order: gain / gain_clip (3 gains), poly10 (the 30 coefficients P[c][k] themselves, not the [0,1] logits of
+    wb_quadratic), gamma (1), (gtm, n) (n-1 knots, each image's own row: no batch-element-0 quirk), ccm (9), skip (0).
+    Runs in the dtype of x; the tests call it in float64 on the kernels' fp32 inputs."""
+    N = x.shape[0]
+    p = p.expand(N, -1)
+    o = 0
+    for s in stages:
+        name, iarg = (s, 0) if isinstance(s, str) else s
+        if name == 'gain':
+            x = wb_manual(x, p[:, o:o + 3]); o += 3
+        elif name == 'gain_clip':
+            x = gain_clip(x, p[:, o:o + 3]); o += 3
+        elif name == 'poly10':
+            x = wb_quadratic(x, (p[:, o:o + 30] + 5) / 10); o += 30
+        elif name == 'gamma':
+            x = gamma_manual(x, p[:, o:o + 1]); o += 1
+        elif name == 'gtm':
+            x = torch.cat([gtm_manual(x[i:i + 1], p[i:i + 1, o:o + iarg - 1], iarg) for i in range(N)]); o += iarg - 1
+        elif name == 'ccm':
+            x = ccm(x, p[:, o:o + 9]); o += 9
+        elif name != 'skip':
+            raise ValueError('pixel_chain: no reference for stage %r' % name)
+    assert o == p.shape[1], (o, p.shape)
+    return x
+
+
 def _lum(x):
     return 0.114 * x[:, 0] + 0.587 * x[:, 1] + 0.299 * x[:, 2]
 
