@@ -132,6 +132,19 @@ int risp_decode_codes(const void* src, float* dst, long long n, int bytes_per_co
  * y0, x0 must be even for a Bayer plane (CFA phase); checked when require_even != 0. */
 int risp_crop_decode(const void* src, float* dst, int planes, int H, int W, int y0, int x0, int h, int w,
                      int bytes_per_code, float denom, int require_even, risp_stream_t stream);
+/* Batched crop + decode from a frame store in HBM: a whole training batch in one launch, the same kernel and division as
+ * risp_crop_decode (bit-identical to it and to risp_decode_codes).
+ *   raw_store: (F,H,W) unsigned codes of raw_bytes_per_code (1 or 2) bytes.  gt_store: (G,3,H,W) uint8 BGR planes.
+ *   pos: DEVICE int32 [B][4] = (raw frame, gt frame, y0, x0), 16-byte aligned; y0 and x0 must be even (CFA phase).
+ *   img_out: (B,1,h,w) fp32 = code / white_level.  gt_out: (B,3,h,w) fp32 = code / 255, nullable (then gt_store and G
+ *   are not used).
+ *   status: DEVICE int32[1]; set to non-zero when a record names a frame outside the store, is odd, or puts the crop
+ *   outside the frame.  That record is skipped (its outputs are left as they were); nothing outside the stores is read.
+ *   Nothing here reads status or waits for the device: the caller checks it when it chooses to.
+ * B * 4 (B without gt_out) must not exceed 65535. */
+int risp_sample_crops(const void* raw_store, int raw_bytes_per_code, int F, const unsigned char* gt_store, int G, int H,
+                      int W, const int* pos, int B, int h, int w, float white_level, float* img_out, float* gt_out,
+                      int* status, risp_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------
  * Fused fixed pipeline (isp_universal.py:210-232 / origin_universal.py:143-161 as ONE pass):

@@ -302,17 +302,84 @@ extern "C" int risp_decode_codes(const void* src, float* dst, long long n, int b
 }
 
 namespace risp {
-// crop + decode: dst[p][y][x] = src[p][y0+y][x0+x] / denom   (the loader's random crop after the PCIe hop)
-template <typename T>
-__global__ void __launch_bounds__(256)
-crop_decode_kernel(const T* __restrict__ src, float* __restrict__ dst, int H, int W, int y0, int x0, int h, int w, float denom) {
-  const long long plane_in = (long long)H * W, plane_out = (long long)h * w;
-  const T* s = src + (long long)blockIdx.y * plane_in;
-  float* d = dst + (long long)blockIdx.y * plane_out;
-  for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < plane_out; i += (long long)gridDim.x * 256) {
-    const int y = (int)(i / w), x = (int)(i - (long long)y * w);
-    d[i] = __fdiv_rn((float)s[(long long)(y0 + y) * W + x0 + x], denom);
+// Crop + decode of a batch of records: the loader's random crop, after the PCIe hop or out of a frame store in HBM.
+// Record r = (frame a, frame b, y0, x0) crops store a (pa planes per frame, codes of T) and store b (pb planes per frame,
+// 8-bit codes) at the same origin:  da[r][p] = a[frame a][p][y0:y0+h, x0:x0+w] / denom_a, and db likewise from b.
+// Records may be device data the host never sees, so each block checks its own: a record out of range, or odd where
+// `odd` asks for even origins (the CFA phase of a Bayer crop), sets *status and is skipped; nothing outside the stores is read.
+struct CropJob {
+  const void* a;
+  const unsigned char* b;
+  float* da;
+  float* db;
+  const int4* pos;       // DEVICE records; null: the single record (0, 0, y0, x0)
+  int fa, fb;            // frames in each store
+  int pa, pb;            // planes per frame (pb = 0: no second store)
+  int H, W, h, w, y0, x0;
+  int odd;               // origin bits that must be clear: 1 for a Bayer crop, 0 for any origin
+  float denom_a, denom_b;
+  int* status;           // nullable when pos is null (the host checked the one record)
+};
+
+// One plane of one record.  s: the crop's first code, d: the output plane.  VEC: four columns per item and one 16-byte
+// store (w % 4 == 0, d 16-byte aligned).  An item's row and column advance by a constant stride: no division in the loop.
+template <typename T, bool VEC>
+__device__ __forceinline__ void crop_plane(const T* __restrict__ s, float* __restrict__ d, int W, int h, int w, float denom) {
+  constexpr int V = VEC ? 4 : 1;
+  const int wq = w / V;
+  const int start = blockIdx.x * 256 + threadIdx.x, step = gridDim.x * 256;
+  int y = start / wq, x = start - y * wq;
+  const int dy = step / wq, dx = step - dy * wq;
+  while (y < h) {
+    const T* p = s + (long long)y * W + x * V;
+    float* o = d + (long long)y * w + x * V;
+    if (VEC)
+      st_stream4(o, make_float4(__fdiv_rn((float)__ldg(p), denom), __fdiv_rn((float)__ldg(p + 1), denom),
+                                __fdiv_rn((float)__ldg(p + 2), denom), __fdiv_rn((float)__ldg(p + 3), denom)));
+    else
+      *o = __fdiv_rn((float)__ldg(p), denom);
+    x += dx;
+    y += dy;
+    if (x >= wq) { x -= wq; ++y; }
   }
+}
+
+// grid: x = blocks per output plane, y = records * (pa + pb) output planes
+template <typename T, bool VEC>
+__global__ void __launch_bounds__(256)
+crop_decode_kernel(const CropJob j) {
+  const int planes = j.pa + j.pb;
+  const int r = blockIdx.y / planes, p = blockIdx.y - r * planes;
+  const int4 rec = j.pos ? j.pos[r] : make_int4(0, 0, j.y0, j.x0);
+  if (rec.x < 0 || rec.x >= j.fa || (j.pb && (rec.y < 0 || rec.y >= j.fb)) || rec.z < 0 || rec.w < 0 ||
+      rec.z > j.H - j.h || rec.w > j.W - j.w || ((rec.z | rec.w) & j.odd)) {
+    if (j.status && threadIdx.x == 0) *j.status = 1;
+    return;
+  }
+  const long long plane_in = (long long)j.H * j.W, plane_out = (long long)j.h * j.w, off = (long long)rec.z * j.W + rec.w;
+  if (p < j.pa)
+    crop_plane<T, VEC>(static_cast<const T*>(j.a) + ((long long)rec.x * j.pa + p) * plane_in + off,
+                       j.da + ((long long)r * j.pa + p) * plane_out, j.W, j.h, j.w, j.denom_a);
+  else
+    crop_plane<unsigned char, VEC>(j.b + ((long long)rec.y * j.pb + p - j.pa) * plane_in + off,
+                                   j.db + ((long long)r * j.pb + p - j.pa) * plane_out, j.W, j.h, j.w, j.denom_b);
+}
+
+// At most max(16 blocks per SM, one block per output plane) blocks; each block strides over its plane.
+static int launch_crops(const CropJob& j, int records, int bytes_per_code, cudaStream_t st) {
+  const bool vec = j.w % 4 == 0 && aligned16(j.da) && (j.pb == 0 || aligned16(j.db));
+  const int planes = records * (j.pa + j.pb);
+  long long g = cdiv((long long)j.h * (vec ? j.w / 4 : j.w), 256), cap = (long long)sm_count() * 16 / planes;
+  if (cap < 1) cap = 1;
+  dim3 grid((unsigned)(g > cap ? cap : g), (unsigned)planes);
+  if (bytes_per_code == 2) {
+    if (vec) crop_decode_kernel<unsigned short, true><<<grid, 256, 0, st>>>(j);
+    else crop_decode_kernel<unsigned short, false><<<grid, 256, 0, st>>>(j);
+  } else {
+    if (vec) crop_decode_kernel<unsigned char, true><<<grid, 256, 0, st>>>(j);
+    else crop_decode_kernel<unsigned char, false><<<grid, 256, 0, st>>>(j);
+  }
+  return check_launch("crop_decode_kernel");
 }
 }  // namespace risp
 
@@ -325,11 +392,31 @@ extern "C" int risp_crop_decode(const void* src, float* dst, int planes, int H, 
   RISP_REQUIRE(bytes_per_code == 1 || bytes_per_code == 2, RISP_E_INVALID, "risp_crop_decode: 1 or 2 bytes per code");
   RISP_REQUIRE(!require_even || ((y0 % 2 == 0) && (x0 % 2 == 0)), RISP_E_ALIGN,
                "risp_crop_decode: a Bayer crop must start on an even row and column (CFA phase), got (%d,%d)", y0, x0);
-  long long g = cdiv((long long)h * w, 256), cap = (long long)sm_count() * 8;
-  dim3 grid((unsigned)(g > cap ? cap : g), (unsigned)planes);
-  if (bytes_per_code == 2)
-    crop_decode_kernel<unsigned short><<<grid, 256, 0, as_stream(stream)>>>(static_cast<const unsigned short*>(src), dst, H, W, y0, x0, h, w, denom);
-  else
-    crop_decode_kernel<unsigned char><<<grid, 256, 0, as_stream(stream)>>>(static_cast<const unsigned char*>(src), dst, H, W, y0, x0, h, w, denom);
-  return check_launch("crop_decode_kernel");
+  CropJob j{};
+  j.a = src; j.da = dst; j.fa = 1; j.pa = planes;
+  j.H = H; j.W = W; j.h = h; j.w = w; j.y0 = y0; j.x0 = x0;
+  j.odd = require_even ? 1 : 0;
+  j.denom_a = denom;
+  return launch_crops(j, 1, bytes_per_code, as_stream(stream));
+}
+
+extern "C" int risp_sample_crops(const void* raw_store, int raw_bytes_per_code, int F, const unsigned char* gt_store, int G,
+                                 int H, int W, const int* pos, int B, int h, int w, float white_level, float* img_out,
+                                 float* gt_out, int* status, risp_stream_t stream) {
+  RISP_REQUIRE(raw_store && pos && img_out && status && F > 0 && H > 0 && W > 0 && B > 0 && h > 0 && w > 0 && white_level > 0.f,
+               RISP_E_INVALID, "risp_sample_crops: bad arguments");
+  RISP_REQUIRE(!gt_out || (gt_store && G > 0), RISP_E_INVALID, "risp_sample_crops: gt_out needs gt_store and G > 0");
+  RISP_REQUIRE(raw_bytes_per_code == 1 || raw_bytes_per_code == 2, RISP_E_INVALID, "risp_sample_crops: 1 or 2 bytes per raw code");
+  RISP_REQUIRE(h <= H && w <= W, RISP_E_INVALID, "risp_sample_crops: a %dx%d crop does not fit the %dx%d frames", h, w, H, W);
+  RISP_REQUIRE((long long)B * (gt_out ? 4 : 1) <= 65535, RISP_E_INVALID, "risp_sample_crops: %d records are too many for one launch", B);
+  RISP_REQUIRE(aligned16(pos), RISP_E_ALIGN, "risp_sample_crops: pos must be 16-byte aligned");
+  CropJob j{};
+  j.a = raw_store; j.da = img_out; j.fa = F; j.pa = 1;
+  if (gt_out) { j.b = gt_store; j.db = gt_out; j.fb = G; j.pb = 3; }
+  j.pos = reinterpret_cast<const int4*>(pos);
+  j.H = H; j.W = W; j.h = h; j.w = w;
+  j.odd = 1;
+  j.denom_a = white_level; j.denom_b = 255.f;
+  j.status = status;
+  return launch_crops(j, B, raw_bytes_per_code, as_stream(stream));
 }

@@ -405,6 +405,38 @@ def crop_decode(codes, y0, x0, h, w, denom, bayer=True):
     return out
 
 
+def sample_crops(raw_store, gt_store, pos, h, w, white_level, status, img_out=None, gt_out=None):
+    """A batch of crops out of frame stores in HBM in one launch (`risp_sample_crops`, the kernel of `crop_decode`).
+    raw_store (F,H,W) uint8 / int16 codes (int16 holds the bit pattern of unsigned 16-bit codes), gt_store (G,3,H,W) uint8 BGR
+    or None, pos (B,4) int32 CUDA records (raw frame, gt frame, y0, x0) with even origins, status (1,) int32 CUDA.
+    -> img (B,1,h,w) = code / white_level and gt (B,3,h,w) = code / 255 (None without gt_store), fp32, written into
+    img_out / gt_out when given.  A bad record sets status and is skipped; nothing here reads status or waits for the device."""
+    F, H, W = raw_store.shape
+    if raw_store.dtype not in (torch.uint8, torch.int16):
+        raise ValueError('sample_crops: raw codes must be uint8 or int16, got %s' % raw_store.dtype)
+    if gt_store is not None and (gt_store.dtype != torch.uint8 or tuple(gt_store.shape[1:]) != (3, H, W)):
+        raise ValueError('sample_crops: gt_store must be uint8 (G,3,%d,%d), got %s %s' % (H, W, gt_store.dtype, tuple(gt_store.shape)))
+    if pos.dtype != torch.int32 or pos.dim() != 2 or pos.shape[1] != 4:
+        raise ValueError('sample_crops: pos must be int32 (B,4), got %s %s' % (pos.dtype, tuple(pos.shape)))
+    if status.dtype != torch.int32 or status.numel() < 1:
+        raise ValueError('sample_crops: status must be an int32 tensor')
+    B = pos.shape[0]
+    dev = raw_store.device
+    if img_out is None:
+        img_out = torch.empty((B, 1, h, w), device=dev, dtype=torch.float32)
+    if gt_store is None:
+        gt_out = None
+    elif gt_out is None:
+        gt_out = torch.empty((B, 3, h, w), device=dev, dtype=torch.float32)
+    if tuple(img_out.shape) != (B, 1, h, w) or img_out.dtype != torch.float32 or \
+            (gt_out is not None and (tuple(gt_out.shape) != (B, 3, h, w) or gt_out.dtype != torch.float32)):
+        raise ValueError('sample_crops: outputs must be fp32 (%d,1,%d,%d) and (%d,3,%d,%d)' % (B, h, w, B, h, w))
+    G = 0 if gt_store is None else gt_store.shape[0]
+    L.call('risp_sample_crops', L.ptr(raw_store), raw_store.element_size(), F, L.ptr(gt_store), G, H, W, L.ptr(pos), B, int(h),
+           int(w), float(white_level), L.ptr(img_out), L.ptr(gt_out), L.ptr(status), L.stream())
+    return img_out, gt_out
+
+
 def to_u8_hwc(x):
     """`utils.util.tensor2bgr(tensor)` on the device: (C,H,W) or (1,C,H,W) fp32 -> (H,W,C) uint8 = trunc(clip(x*255, 0, 255))."""
     x = (x[0] if x.dim() == 4 else x).detach().contiguous()
