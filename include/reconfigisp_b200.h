@@ -196,6 +196,20 @@ int risp_pipeline_eval(const float* raw, const float* gt, unsigned char* u8_out,
                        int dm_kind, float dm_clip_hi, const int* ops, const int* param_off, const int* iarg, int S,
                        const float* params, int param_stride, void* workspace, size_t workspace_bytes,
                        risp_stream_t stream);
+/* risp_pipeline_eval on whole frames of the stores of risp_sample_crops, read as codes (5 B/px with a 16-bit raw): image n
+ * is raw frame pos[n].x, decoded in registers as code / white_level with the sampler's correctly rounded division, against
+ * the 8-bit planar GT frame pos[n].y, whose codes are compared as they are (a stored code is its own tensor2bgr code).
+ * sse_out and u8_out are risp_pipeline_eval's on the batch risp_sample_crops decodes from the same whole-frame records,
+ * bit for bit, with the same dispatch (RISP_FUSED=0 included).
+ *   pos: DEVICE int32 [N][4] = (raw frame, GT frame, 0, 0), 16-byte aligned.  A record that names a frame outside a store
+ *   or a non-zero origin sets *status (DEVICE int32) and adds nothing (its sse_out is 0); nothing outside the stores is read.
+ *   H even, W % 4 == 0.  The packed kernels read the stores through tensor maps: where they take the chain, W must be a
+ *   multiple of 16 (16-byte rows), else RISP_E_UNSUPPORTED.  Workspace: risp_pipeline_eval_workspace(N, H, W). */
+int risp_pipeline_eval_store(const void* raw_store, int raw_bytes_per_code, int F, const unsigned char* gt_store, int G,
+                             int H, int W, const int* pos, int N, float white_level, int* status, unsigned char* u8_out,
+                             long long* sse_out, int dm_kind, float dm_clip_hi, const int* ops, const int* param_off,
+                             const int* iarg, int S, const float* params, int param_stride, void* workspace,
+                             size_t workspace_bytes, risp_stream_t stream);
 
 /* Per-image SSIM of the same 8-bit codes (skimage 0.16 compare_ssim(a, b, multichannel=True) with its defaults: uniform 7x7
  * window, sample covariance, K1 = 0.01, K2 = 0.03, data_range 255, a border of 3 pixels cropped).  For every channel and
@@ -209,6 +223,12 @@ int risp_pipeline_eval(const float* raw, const float* gt, unsigned char* u8_out,
 enum risp_image_layout { RISP_IMG_F32_NCHW = 0, RISP_IMG_U8_NHWC = 1 };
 int risp_ssim_u8(const void* y, int y_layout, const float* gt, long long* ssim_sum_out, int N, int C, int H, int W,
                  risp_stream_t stream);
+/* The same sums against GT frames of a store: image n of y (C = 3) against the 8-bit planar frame pos[n].y of gt_store
+ * (G,3,H,W), whose codes enter as they are -- bit-identical to risp_ssim_u8 with the decoded fp32 GT.  pos: DEVICE int32
+ * [N][4] records of risp_pipeline_eval_store; a record whose GT frame lies outside the store or whose origin is not
+ * (0, 0) sets *status and adds nothing (its sum is 0). */
+int risp_ssim_u8_store(const void* y, int y_layout, const unsigned char* gt_store, int G, const int* pos, int* status,
+                       long long* ssim_sum_out, int N, int H, int W, risp_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------
  * Per-image statistics (grayworld tools_origin.py:35-41, SRCNNRes global features

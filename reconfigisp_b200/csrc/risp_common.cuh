@@ -99,6 +99,19 @@ __device__ __forceinline__ uint32_t sq_codes4(float4 y, float4 t) {
   const int d2 = u8_code(y.z) - u8_code(t.z), d3 = u8_code(y.w) - u8_code(t.w);
   return (uint32_t)(d0 * d0 + d1 * d1 + d2 * d2 + d3 * d3);
 }
+// the same against 4 GT codes of a frame store (bytes of t, lowest first).  A stored code c is its own tensor2bgr code:
+// trunc(clip(fl32(fl32(c/255)*255), 0, 255)) == c for every c in 0..255, so the GT needs no quantisation
+__device__ __forceinline__ uint32_t sq_codes4_u8(float4 y, uint32_t t) {
+  const int d0 = u8_code(y.x) - (int)(t & 0xffu), d1 = u8_code(y.y) - (int)((t >> 8) & 0xffu);
+  const int d2 = u8_code(y.z) - (int)((t >> 16) & 0xffu), d3 = u8_code(y.w) - (int)(t >> 24);
+  return (uint32_t)(d0 * d0 + d1 * d1 + d2 * d2 + d3 * d3);
+}
+// a raw code of a frame store as the sampler decodes it (risp_sample_crops): code / white_level, correctly rounded
+__device__ __forceinline__ float decode_code(uint32_t c, float white_level) { return __fdiv_rn((float)c, white_level); }
+// the record of a whole-frame evaluation: (raw slot, GT slot, 0, 0) with both slots inside their stores
+__device__ __forceinline__ bool whole_frame_record(int4 r, int F, int G) {
+  return r.x >= 0 && r.x < F && r.y >= 0 && r.y < G && r.z == 0 && r.w == 0;
+}
 __device__ __forceinline__ unsigned long long warp_sum_u64(unsigned long long v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

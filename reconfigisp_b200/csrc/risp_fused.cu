@@ -26,7 +26,10 @@ namespace fused {
 __constant__ float g_cpar[kCSlots][kCRows][kCRowFloats];
 
 // STEP: MSE loss; STEP_L1: L1 loss (isp_model.py:44-49); EVAL: inference arithmetic + squared 8-bit code differences to the GT
-enum { MODE_FWD = 0, MODE_STEP = 1, MODE_BWD = 2, MODE_STEP_L1 = 3, MODE_EVAL = 4 };
+// EVAL_S16 / EVAL_U8: EVAL reading a frame store (16-bit / 8-bit raw codes, 8-bit planar GT codes; frames named by records)
+enum { MODE_FWD = 0, MODE_STEP = 1, MODE_BWD = 2, MODE_STEP_L1 = 3, MODE_EVAL = 4, MODE_EVAL_S16 = 5, MODE_EVAL_U8 = 6 };
+__host__ __device__ constexpr bool is_store(int mode) { return mode == MODE_EVAL_S16 || mode == MODE_EVAL_U8; }
+__host__ __device__ constexpr bool is_eval(int mode) { return mode == MODE_EVAL || is_store(mode); }
 // A CTA is one warp (32 threads), so everything but the lane index is CTA-uniform (uniform datapath, no R2UR).  The warp
 // owns a strip of kStrip columns.
 constexpr int kStrip = 128;
@@ -47,6 +50,15 @@ struct FusedArgs {
   // narrow items (backward-carrying kernels): the last strip of a frame, nw = 32 or 64 columns wide (0: none), marched by
   // 128/nw lane groups on as many row pairs at once; the strip_blocks full strips lie to its left
   int nw, nrows_per_chunk, nchunks;
+};
+
+// store modes: image n of the launch is frame pos[n].x of the raw store against frame pos[n].y of the GT store (FusedArgs'
+// raw / gt hold the stores).  A kernel parameter of its own, after the others: the other modes' parameters keep their offsets
+struct StoreArgs {
+  const int4* pos;
+  int* status;          // set when a record is not a whole frame of the stores; that image adds nothing
+  float white_level;
+  int F, G;             // frames in the raw / GT store
 };
 
 // ---- preparation: derived constants of every parameter row ---------------------------------------------------------
@@ -139,6 +151,47 @@ __device__ __forceinline__ float lds1(uint32_t addr) {
   asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
   return v;
 }
+__device__ __forceinline__ uint32_t lds_u32(uint32_t addr) {
+  uint32_t v;
+  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
+  return v;
+}
+__device__ __forceinline__ uint2 lds_u64(uint32_t addr) {
+  uint2 v;
+  asm volatile("ld.shared.v2.u32 {%0,%1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(addr));
+  return v;
+}
+__device__ __forceinline__ uint32_t lds_u16(uint32_t addr) {
+  unsigned short v;
+  asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(addr));
+  return v;
+}
+__device__ __forceinline__ uint32_t lds_u8(uint32_t addr) {
+  unsigned short v;
+  asm volatile("ld.shared.u8 %0, [%1];" : "=h"(v) : "r"(addr));
+  return v;
+}
+// raw window values out of a ring record: fp32 as copied, or store codes decoded in registers (decode_code)
+template <int MODE>
+__device__ __forceinline__ float4 ld_raw4(uint32_t addr, float wl) {
+  if constexpr (MODE == MODE_EVAL_S16) {
+    const uint2 v = lds_u64(addr);
+    return make_float4(decode_code(v.x & 0xffffu, wl), decode_code(v.x >> 16, wl), decode_code(v.y & 0xffffu, wl),
+                       decode_code(v.y >> 16, wl));
+  } else if constexpr (MODE == MODE_EVAL_U8) {
+    const uint32_t v = lds_u32(addr);
+    return make_float4(decode_code(v & 0xffu, wl), decode_code((v >> 8) & 0xffu, wl), decode_code((v >> 16) & 0xffu, wl),
+                       decode_code(v >> 24, wl));
+  } else {
+    return lds4(addr);
+  }
+}
+template <int MODE>
+__device__ __forceinline__ float ld_raw1(uint32_t addr, float wl) {
+  if constexpr (MODE == MODE_EVAL_S16) return decode_code(lds_u16(addr), wl);
+  else if constexpr (MODE == MODE_EVAL_U8) return decode_code(lds_u8(addr), wl);
+  else return lds1(addr);
+}
 __device__ __forceinline__ void sts4(uint32_t addr, float4 v) {
   asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
 }
@@ -157,9 +210,15 @@ struct RingCfg {
   // (measured: 1 KB boxes deliver 1.9 TB/s chip-wide), so the inference kernel, which has nothing but the copies to wait
   // for, uses 4-row boxes; the backward-carrying kernels are issue-bound and keep the smaller ring
   static constexpr int RR = (MODE == MODE_FWD) ? 4 : 2;
-  static constexpr int RAWROWB = (kStrip + 2 * kPad) * 4;                // 544 B: one raw row of the box
+  static constexpr int ES = (MODE == MODE_EVAL_S16) ? 2 : (MODE == MODE_EVAL_U8) ? 1 : 4;   // bytes per raw value
+  static constexpr int GES = is_store(MODE) ? 1 : 4;                                         // bytes per GT value
+  // columns of left pad: 16 bytes, so that a box starts on a 16-byte boundary of the row (kPad floats; 8 / 16 codes)
+  static constexpr int PADL = 16 / ES;
+  // one raw row of the box (left pad, strip, the right halo), widened to a 16-byte multiple (a tensor-map rule): 544 B of
+  // fp32 (136 columns), 288 B of 16-bit codes (144), 160 B of 8-bit codes (160)
+  static constexpr int RAWROWB = ((PADL + kStrip + 2) * ES + 15) / 16 * 16;
   static constexpr int RAWB = (RR * RAWROWB + 127) / 128 * 128;          // RR rows, padded to a 128-B multiple
-  static constexpr int GTPLANEB = RR * kStrip * 4;
+  static constexpr int GTPLANEB = RR * kStrip * GES;
   static constexpr int GTB = (MODE == MODE_FWD) ? 0 : 3 * GTPLANEB;  // [plane][row][128]
   static constexpr int RECB = RAWB + GTB;                                // multiple of 128
   static constexpr int WARPB = D * RECB;
@@ -420,20 +479,30 @@ constexpr int kMaxRows = 256;        // rows per item at most
 template <int DM, int MODE, unsigned SIG, bool NARROW>
 __global__ void __launch_bounds__(32, (MODE == MODE_FWD) ? kFwdMinBlocks : kStepMinBlocks)
 fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_raw, const __grid_constant__ CUtensorMap tm_gt,
-             const __grid_constant__ CUtensorMap tm_rawn, const __grid_constant__ CUtensorMap tm_gtn) {
+             const __grid_constant__ CUtensorMap tm_rawn, const __grid_constant__ CUtensorMap tm_gtn, const StoreArgs sa) {
   constexpr EffChain E = Eff<SIG>::e;
   constexpr int HL = (DM == RISP_DM_MALVAR) ? 2 : 1;
   constexpr int WR = 2 * HL + 1, WC = 4 + 2 * HL;
-  constexpr int NACC = (MODE == MODE_FWD || MODE == MODE_EVAL || E.nacc == 0) ? 1 : E.nacc;
+  constexpr int NACC = (MODE == MODE_FWD || is_eval(MODE) || E.nacc == 0) ? 1 : E.nacc;
   constexpr int NCST = E.ncst > 0 ? E.ncst : 1;
   static_assert(E.ncst <= kCRowFloats, "the chain's derived constants must fit one row of the constant slot");
   constexpr bool PKDM = E.n > 0 && (E.op[0] == RISP_OP_POLY10 || E.op[0] == FOP_POLYG || E.op[0] == RISP_OP_GAIN);
   using RC = RingCfg<MODE>;
   constexpr int D = RC::D;
+  constexpr int ES = RC::ES, GES = RC::GES;
   extern __shared__ unsigned char smem_raw[];
   const int lane = threadIdx.x;
   const int n = blockIdx.y, j0 = blockIdx.x;       // frame, CTA within the frame (both uniform)
   const int H = a.H, W = a.W;
+  int zraw = 0, zgt = 0;                           // store modes: tensor-map frame / first GT plane of image n
+  if constexpr (is_store(MODE)) {
+    const int4 rec = sa.pos[n];
+    if (!whole_frame_record(rec, sa.F, sa.G)) {
+      if (lane == 0) { *sa.status = 1; a.sse[(long long)n * a.cpf + j0] = 0ull; }
+      return;
+    }
+    zraw = rec.x; zgt = 3 * rec.y;
+  }
   const long long plane = (long long)H * W;
   float* __restrict__ yb = a.y ? a.y + (long long)n * 3 * plane : nullptr;
   // derived constants of this frame's parameter row (written by fused_prep_kernel earlier on the stream): they enter the
@@ -455,7 +524,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
 #pragma unroll
     for (int s = 0; s < D; ++s) mbar_init(bars + 8 * s, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    if constexpr (MODE != MODE_FWD && MODE != MODE_EVAL) {
+    if constexpr (MODE != MODE_FWD && !is_eval(MODE)) {
 #pragma unroll
       for (int k = 0; k < E.n; ++k)
         if (E.op[k] == RISP_OP_GTM) gtm_table_fill(tbl + k * kGtmTableBytes, cp + E.coff[k]);
@@ -490,19 +559,21 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
 #pragma unroll
     for (int j = 0; j < WR; ++j) {
       const uint32_t rj = wa(j);
-      const float4 v = lds4(rj + L.own);
+      const float wl = sa.white_level;
+      const float4 v = ld_raw4<MODE>(rj + L.own, wl);
       if constexpr (HL == 1) {
-        w[j][0] = lds1(rj + L.oL0); w[j][1] = v.x; w[j][2] = v.y; w[j][3] = v.z; w[j][4] = v.w; w[j][5] = lds1(rj + L.oR0);
+        w[j][0] = ld_raw1<MODE>(rj + L.oL0, wl); w[j][1] = v.x; w[j][2] = v.y; w[j][3] = v.z; w[j][4] = v.w;
+        w[j][5] = ld_raw1<MODE>(rj + L.oR0, wl);
       } else {
-        w[j][0] = lds1(rj + L.oL0); w[j][1] = lds1(rj + L.oL1);
+        w[j][0] = ld_raw1<MODE>(rj + L.oL0, wl); w[j][1] = ld_raw1<MODE>(rj + L.oL1, wl);
         w[j][2] = v.x; w[j][3] = v.y; w[j][4] = v.z; w[j][5] = v.w;
-        w[j][6] = lds1(rj + L.oR0); w[j][7] = lds1(rj + L.oR1);
+        w[j][6] = ld_raw1<MODE>(rj + L.oR0, wl); w[j][7] = ld_raw1<MODE>(rj + L.oR1, wl);
       }
     }
     P2 lo, hi;
     demosaic4<DM, HL, 0, ODD, WR, PKDM>(w, a.clip_hi, lo, hi);
     P2 ylo, yhi;
-    if constexpr (MODE == MODE_EVAL) {
+    if constexpr (is_eval(MODE)) {
       // the inference arithmetic (Fwd, not Run): the codes are those of risp_pipeline_fwd's image, byte for byte
       ylo = Fwd<SIG, 0>::go(lo, cp, slow);
       yhi = Fwd<SIG, 0>::go(hi, cp, slow);
@@ -510,8 +581,13 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
                    yR = make_float4(ylo.r.x, ylo.r.y, yhi.r.x, yhi.r.y);
       // lanes beyond the right edge compute garbage from zero-filled raw (a zero pixel is not zero after the chain): masked
       if (L.active) {
-        const uint32_t s = sq_codes4(yB, lds4(gta + L.gt)) + sq_codes4(yG, lds4(gta + RC::GTPLANEB + L.gt)) +
-                           sq_codes4(yR, lds4(gta + 2 * RC::GTPLANEB + L.gt));
+        uint32_t s;
+        if constexpr (is_store(MODE))
+          s = sq_codes4_u8(yB, lds_u32(gta + L.gt)) + sq_codes4_u8(yG, lds_u32(gta + RC::GTPLANEB + L.gt)) +
+              sq_codes4_u8(yR, lds_u32(gta + 2 * RC::GTPLANEB + L.gt));
+        else
+          s = sq_codes4(yB, lds4(gta + L.gt)) + sq_codes4(yG, lds4(gta + RC::GTPLANEB + L.gt)) +
+              sq_codes4(yR, lds4(gta + 2 * RC::GTPLANEB + L.gt));
         sse += s;
         if (a.u8) {      // (H,W,3) BGR bytes of the lane's 4 pixels: 12 contiguous bytes, 4-byte aligned (c0 % 4 == 0)
           const uint32_t b0 = u8_code(yB.x), b1 = u8_code(yB.y), b2 = u8_code(yB.z), b3 = u8_code(yB.w);
@@ -539,7 +615,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
       Run<SIG, 0, MODE>::go(lo, tlo, cp, acc, loss, ylo, slow, L.lane_w, tbl);
       Run<SIG, 0, MODE>::go(hi, thi, cp, acc, loss, yhi, slow, L.lane_w, tbl);
     }
-    if (MODE != MODE_EVAL && yb && L.active) {
+    if (!is_eval(MODE) && yb && L.active) {
       float* po = yb + (size_t)(r + L.dr) * W + L.c0;
       st_stream4(po, make_float4(ylo.b.x, ylo.b.y, yhi.b.x, yhi.b.y));
       st_stream4(po + plane, make_float4(ylo.g.x, ylo.g.y, yhi.g.x, yhi.g.y));
@@ -566,8 +642,8 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
       const uint32_t rec = ring + (g & (D - 1)) * RC::RECB, bar = bars + (g & (D - 1)) * 8;
       const bool has_gt = (MODE != MODE_FWD) && (k >= 1) && (k < nrec - 1);
       mbar_expect_tx(bar, (uint32_t)(RR * RC::RAWROWB) + (has_gt ? (uint32_t)RC::GTB : 0u));
-      tma_load_3d(rec, &tm_raw, c0s - kPad, rbase + RR * k, n, bar);
-      if (has_gt) tma_load_3d(rec + RC::RAWB, &tm_gt, c0s, rbase + RR * k, 3 * n, bar);
+      tma_load_3d(rec, &tm_raw, c0s - RC::PADL, rbase + RR * k, is_store(MODE) ? zraw : n, bar);
+      if (has_gt) tma_load_3d(rec + RC::RAWB, &tm_gt, c0s, rbase + RR * k, is_store(MODE) ? zgt : 3 * n, bar);
     };
     auto wait_rec = [&](int k) {
       const unsigned g = gcount + (unsigned)k;
@@ -589,16 +665,17 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
 
     // lane offsets inside a raw row (bytes): own 4 columns; the strip's first / last lane reads its outer halo from the
     // record (frame border folded into the offset), every other lane gets it from its neighbour by shuffle
-    const uint32_t own = (uint32_t)(kPad + lane * 4) * 4u;
+    const uint32_t own = (uint32_t)(RC::PADL + lane * 4) * ES;
     const bool endL = (lane == 0), endR = (lane == 31) || last;
-    const uint32_t oL0 = own + (first ? (HL == 1 ? 4 : 8) : -4 * HL);    // column c0-HL   (reflect: -1 -> 1, -2 -> 2)
-    const uint32_t oL1 = own + (first ? 4 : -4);                         // column c0-1    (HL == 2 only)
-    const uint32_t oR0 = own + (last ? 8 : 16);                          // column c0+4    (reflect: W -> W-2)
-    const uint32_t oR1 = own + (last ? 4 : 20);                          // column c0+5    (reflect: W+1 -> W-3)
+    // byte offsets of columns; ES == 4 spelled out (the fp32 kernels' instruction stream stays as it was)
+    const uint32_t oL0 = own + (ES == 4 ? (first ? (HL == 1 ? 4 : 8) : -4 * HL) : ES * (first ? (HL == 1 ? 1 : 2) : -HL));  // column c0-HL (reflect: -1 -> 1, -2 -> 2)
+    const uint32_t oL1 = own + (ES == 4 ? (first ? 4 : -4) : ES * (first ? 1 : -1));     // column c0-1    (HL == 2 only)
+    const uint32_t oR0 = own + (ES == 4 ? (last ? 8 : 16) : ES * (last ? 2 : 4));        // column c0+4    (reflect: W -> W-2)
+    const uint32_t oR1 = own + (ES == 4 ? (last ? 4 : 20) : ES * (last ? 1 : 5));        // column c0+5    (reflect: W+1 -> W-3)
 
     if constexpr (MODE != MODE_FWD) {
       // ---- backward-carrying kernels: 2-row records ----
-      const LanePos L{own, oL0, oL1, oR0, oR1, (uint32_t)lane * 16u, c0, 0, active, lane_w};
+      const LanePos L{own, oL0, oL1, oR0, oR1, (uint32_t)lane * (4u * GES), c0, 0, active, lane_w};
 
       // iteration m computes rows r = ra + 2(m-1) (even) and r+1 (odd) from records m-1, m, m+1.
       // The loop exists twice, with the tone curve's slow flag (a knot outside [0,1]: final clamp active) as a compile-time
@@ -625,7 +702,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
           for (int j = 0; j < WR; ++j) { we[j] = row_addr(r - HL + j); wo[j] = row_addr(r + 1 - HL + j); }
         }
         do_row(std::false_type{}, slow_tag, std::false_type{}, r, [&](int j) { return we[j]; }, recB + RC::RAWB, L);
-        do_row(std::true_type{}, slow_tag, std::false_type{}, r + 1, [&](int j) { return wo[j]; }, recB + RC::RAWB + kStrip * 4, L);
+        do_row(std::true_type{}, slow_tag, std::false_type{}, r + 1, [&](int j) { return wo[j]; }, recB + RC::RAWB + kStrip * GES, L);
         __syncwarp();                              // every lane has read record m-1: its slot may be refilled
         if (m - 1 + D < nrec) {
           if (elect_one()) issue(m - 1 + D);
@@ -719,20 +796,21 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
     const int RRn = 1 << sh;
     const int grp = lane >> (6 - sh), li = lane & ((1 << (6 - sh)) - 1);
     const int c0s = a.strip_blocks * kStrip, c0 = c0s + 4 * li;
-    const uint32_t rowb = (uint32_t)(nw + kPad) * 4u;
+    // bytes per box row: fp32 rows are 16-byte multiples already, code rows widen to one (a tensor-map rule)
+    const uint32_t rowb = ES == 4 ? (uint32_t)(nw + kPad) * 4u : ((uint32_t)(nw + RC::PADL) * ES + 15u) & ~15u;
     const bool incol = c0 < W, first = (c0 == 0), last = incol && (c0 + 4 >= W);
     LanePos L;
-    L.own = (uint32_t)(kPad + 4 * li) * 4u;
-    L.oL0 = L.own + (first ? (HL == 1 ? 4 : 8) : -4 * HL);
-    L.oL1 = L.own + (first ? 4 : -4);
+    L.own = (uint32_t)(RC::PADL + 4 * li) * ES;
+    L.oL0 = L.own + (ES == 4 ? (first ? (HL == 1 ? 4 : 8) : -4 * HL) : ES * (first ? (HL == 1 ? 1 : 2) : -HL));
+    L.oL1 = L.own + (ES == 4 ? (first ? 4 : -4) : ES * (first ? 1 : -1));
     // a lane with c0 + 4 < W is never the last of its group (W <= c0s + nw).  Lanes past the frame read inside their row
     // as well: past the last row of a 64-wide box lie pad bytes that no copy writes (stale data, possibly NaN)
     const bool fold = last || !incol;
-    L.oR0 = L.own + (fold ? 8 : 16);
-    L.oR1 = L.own + (fold ? 4 : 20);
+    L.oR0 = L.own + (ES == 4 ? (fold ? 8 : 16) : ES * (fold ? 2 : 4));
+    L.oR1 = L.own + (ES == 4 ? (fold ? 4 : 20) : ES * (fold ? 1 : 5));
     L.c0 = c0;
     L.dr = 2 * grp;
-    const uint32_t gt_even = (uint32_t)(2 * grp * nw + 4 * li) * 4u;
+    const uint32_t gt_even = (uint32_t)(2 * grp * nw + 4 * li) * GES;
     for (int t = a.cpf - 1 - j0; t < a.nchunks; t += a.cpf) {
       const int ra = t * a.nrows_per_chunk;
       const int rb = min(H, ra + a.nrows_per_chunk);
@@ -743,8 +821,8 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
         const uint32_t rec = ring + (g & (D - 1)) * RC::RECB, bar = bars + (g & (D - 1)) * 8;
         const bool has_gt = (k >= 1) && (k < nrec - 1);
         mbar_expect_tx(bar, (uint32_t)RRn * rowb + (has_gt ? (uint32_t)RC::GTB : 0u));
-        tma_load_3d(rec, &tm_rawn, c0s - kPad, rbase + RRn * k, n, bar);
-        if (has_gt) tma_load_3d(rec + RC::RAWB, &tm_gtn, c0s, rbase + RRn * k, 3 * n, bar);
+        tma_load_3d(rec, &tm_rawn, c0s - RC::PADL, rbase + RRn * k, is_store(MODE) ? zraw : n, bar);
+        if (has_gt) tma_load_3d(rec + RC::RAWB, &tm_gtn, c0s, rbase + RRn * k, is_store(MODE) ? zgt : 3 * n, bar);
       };
       auto wait_rec = [&](int k) {
         const unsigned g = gcount + (unsigned)k;
@@ -773,7 +851,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
           const uint32_t gta = ring + ((gcount + (unsigned)m) & (D - 1)) * RC::RECB + RC::RAWB;
           // window rows are computed where they are read: per-lane addresses live across the chain would cost registers
           do_row(std::false_type{}, slow_tag, std::true_type{}, R, [&](int j) { return row_addr(R + L.dr - HL + j); }, gta, L);
-          L.gt = gt_even + (uint32_t)nw * 4u;
+          L.gt = gt_even + (uint32_t)nw * GES;
           do_row(std::true_type{}, slow_tag, std::true_type{}, R + 1, [&](int j) { return row_addr(R + L.dr + 1 - HL + j); }, gta, L);
           __syncwarp();                              // every lane has read record m-1: its slot may be refilled
           if (m - 1 + D < nrec) {
@@ -786,7 +864,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
     }
   }
 
-  if constexpr (MODE == MODE_EVAL) {
+  if constexpr (is_eval(MODE)) {
     const unsigned long long tot = warp_sum_u64(sse);
     if (lane == 0) a.sse[(long long)n * a.cpf + j0] = tot;
   } else if constexpr (MODE != MODE_FWD) {
@@ -979,15 +1057,18 @@ static EncodeTiledFn encode_fn() {
   }
   return fn;
 }
-// fp32 tensor (W, H, Z) with rows of W floats, box (bx, by, bz); out-of-bounds elements read as zero
-static int make_map(CUtensorMap* tm, const float* base, int W, int H, long long Z, int bx, int by, int bz) {
+// tensor (W, H, Z) of es-byte elements (fp32, or the codes of a frame store), box (bx, by, bz); out-of-bounds elements
+// read as zero
+static int make_map(CUtensorMap* tm, const void* base, int W, int H, long long Z, int bx, int by, int bz, int es = 4) {
   EncodeTiledFn fn = encode_fn();
   RISP_REQUIRE(fn, RISP_E_CUDA, "fused pipeline: cuTensorMapEncodeTiled is not available");
   const cuuint64_t dims[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)Z};
-  const cuuint64_t strides[2] = {(cuuint64_t)W * 4, (cuuint64_t)W * H * 4};
+  const cuuint64_t strides[2] = {(cuuint64_t)W * es, (cuuint64_t)W * H * es};
   const cuuint32_t box[3] = {(cuuint32_t)bx, (cuuint32_t)by, (cuuint32_t)bz};
   const cuuint32_t estr[3] = {1u, 1u, 1u};
-  CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(base), dims, strides, box, estr,
+  const CUtensorMapDataType dt = es == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : es == 2 ? CU_TENSOR_MAP_DATA_TYPE_UINT16
+                                                                                  : CU_TENSOR_MAP_DATA_TYPE_UINT8;
+  CUresult r = fn(tm, dt, 3, const_cast<void*>(base), dims, strides, box, estr,
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   RISP_REQUIRE(r == CUDA_SUCCESS, RISP_E_CUDA, "fused pipeline: cuTensorMapEncodeTiled failed (%d) for %dx%dx%lld", (int)r, W, H, Z);
@@ -995,7 +1076,7 @@ static int make_map(CUtensorMap* tm, const float* base, int W, int H, long long 
 }
 
 template <int DM, int MODE, unsigned SIG>
-static int launch_one(FusedArgs a, const ChainDesc& d, int N, cudaStream_t st, int* rows_per_frame) {
+static int launch_one(FusedArgs a, const ChainDesc& d, int N, cudaStream_t st, int* rows_per_frame, const StoreArgs& sa) {
   // RISP_FUSED_STEP_ROWS: cap of the rows per item of the backward-carrying and evaluation kernels (many short items)
   static const int cap = [] { const char* e = MODE == MODE_FWD ? nullptr : getenv("RISP_FUSED_STEP_ROWS"); return e ? atoi(e) : 0; }();
   // narrow items where the kernel that runs them keeps the occupancy of the one that does not
@@ -1007,42 +1088,52 @@ static int launch_one(FusedArgs a, const ChainDesc& d, int N, cudaStream_t st, i
   a.rows_per_chunk = g.rows_per_chunk; a.chunks = g.chunks; a.strip_blocks = g.strip_blocks; a.cpf = g.cpf;
   a.nw = g.nw; a.nrows_per_chunk = g.nrows_per_chunk; a.nchunks = g.nchunks;
   CUtensorMap tm_raw, tm_gt, tm_rawn, tm_gtn;
-  int rc = make_map(&tm_raw, a.raw, a.W, a.H, N, kStrip + 2 * kPad, RingCfg<MODE>::RR, 1);
+  using RC = RingCfg<MODE>;
+  // store modes: the maps span the whole stores (F raw frames, 3G GT planes); the kernel picks frames by record
+  const long long zr = is_store(MODE) ? sa.F : N, zg = 3ll * (is_store(MODE) ? sa.G : N);
+  int rc = make_map(&tm_raw, a.raw, a.W, a.H, zr, RC::RAWROWB / RC::ES, RC::RR, 1, RC::ES);
   if (rc != RISP_OK) return rc;
   if (MODE != MODE_FWD) {
-    rc = make_map(&tm_gt, a.gt, a.W, a.H, 3ll * N, kStrip, RingCfg<MODE>::RR, 3);
+    rc = make_map(&tm_gt, a.gt, a.W, a.H, zg, kStrip, RC::RR, 3, RC::GES);
     if (rc != RISP_OK) return rc;
   } else {
     tm_gt = tm_raw;
   }
-  if (g.nw) {     // narrow boxes: 4 pad columns on the left only (the strip ends at the frame's right edge), 2G rows
+  if (g.nw) {     // narrow boxes: the left pad only (the strip ends at the frame's right edge), 2G rows
     const int rrn = 2 * (kStrip / g.nw);
     static_assert(RingCfg<MODE_STEP>::RAWB >= 36 * 8 * 4 && RingCfg<MODE_STEP>::RAWB >= 68 * 4 * 4 &&
                   RingCfg<MODE_STEP>::GTB == 3 * 32 * 8 * 4 && RingCfg<MODE_STEP>::GTB == 3 * 64 * 4 * 4,
                   "a narrow record must fit the ring's record");
-    rc = make_map(&tm_rawn, a.raw, a.W, a.H, N, g.nw + kPad, rrn, 1);
+    // code boxes: 16 bytes of left pad, widened to 16-byte rows: 40 / 72 columns of 16-bit codes, 48 / 80 of 8-bit codes
+    static_assert(RingCfg<MODE_EVAL_S16>::RAWB >= 80 * 8 && RingCfg<MODE_EVAL_S16>::RAWB >= 144 * 4 &&
+                  RingCfg<MODE_EVAL_U8>::RAWB >= 48 * 8 && RingCfg<MODE_EVAL_U8>::RAWB >= 80 * 4 &&
+                  RingCfg<MODE_EVAL_U8>::GTB == 3 * 32 * 8 && RingCfg<MODE_EVAL_U8>::GTB == 3 * 64 * 4,
+                  "a narrow record of codes must fit the ring's record");
+    const int ncols = (((g.nw + RC::PADL) * RC::ES + 15) / 16 * 16) / RC::ES;
+    rc = make_map(&tm_rawn, a.raw, a.W, a.H, zr, ncols, rrn, 1, RC::ES);
     if (rc != RISP_OK) return rc;
-    rc = make_map(&tm_gtn, a.gt, a.W, a.H, 3ll * N, g.nw, rrn, 3);
+    rc = make_map(&tm_gtn, a.gt, a.W, a.H, zg, g.nw, rrn, 3, RC::GES);
     if (rc != RISP_OK) return rc;
   } else {
     tm_rawn = tm_raw; tm_gtn = tm_gt;
   }
   if constexpr (MODE != MODE_FWD) {
     if (g.nw) {
-      fused_kernel<DM, MODE, SIG, true><<<dim3(g.cpf, N), 32, RingCfg<MODE>::SMEM, st>>>(a, d, tm_raw, tm_gt, tm_rawn, tm_gtn);
+      fused_kernel<DM, MODE, SIG, true><<<dim3(g.cpf, N), 32, RingCfg<MODE>::SMEM, st>>>(a, d, tm_raw, tm_gt, tm_rawn, tm_gtn, sa);
       return check_launch("fused_kernel");
     }
   }
-  fused_kernel<DM, MODE, SIG, false><<<dim3(g.cpf, N), 32, RingCfg<MODE>::SMEM, st>>>(a, d, tm_raw, tm_gt, tm_rawn, tm_gtn);
+  fused_kernel<DM, MODE, SIG, false><<<dim3(g.cpf, N), 32, RingCfg<MODE>::SMEM, st>>>(a, d, tm_raw, tm_gt, tm_rawn, tm_gtn, sa);
   return check_launch("fused_kernel");
 }
 
 template <int MODE>
-static int dispatch(const FusedArgs& a, const ChainDesc& d, int N, int dm_kind, cudaStream_t st, int* rows_per_frame) {
+static int dispatch(const FusedArgs& a, const ChainDesc& d, int N, int dm_kind, cudaStream_t st, int* rows_per_frame,
+                    const StoreArgs& sa = StoreArgs{}) {
   const unsigned sig = chain_signature(d);
-#define RISP_F_SIG(DMK, SG) if (sig == (SG)) return launch_one<DMK, MODE, (SG)>(a, d, N, st, rows_per_frame);
+#define RISP_F_SIG(DMK, SG) if (sig == (SG)) return launch_one<DMK, MODE, (SG)>(a, d, N, st, rows_per_frame, sa);
 #define RISP_F_DM(DMK) RISP_F_SIG(DMK, RISP_SIG_A) RISP_F_SIG(DMK, RISP_SIG_B) RISP_F_SIG(DMK, RISP_SIG_C) RISP_F_SIG(DMK, RISP_SIG_D) \
-  if constexpr (MODE == MODE_FWD || MODE == MODE_EVAL) { RISP_F_SIG(DMK, RISP_SIG_SKIP) }
+  if constexpr (MODE == MODE_FWD || is_eval(MODE)) { RISP_F_SIG(DMK, RISP_SIG_SKIP) }
   switch (dm_kind) {
     case RISP_DM_NEAREST: RISP_F_DM(RISP_DM_NEAREST) break;
     case RISP_DM_BILINEAR: RISP_F_DM(RISP_DM_BILINEAR) break;
@@ -1093,6 +1184,28 @@ int fused_eval_launch(const float* raw, const float* gt, unsigned char* u8, unsi
   if (rc != RISP_OK) return rc;
   const FusedArgs a{raw, gt, nullptr, nullptr, params, pstride, H, W, 0, 0, 0, 0, clip_hi, slot, u8, partial};
   return dispatch<MODE_EVAL>(a, d, N, dm_kind, st, rows_per_frame);
+}
+
+// evaluation mode reading frame stores: image n is raw frame pos[n].x (codes of raw_bpc bytes, decoded as code / white_level)
+// against the 8-bit planar GT frame pos[n].y.  Returns RISP_OK, an error, or 1 when the chain is not handled;
+// RISP_E_UNSUPPORTED when the stores cannot be described by tensor maps (rows of 16-byte multiples).
+int fused_eval_store_launch(const void* raw_store, int raw_bpc, int F, const unsigned char* gt_store, int G, const int* pos,
+                            int* status, float white_level, unsigned char* u8, unsigned long long* partial, const float* params,
+                            int pstride, int N, int H, int W, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st,
+                            int* rows_per_frame) {
+  using namespace fused;
+  if (!fused_handles(d, N, pstride, H, W)) return 1;
+  RISP_REQUIRE((long long)W * raw_bpc % 16 == 0 && W % 16 == 0 && aligned16(raw_store) && aligned16(gt_store),
+               RISP_E_UNSUPPORTED, "risp_pipeline_eval_store: the packed kernels read the stores through tensor maps, which need "
+               "16-byte aligned stores and rows of a 16-byte multiple (W %% 16 == 0), got W = %d", W);
+  int slot;
+  const int rc = prep_constants(params, pstride, N, d, st, &slot);
+  if (rc != RISP_OK) return rc;
+  const FusedArgs a{static_cast<const float*>(raw_store), reinterpret_cast<const float*>(gt_store), nullptr, nullptr, params,
+                    pstride, H, W, 0, 0, 0, 0, clip_hi, slot, u8, partial};
+  const StoreArgs sa{reinterpret_cast<const int4*>(pos), status, white_level, F, G};
+  return raw_bpc == 2 ? dispatch<MODE_EVAL_S16>(a, d, N, dm_kind, st, rows_per_frame, sa)
+                      : dispatch<MODE_EVAL_U8>(a, d, N, dm_kind, st, rows_per_frame, sa);
 }
 
 // mode: 0 forward, 1 MSE step, 2 backward with upstream dy, 3 L1 step.  Returns RISP_OK, an error, or 1 when the chain is not handled.

@@ -17,6 +17,7 @@
 #include "risp_stage.cuh"
 
 #include <stdlib.h>
+#include <type_traits>
 
 namespace risp {
 
@@ -44,6 +45,44 @@ __device__ __forceinline__ void row_issue(RawRow<HL>& q, const float* __restrict
     if (active && lane == 0 && c0 > 0) q.l = __ldg(reinterpret_cast<const float2*>(rp + c0 - 2));
     if (active && lane == 31 && c0 + 4 < W) q.r = __ldg(reinterpret_cast<const float2*>(rp + c0 + 4));
   }
+}
+
+// the same row out of a frame store of ES-byte codes (ES = 2: 16-bit, 1: 8-bit): the codes are loaded here and decoded in
+// row_decode, after the loads have been issued
+template <int HL> struct CodeRow { uint2 v; uint32_t l, r; };   // 4 codes (ES = 1: v.x only); HL halo codes each side
+template <int HL, int ES>
+__device__ __forceinline__ void row_issue_codes(CodeRow<HL>& q, const unsigned char* __restrict__ img, int row, int W, int c0,
+                                                bool active, int lane) {
+  const unsigned char* rp = img + (long long)row * W * ES;
+  q.v = make_uint2(0u, 0u); q.l = 0u; q.r = 0u;
+  if (active) {
+    if constexpr (ES == 2) q.v = __ldg(reinterpret_cast<const uint2*>(rp + 2 * c0));
+    else q.v.x = __ldg(reinterpret_cast<const uint32_t*>(rp + c0));
+  }
+  // HL codes at c0-HL and at c0+4: 2-byte aligned (c0 % 4 == 0)
+  auto ld = [&](int c) -> uint32_t {
+    if constexpr (ES == 2) return HL == 1 ? (uint32_t)__ldg(reinterpret_cast<const unsigned short*>(rp + 2 * c))
+                                          : __ldg(reinterpret_cast<const uint32_t*>(rp + 2 * c));
+    else return HL == 1 ? (uint32_t)__ldg(rp + c) : (uint32_t)__ldg(reinterpret_cast<const unsigned short*>(rp + c));
+  };
+  if (active && lane == 0 && c0 > 0) q.l = ld(c0 - HL);
+  if (active && lane == 31 && c0 + 4 < W) q.r = ld(c0 + 4);
+}
+template <int HL, int ES>
+__device__ __forceinline__ RawRow<HL> row_decode(const CodeRow<HL>& q, float wl) {
+  constexpr int B = 8 * ES;                 // bits per code
+  constexpr uint32_t M = (1u << B) - 1u;
+  RawRow<HL> o;
+  const uint32_t c1 = ES == 2 ? q.v.x >> 16 : (q.v.x >> 8) & M, c2 = ES == 2 ? q.v.y & M : (q.v.x >> 16) & M,
+                 c3 = ES == 2 ? q.v.y >> 16 : q.v.x >> 24;
+  o.v = make_float4(decode_code(q.v.x & M, wl), decode_code(c1, wl), decode_code(c2, wl), decode_code(c3, wl));
+  if constexpr (HL == 1) {
+    o.l = decode_code(q.l, wl); o.r = decode_code(q.r, wl);
+  } else {
+    o.l = make_float2(decode_code(q.l & M, wl), decode_code(q.l >> B, wl));
+    o.r = make_float2(decode_code(q.r & M, wl), decode_code(q.r >> B, wl));
+  }
+  return o;
 }
 
 // halo exchange: dst[0 .. 4+2*HL) = columns c0-HL .. c0+3+HL of the row
@@ -119,7 +158,10 @@ __device__ __forceinline__ void demosaic4(const float (&w)[2 * HL + 1][4 + 2 * H
 }
 
 // EVAL: the forward of MODE_FWD, then the squared 8-bit code differences to the GT (per-image PSNR numerator); writes no y
-enum { MODE_FWD = 0, MODE_STEP = 1, MODE_EVAL = 2 };
+// EVAL_S16 / EVAL_U8: EVAL reading a frame store (16-bit / 8-bit raw codes, 8-bit planar GT codes; frames named by records)
+enum { MODE_FWD = 0, MODE_STEP = 1, MODE_EVAL = 2, MODE_EVAL_S16 = 3, MODE_EVAL_U8 = 4 };
+constexpr bool is_store(int mode) { return mode == MODE_EVAL_S16 || mode == MODE_EVAL_U8; }
+constexpr bool is_eval(int mode) { return mode == MODE_EVAL || is_store(mode); }
 
 // packed-fp32 / constant-bank kernels for the pre-instantiated signatures (risp_fused.cu)
 bool fused_handles(const ChainDesc& d, int N, int param_stride, int H, int W);
@@ -129,6 +171,10 @@ int fused_launch(int mode, const float* raw, const float* gt, float* y, float* p
 int fused_eval_launch(const float* raw, const float* gt, unsigned char* u8, unsigned long long* partial, const float* params,
                       int pstride, int N, int H, int W, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st,
                       int* rows_per_frame);
+int fused_eval_store_launch(const void* raw_store, int raw_bpc, int F, const unsigned char* gt_store, int G, const int* pos,
+                            int* status, float white_level, unsigned char* u8, unsigned long long* partial, const float* params,
+                            int pstride, int N, int H, int W, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st,
+                            int* rows_per_frame);
 
 struct PipeArgs {
   const float* raw;   // (N,1,H,W)
@@ -142,6 +188,13 @@ struct PipeArgs {
   int gt_is_dy;       // MODE_STEP: `gt` holds dL/dy (container-level backward) instead of the target
   unsigned char* u8;  // MODE_EVAL: (N,H,W,3) 8-bit codes of y, nullable
   unsigned long long* sse;   // MODE_EVAL: [N][warps_per_image] sums of squared code differences
+  // store modes: image n is raw frame pos[n].x of `store` against the 8-bit planar GT frame pos[n].y of `gstore`
+  const unsigned char* store;
+  const unsigned char* gstore;
+  const int4* pos;
+  int* status;        // set when a record is not a whole frame of the stores; that image adds nothing
+  float white_level;
+  int F, G;
 };
 
 // resident CTAs per SM the kernels are compiled for (register cap)
@@ -154,7 +207,7 @@ constexpr int kPairUnroll = 2;
 
 template <int DM, int MODE, unsigned SIG, bool BIGG>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, (MODE == MODE_STEP) ? ((SIG == 0) ? 1 : kStepMinBlocks)
-                                                    : (MODE == MODE_EVAL) ? kEvalMinBlocks : kFwdMinBlocks)
+                                                    : is_eval(MODE) ? kEvalMinBlocks : kFwdMinBlocks)
 pipeline_kernel(PipeArgs a, ChainDesc d) {
   using SG = Sig<SIG>;
   constexpr int SMAX = SG::S;
@@ -170,7 +223,19 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
   const int ra = blockIdx.y * a.rows_per_chunk;
   const int rb = min(H, ra + a.rows_per_chunk);
   const long long plane = (long long)H * W;
-  const float* __restrict__ img = a.raw + (long long)n * plane;
+  constexpr bool ST = is_store(MODE);
+  constexpr int ES = (MODE == MODE_EVAL_S16) ? 2 : 1;      // store modes: bytes per raw code
+  bool ok = true;                                          // store modes: the record names a whole frame of the stores
+  const unsigned char* __restrict__ simg = nullptr;        // store modes: the raw frame's codes and the GT frame's planes
+  const unsigned char* __restrict__ sgt = nullptr;
+  if constexpr (ST) {
+    const int4 rec = a.pos[n];
+    ok = whole_frame_record(rec, a.F, a.G);
+    if (!ok && threadIdx.x == 0) *a.status = 1;
+    simg = a.store + (long long)(ok ? rec.x : 0) * plane * ES;
+    sgt = a.gstore + (long long)(ok ? rec.y : 0) * 3 * plane;
+  }
+  const float* __restrict__ img = ST ? nullptr : a.raw + (long long)n * plane;
   const float* __restrict__ prow = a.params + (long long)n * a.pstride;
   const float* __restrict__ gtb = (MODE != MODE_FWD) ? a.gt + (long long)n * 3 * plane : nullptr;
   float* __restrict__ yb = a.y ? a.y + (long long)n * 3 * plane : nullptr;
@@ -188,34 +253,48 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
     for (int k = 0; k < RISP_BIG_ACC; ++k) accB[k] = make_float2(0.f, 0.f);
   }
 
-  if (strip * kStripCols < W) {   // warp-uniform: the whole strip is outside the frame otherwise
+  if (strip * kStripCols < W && (!ST || ok)) {   // warp-uniform: the whole strip is outside the frame otherwise
     float w[WR][WC];
-    RawRow<HL> q;
+    std::conditional_t<ST, CodeRow<HL>, RawRow<HL>> q;     // store modes: codes, decoded when the row is finished
 #pragma unroll
     for (int j = 0; j < WR - 1; ++j) {
-      row_issue<HL>(q, img, reflect101(ra - HL + j, H), W, c0, active, lane);
-      row_finish<HL>(w[j], q, W, c0, active, lane);
+      if constexpr (ST) {
+        row_issue_codes<HL, ES>(q, simg, reflect101(ra - HL + j, H), W, c0, active, lane);
+        row_finish<HL>(w[j], row_decode<HL, ES>(q, a.white_level), W, c0, active, lane);
+      } else {
+        row_issue<HL>(q, img, reflect101(ra - HL + j, H), W, c0, active, lane);
+        row_finish<HL>(w[j], q, W, c0, active, lane);
+      }
     }
-    row_issue<HL>(q, img, reflect101(ra + HL, H), W, c0, active, lane);
+    if constexpr (ST) row_issue_codes<HL, ES>(q, simg, reflect101(ra + HL, H), W, c0, active, lane);
+    else row_issue<HL>(q, img, reflect101(ra + HL, H), W, c0, active, lane);
     float4 gB = make_float4(0.f, 0.f, 0.f, 0.f), gG = gB, gR = gB;   // GT of the row being computed, fetched one row ahead
     if (MODE == MODE_STEP && active) {
       const long long o = (long long)ra * W + c0;
       gB = ld_stream4(gtb + o); gG = ld_stream4(gtb + plane + o); gR = ld_stream4(gtb + 2 * plane + o);
     }
     for (int r = ra; r < rb; ++r) {
-      row_finish<HL>(w[WR - 1], q, W, c0, active, lane);
+      if constexpr (ST) row_finish<HL>(w[WR - 1], row_decode<HL, ES>(q, a.white_level), W, c0, active, lane);
+      else row_finish<HL>(w[WR - 1], q, W, c0, active, lane);
       const float4 tB = gB, tG = gG, tR = gR;
       float4 eB, eG, eR;         // MODE_EVAL: GT of this row
-      if constexpr (MODE == MODE_EVAL) {
+      [[maybe_unused]] uint32_t sB, sG, sR;   // store modes: its 4 codes per plane
+      if constexpr (is_eval(MODE)) {
         // requested before the demosaic and the chain it waits behind (a row-ahead prefetch as in MODE_STEP keeps two GT
         // rows live and spills)
         if (active) {
           const long long o = (long long)r * W + c0;
-          eB = ld_stream4(gtb + o); eG = ld_stream4(gtb + plane + o); eR = ld_stream4(gtb + 2 * plane + o);
+          if constexpr (ST) {
+            sB = __ldg(reinterpret_cast<const uint32_t*>(sgt + o)); sG = __ldg(reinterpret_cast<const uint32_t*>(sgt + plane + o));
+            sR = __ldg(reinterpret_cast<const uint32_t*>(sgt + 2 * plane + o));
+          } else {
+            eB = ld_stream4(gtb + o); eG = ld_stream4(gtb + plane + o); eR = ld_stream4(gtb + 2 * plane + o);
+          }
         }
       }
       if (r + 1 < rb) {
-        row_issue<HL>(q, img, reflect101(r + 1 + HL, H), W, c0, active, lane);
+        if constexpr (ST) row_issue_codes<HL, ES>(q, simg, reflect101(r + 1 + HL, H), W, c0, active, lane);
+        else row_issue<HL>(q, img, reflect101(r + 1 + HL, H), W, c0, active, lane);
         if (MODE == MODE_STEP && active) {
           const long long o = (long long)(r + 1) * W + c0;
           gB = ld_stream4(gtb + o); gG = ld_stream4(gtb + plane + o); gR = ld_stream4(gtb + 2 * plane + o);
@@ -223,14 +302,15 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
       }
       Px<4> px;
       demosaic4<DM, HL>(w, (r & 1) != 0, a.clip_hi, px);
-      if constexpr (MODE == MODE_EVAL) {
+      if constexpr (is_eval(MODE)) {
 #pragma unroll
         for (int s = 0; s < SMAX; ++s)
           if (SG::live(d, s)) stage_fwd(SG::op(d, s), SG::iarg(d, s), prow + d.off[s], px);
         if (active) {
           const float4 yB = make_float4(px.b[0], px.b[1], px.b[2], px.b[3]), yG = make_float4(px.g[0], px.g[1], px.g[2], px.g[3]),
                        yR = make_float4(px.r[0], px.r[1], px.r[2], px.r[3]);
-          sse += sq_codes4(yB, eB) + sq_codes4(yG, eG) + sq_codes4(yR, eR);
+          if constexpr (ST) sse += sq_codes4_u8(yB, sB) + sq_codes4_u8(yG, sG) + sq_codes4_u8(yR, sR);
+          else sse += sq_codes4(yB, eB) + sq_codes4(yG, eG) + sq_codes4(yR, eR);
           if (a.u8) {        // (H,W,3) BGR bytes of the lane's 4 pixels: 12 contiguous bytes, 4-byte aligned (c0 % 4 == 0)
             uint32_t b[4], g[4], rr[4];
 #pragma unroll
@@ -327,7 +407,7 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
     float v = warp_sum(loss);
     if (lane == 0) { out[RISP_SLOT_LOSS] = v; out[RISP_SLOT_LOSS + 1] = 0.f; }
   }
-  if constexpr (MODE == MODE_EVAL) {    // every warp writes its row, also one whose strip lies outside the frame
+  if constexpr (is_eval(MODE)) {    // every warp writes its row, also one whose strip lies outside the frame
     const int warps_per_image = gridDim.y * gridDim.x * kWarpsPerBlock;
     const int widx = (blockIdx.y * gridDim.x + blockIdx.x) * kWarpsPerBlock + wid;
     const unsigned long long v = warp_sum_u64(sse);
@@ -366,7 +446,7 @@ static int launch_pipeline(const PipeArgs& a, const ChainDesc& d, int N, int dm_
   bool done = false;
   // the evaluation mode has the generic instantiation only: the same stage_fwd arithmetic, 3 kernels instead of 15
 #define RISP_PIPE_SIG(DMK, SG)                                                       \
-  if constexpr (MODE != MODE_EVAL) {                                                 \
+  if constexpr (!is_eval(MODE)) {                                                    \
     if (!done && sig == (SG)) {                                                      \
       pipeline_kernel<DMK, MODE, (SG), false><<<grid, block, 0, st>>>(b, d);         \
       done = true;                                                                   \
@@ -376,7 +456,7 @@ static int launch_pipeline(const PipeArgs& a, const ChainDesc& d, int N, int dm_
   do {                                                                               \
     RISP_PIPE_SIG(DMK, RISP_SIG_A) RISP_PIPE_SIG(DMK, RISP_SIG_B) RISP_PIPE_SIG(DMK, RISP_SIG_C) RISP_PIPE_SIG(DMK, RISP_SIG_D) \
     if (!done) {                                                                     \
-      if constexpr (MODE == MODE_EVAL) pipeline_kernel<DMK, MODE, 0u, false><<<grid, block, 0, st>>>(b, d); \
+      if constexpr (is_eval(MODE)) pipeline_kernel<DMK, MODE, 0u, false><<<grid, block, 0, st>>>(b, d);    \
       else if (big) pipeline_kernel<DMK, MODE, 0u, true><<<grid, block, 0, st>>>(b, d); \
       else pipeline_kernel<DMK, MODE, 0u, false><<<grid, block, 0, st>>>(b, d);      \
     }                                                                                \
@@ -483,6 +563,60 @@ extern "C" int risp_pipeline_eval(const float* raw, const float* gt, unsigned ch
   if (rc == 1) {
     PipeArgs a{raw, gt, nullptr, nullptr, params, param_stride, H, W, 0, dm_clip_hi, 0, u8_out, partial};
     rc = launch_pipeline<MODE_EVAL>(a, d, N, dm_kind, false, st);
+    rows = pipe_geometry(N, H, W).warps_per_image;
+  }
+  if (rc != RISP_OK) return rc;
+  return finalize_sse(partial, sse_out, N, rows, st);
+}
+
+// risp_pipeline_eval on frames of stores of codes: image n is raw frame pos[n].x (decoded as the sampler decodes it) against
+// GT frame pos[n].y, whose codes are compared as they are.  The same dispatch as risp_pipeline_eval, so the codes and sums
+// are that entry point's on the decoded batch under either setting of RISP_FUSED.
+extern "C" int risp_pipeline_eval_store(const void* raw_store, int raw_bytes_per_code, int F, const unsigned char* gt_store,
+                                        int G, int H, int W, const int* pos, int N, float white_level, int* status,
+                                        unsigned char* u8_out, long long* sse_out, int dm_kind, float dm_clip_hi,
+                                        const int* ops, const int* param_off, const int* iarg, int S, const float* params,
+                                        int param_stride, void* workspace, size_t workspace_bytes, risp_stream_t stream) {
+  const char* who = "risp_pipeline_eval_store";
+  RISP_REQUIRE(raw_store && gt_store && pos && status && sse_out, RISP_E_INVALID,
+               "%s: raw_store, gt_store, pos, status and sse_out must be non-null", who);
+  RISP_REQUIRE(raw_bytes_per_code == 1 || raw_bytes_per_code == 2, RISP_E_INVALID, "%s: 1 or 2 bytes per raw code", who);
+  RISP_REQUIRE(F > 0 && G > 0 && N > 0 && N <= 65535 && H >= 4 && W >= 4 && white_level > 0.f, RISP_E_INVALID,
+               "%s: bad store arguments (F %d, G %d, N %d, %dx%d, white_level %g)", who, F, G, N, H, W, (double)white_level);
+  RISP_REQUIRE(H % 2 == 0 && W % 4 == 0, RISP_E_ALIGN, "%s: needs H even and W %% 4 == 0 (got %dx%d)", who, H, W);
+  RISP_REQUIRE((long long)F * H * W < (1ll << 40) && (long long)G * 3 * H * W < (1ll << 40), RISP_E_INVALID,
+               "%s: stores of %d / %d frames of %dx%d are too large", who, F, G, H, W);
+  RISP_REQUIRE(aligned16(raw_store) && aligned16(gt_store) && aligned16(pos), RISP_E_ALIGN,
+               "%s: raw_store, gt_store and pos must be 16-byte aligned", who);
+  RISP_REQUIRE((reinterpret_cast<uintptr_t>(sse_out) & 7u) == 0, RISP_E_ALIGN, "%s: sse_out must be 8-byte aligned", who);
+  RISP_REQUIRE((reinterpret_cast<uintptr_t>(u8_out) & 3u) == 0, RISP_E_ALIGN, "%s: u8_out must be 4-byte aligned", who);
+  RISP_REQUIRE(dm_kind == RISP_DM_NEAREST || dm_kind == RISP_DM_BILINEAR || dm_kind == RISP_DM_MALVAR, RISP_E_INVALID,
+               "%s: unknown demosaic kind %d", who, dm_kind);
+  ChainDesc d;
+  int P = 0;
+  int rc = make_chain(&d, ops, param_off, iarg, S, &P);
+  if (rc != RISP_OK) return rc;
+  RISP_REQUIRE(P == 0 || params, RISP_E_INVALID, "%s: chain needs %d parameters but params is null", who, P);
+  RISP_REQUIRE(param_stride == 0 || param_stride >= P, RISP_E_INVALID, "%s: param_stride %d < %d", who, param_stride, P);
+  RISP_REQUIRE(workspace, RISP_E_INVALID, "%s: workspace is null", who);
+  const size_t need = risp_pipeline_eval_workspace(N, H, W);
+  RISP_REQUIRE(workspace_bytes >= need, RISP_E_WORKSPACE, "%s: workspace %zu < %zu", who, workspace_bytes, need);
+  cudaStream_t st = as_stream(stream);
+  unsigned long long* partial = static_cast<unsigned long long*>(workspace);
+  int rows = 0;
+  rc = 1;
+  if (use_fused()) {
+    ChainDesc df = d;
+    if (S == 0) { df.S = 1; df.op[0] = RISP_OP_SKIP; df.off[0] = 0; df.iarg[0] = 0; }     // demosaic only
+    rc = fused_eval_store_launch(raw_store, raw_bytes_per_code, F, gt_store, G, pos, status, white_level, u8_out, partial,
+                                 params, param_stride, N, H, W, dm_kind, dm_clip_hi, df, st, &rows);
+  }
+  if (rc == 1) {
+    PipeArgs a{nullptr, nullptr, nullptr, nullptr, params, param_stride, H, W, 0, dm_clip_hi, 0, u8_out, partial,
+               static_cast<const unsigned char*>(raw_store), gt_store, reinterpret_cast<const int4*>(pos), status,
+               white_level, F, G};
+    rc = raw_bytes_per_code == 2 ? launch_pipeline<MODE_EVAL_S16>(a, d, N, dm_kind, false, st)
+                                 : launch_pipeline<MODE_EVAL_U8>(a, d, N, dm_kind, false, st);
     rows = pipe_geometry(N, H, W).warps_per_image;
   }
   if (rc != RISP_OK) return rc;

@@ -27,12 +27,14 @@ constexpr float kC2 = 137644.92f;         // 49 * 48 (0.03 * 255)^2
 __device__ __forceinline__ float comp(const float4& v, int i) { return i == 0 ? v.x : i == 1 ? v.y : i == 2 ? v.z : v.w; }
 __device__ __forceinline__ int byte_of(uint32_t w, int j) { return (int)__byte_perm(w, 0u, 0x4440u | (uint32_t)j); }
 
-// One row of a lane's 4 columns, as loaded: gt (fp32) for KC channels, and y as fp32 (NCHW), as the 12 interleaved bytes of
-// 4 BGR pixels (NHWC, vector path, KC == 3) or as one word of 4 codes per channel (NHWC, scalar path).
-template <int LAYOUT, int KC, bool VEC>
+// One row of a lane's 4 columns, as loaded: gt (fp32, or with GS one word of 4 codes of a frame store) for KC channels, and y
+// as fp32 (NCHW), as the 12 interleaved bytes of 4 BGR pixels (NHWC, vector path, KC == 3) or as one word of 4 codes per
+// channel (NHWC, scalar path).
+template <int LAYOUT, int KC, bool VEC, bool GS>
 struct Row {
   static constexpr bool kU8 = LAYOUT == RISP_IMG_U8_NHWC;
-  float4 g[KC];
+  float4 g[GS ? 1 : KC];
+  uint32_t g8[GS ? KC : 1];
   float4 yf[kU8 ? 1 : KC];
   uint32_t y8[kU8 ? (VEC ? 3 : KC) : 1];
 };
@@ -45,14 +47,30 @@ __device__ __forceinline__ float4 ld4(const float* __restrict__ row, int c, int 
   return make_float4(ld_or0(row, c, W), ld_or0(row, c + 1, W), ld_or0(row, c + 2, W), ld_or0(row, c + 3, W));
 }
 
-// Row q, columns [c, c+4) (c % 4 == 0), channels ch0 .. ch0+KC-1 of image n.  Columns outside the frame read 0; they only
-// feed lanes whose outputs lie outside the interior.  With VEC (W % 4 == 0, aligned operands) a lane is wholly inside or
-// wholly outside the frame.
-template <int LAYOUT, int KC, bool VEC>
-__device__ __forceinline__ void load_row(Row<LAYOUT, KC, VEC>& r, const void* __restrict__ y, const float* __restrict__ gt,
-                                         long long n, int ch0, int C, int H, int W, int q, int c) {
+// Row q, columns [c, c+4) (c % 4 == 0), channels ch0 .. ch0+KC-1 of image n (with GS: gt is the GT store and gn the frame
+// of image n in it).  Columns outside the frame read 0; they only feed lanes whose outputs lie outside the interior.  With VEC
+// (W % 4 == 0, aligned operands) a lane is wholly inside or wholly outside the frame.
+template <int LAYOUT, int KC, bool VEC, bool GS>
+__device__ __forceinline__ void load_row(Row<LAYOUT, KC, VEC, GS>& r, const void* __restrict__ y, const float* __restrict__ gt,
+                                         long long n, long long gn, int ch0, int C, int H, int W, int q, int c) {
+  if constexpr (GS) {
 #pragma unroll
-  for (int k = 0; k < KC; ++k) r.g[k] = ld4(gt + (((n * C + ch0 + k) * H) + q) * (long long)W, c, W, VEC);
+    for (int k = 0; k < KC; ++k) {
+      const unsigned char* __restrict__ row = reinterpret_cast<const unsigned char*>(gt) + (((gn * C + ch0 + k) * H) + q) * (long long)W;
+      uint32_t w = 0;
+      if constexpr (VEC) {
+        if (c >= 0 && c < W) w = __ldg(reinterpret_cast<const uint32_t*>(row + c));
+      } else {
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+          if (c + i >= 0 && c + i < W) w |= (uint32_t)__ldg(row + c + i) << (8 * i);
+      }
+      r.g8[k] = w;
+    }
+  } else {
+#pragma unroll
+    for (int k = 0; k < KC; ++k) r.g[k] = ld4(gt + (((n * C + ch0 + k) * H) + q) * (long long)W, c, W, VEC);
+  }
   if constexpr (LAYOUT == RISP_IMG_F32_NCHW) {
 #pragma unroll
     for (int k = 0; k < KC; ++k)
@@ -79,14 +97,18 @@ __device__ __forceinline__ void load_row(Row<LAYOUT, KC, VEC>& r, const void* __
 }
 
 // the codes of channel k, column i of a loaded row
-template <int LAYOUT, int KC, bool VEC>
-__device__ __forceinline__ int code_y(const Row<LAYOUT, KC, VEC>& r, int k, int i) {
+template <int LAYOUT, int KC, bool VEC, bool GS>
+__device__ __forceinline__ int code_y(const Row<LAYOUT, KC, VEC, GS>& r, int k, int i) {
   if constexpr (LAYOUT == RISP_IMG_F32_NCHW) return u8_code(comp(r.yf[k], i));
   else if constexpr (VEC) return byte_of(r.y8[(3 * i + k) >> 2], (3 * i + k) & 3);
   else return byte_of(r.y8[k], i);
 }
-template <int LAYOUT, int KC, bool VEC>
-__device__ __forceinline__ int code_g(const Row<LAYOUT, KC, VEC>& r, int k, int i) { return u8_code(comp(r.g[k], i)); }
+// a stored GT code is its own tensor2bgr code (trunc(clip(fl32(fl32(c/255)*255), 0, 255)) == c for all 256 codes)
+template <int LAYOUT, int KC, bool VEC, bool GS>
+__device__ __forceinline__ int code_g(const Row<LAYOUT, KC, VEC, GS>& r, int k, int i) {
+  if constexpr (GS) return byte_of(r.g8[k], i);
+  else return u8_code(comp(r.g[k], i));
+}
 
 // 7-wide window sums of a per-column quantity: columns i-3 .. i+3 of the lane's 4 columns, the outer ones from the
 // neighbouring lanes (their suffix / prefix sums).  Lanes 0 and 31 receive their own values; they produce no output.
@@ -118,14 +140,25 @@ __device__ __forceinline__ long long ssim_fixed(int s, int q, int x) {
 // grid (cdiv(strips, kWarps), min(chunks * groups, 65535), N); groups = C / KC channel groups.  Work item t of blockIdx.y's
 // stride is (row chunk t / groups, channel group t % groups): the channel groups of one chunk are neighbours, so with
 // KC < C on the NHWC operand the other channels' bytes are still in L2.
-template <int LAYOUT, int KC, bool VEC>
+// GS: gt is a store of G frames of 8-bit planar codes and image n is scored against frame pos[n].y (a record that is not a
+// whole frame of the store sets *status and adds nothing).
+template <int LAYOUT, int KC, bool VEC, bool GS>
 __global__ void __launch_bounds__(kWarps * 32)
 ssim_u8_kernel(const void* __restrict__ y, const float* __restrict__ gt, unsigned long long* __restrict__ out, int C, int H,
-               int W, int strips, int rows_per_chunk, int items) {
+               int W, int strips, int rows_per_chunk, int items, const int4* __restrict__ pos, int G, int* status) {
   const int lane = threadIdx.x & 31;
   const int strip = blockIdx.x * kWarps + (threadIdx.x >> 5);
   if (strip >= strips) return;                                      // whole warps only
   const long long n = blockIdx.z;
+  long long gn = n;
+  if constexpr (GS) {
+    const int4 rec = pos[n];
+    if (rec.y < 0 || rec.y >= G || rec.z != 0 || rec.w != 0) {
+      if (threadIdx.x == 0) *status = 1;
+      return;
+    }
+    gn = rec.y;
+  }
   const int groups = C / KC;
   const int c = strip * kOutCols - 4 + lane * 4;                    // first of the lane's 4 columns
   bool valid[4];                                                    // interior output columns of this lane
@@ -140,9 +173,9 @@ ssim_u8_kernel(const void* __restrict__ y, const float* __restrict__ gt, unsigne
     for (int k = 0; k < KC; ++k)
 #pragma unroll
       for (int i = 0; i < 4; ++i) vs[k][i] = vq[k][i] = vx[k][i] = 0;
-    Row<LAYOUT, KC, VEC> rin, rout;
+    Row<LAYOUT, KC, VEC, GS> rin, rout;
     for (int d = -3; d <= 3; ++d) {
-      load_row(rin, y, gt, n, ch0, C, H, W, ra + d, c);
+      load_row(rin, y, gt, n, gn, ch0, C, H, W, ra + d, c);
 #pragma unroll
       for (int k = 0; k < KC; ++k)
 #pragma unroll
@@ -156,8 +189,8 @@ ssim_u8_kernel(const void* __restrict__ y, const float* __restrict__ gt, unsigne
     for (int r = ra; r < rb; ++r) {
       const bool more = r + 1 < rb;
       if (more) {                                                   // in flight while row r is scored
-        load_row(rin, y, gt, n, ch0, C, H, W, r + 4, c);
-        load_row(rout, y, gt, n, ch0, C, H, W, r - 3, c);
+        load_row(rin, y, gt, n, gn, ch0, C, H, W, r + 4, c);
+        load_row(rout, y, gt, n, gn, ch0, C, H, W, r - 3, c);
       }
 #pragma unroll
       for (int k = 0; k < KC; ++k) {
@@ -189,8 +222,9 @@ ssim_u8_kernel(const void* __restrict__ y, const float* __restrict__ gt, unsigne
   if (lane == 0 && acc != 0) atomicAdd(out + n, acc);               // integer addition: exact in any order
 }
 
-template <int LAYOUT, int KC, bool VEC>
-static int launch(const void* y, const float* gt, long long* out, int N, int C, int H, int W, cudaStream_t st) {
+template <int LAYOUT, int KC, bool VEC, bool GS = false>
+static int launch(const void* y, const float* gt, long long* out, int N, int C, int H, int W, cudaStream_t st,
+                  const int4* pos = nullptr, int G = 0, int* status = nullptr) {
   const int strips = (int)cdiv(W - 3, kOutCols), bx = (int)cdiv(strips, kWarps), groups = C / KC;
   // about 32 warps per SM over the whole batch, at least kMinRows rows per chunk (a chunk start costs 6 extra rows)
   const long long want = cdiv((long long)sm_count() * 32, (long long)strips * N * groups);
@@ -198,8 +232,8 @@ static int launch(const void* y, const float* gt, long long* out, int N, int C, 
   if (rows < kMinRows) rows = kMinRows;
   const long long items = cdiv(H - 6, rows) * (long long)groups;     // <= C (H-6) < 2^31
   const unsigned gy = (unsigned)(items < 65535 ? items : 65535);
-  ssim_u8_kernel<LAYOUT, KC, VEC><<<dim3((unsigned)bx, gy, (unsigned)N), kWarps * 32, 0, st>>>(
-      y, gt, reinterpret_cast<unsigned long long*>(out), C, H, W, strips, rows, (int)items);
+  ssim_u8_kernel<LAYOUT, KC, VEC, GS><<<dim3((unsigned)bx, gy, (unsigned)N), kWarps * 32, 0, st>>>(
+      y, gt, reinterpret_cast<unsigned long long*>(out), C, H, W, strips, rows, (int)items, pos, G, status);
   return check_launch("ssim_u8_kernel");
 }
 
@@ -238,4 +272,34 @@ extern "C" int risp_ssim_u8(const void* y, int y_layout, const float* gt, long l
                                  : ssim::launch<RISP_IMG_U8_NHWC, 3, false>(y, gt, ssim_sum_out, N, C, H, W, st);
   }
   return ssim::launch<RISP_IMG_U8_NHWC, 1, false>(y, gt, ssim_sum_out, N, C, H, W, st);
+}
+
+extern "C" int risp_ssim_u8_store(const void* y, int y_layout, const unsigned char* gt_store, int G, const int* pos, int* status,
+                                  long long* ssim_sum_out, int N, int H, int W, risp_stream_t stream) {
+  RISP_REQUIRE(y && gt_store && pos && status && ssim_sum_out, RISP_E_INVALID,
+               "risp_ssim_u8_store: y, gt_store, pos, status and ssim_sum_out must be non-null");
+  RISP_REQUIRE(y_layout == RISP_IMG_F32_NCHW || y_layout == RISP_IMG_U8_NHWC, RISP_E_INVALID,
+               "risp_ssim_u8_store: unknown y_layout %d", y_layout);
+  RISP_REQUIRE(N >= 1 && N <= 65535 && G >= 1, RISP_E_INVALID, "risp_ssim_u8_store: batch %d outside [1, 65535] or G = %d", N, G);
+  RISP_REQUIRE(H >= 7 && W >= 7, RISP_E_INVALID, "risp_ssim_u8_store: the 7x7 window needs H and W >= 7, got %d x %d", H, W);
+  RISP_REQUIRE(3ll * (H - 6) * (W - 6) < (1ll << 31), RISP_E_INVALID,
+               "risp_ssim_u8_store: 3 (H-6)(W-6) = %lld interior values must stay below 2^31", 3ll * (H - 6) * (W - 6));
+  const uintptr_t py = reinterpret_cast<uintptr_t>(y), pg = reinterpret_cast<uintptr_t>(gt_store);
+  RISP_REQUIRE((y_layout != RISP_IMG_F32_NCHW || (py & 3u) == 0) && (reinterpret_cast<uintptr_t>(ssim_sum_out) & 7u) == 0 &&
+                   aligned16(pos),
+               RISP_E_ALIGN, "risp_ssim_u8_store: fp32 y must be 4-byte, ssim_sum_out 8-byte and pos 16-byte aligned");
+  cudaStream_t st = as_stream(stream);
+  if (cudaMemsetAsync(ssim_sum_out, 0, sizeof(long long) * (size_t)N, st) != cudaSuccess) {
+    set_error("risp_ssim_u8_store: memset failed");
+    return RISP_E_CUDA;
+  }
+  // vector loads: every GT row starts on a 4-byte boundary and every fp32 / NHWC row of y on a 16- / 4-byte one
+  const bool vec = W % 4 == 0 && (pg & 3u) == 0;
+  const float* gt = reinterpret_cast<const float*>(gt_store);
+  const int4* p = reinterpret_cast<const int4*>(pos);
+  if (y_layout == RISP_IMG_F32_NCHW)
+    return vec && (py & 15u) == 0 ? ssim::launch<RISP_IMG_F32_NCHW, 1, true, true>(y, gt, ssim_sum_out, N, 3, H, W, st, p, G, status)
+                                  : ssim::launch<RISP_IMG_F32_NCHW, 1, false, true>(y, gt, ssim_sum_out, N, 3, H, W, st, p, G, status);
+  return vec && (py & 3u) == 0 ? ssim::launch<RISP_IMG_U8_NHWC, 3, true, true>(y, gt, ssim_sum_out, N, 3, H, W, st, p, G, status)
+                               : ssim::launch<RISP_IMG_U8_NHWC, 3, false, true>(y, gt, ssim_sum_out, N, 3, H, W, st, p, G, status);
 }

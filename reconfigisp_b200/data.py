@@ -9,6 +9,7 @@ plan -- B records of 16 bytes -- crosses PCIe per batch.
     ds = DeviceDataset(raws, gts, white_level=1023., crop=224, rank=rank, world=world)
     model.feed_data(ds.sample(8, 'all'))                        # tuning (IspModel): every frame of the shard
     model.feed_data(ds.sample(4) + ds.sample(4, 'val'))         # search (DartsModel): DARTS train / validation halves
+    frames, sse = ds.evaluate(net, 'val')                       # validation: every frame of the split, whole, once
 
 PNG decode stays on the host (cv2), once per frame, before the store is built.  The reference's dataset classes, file
 layouts and augmentation are not reproduced.  The SID loader's exposure-ratio amplification (sid_sony_ratio_...) is not
@@ -16,8 +17,9 @@ applied either: its formula is not recorded in this repository, so a caller that
 """
 import numpy as np
 import torch
+import torch.distributed as tdist
 
-from . import ops
+from . import dist, ops
 
 SPLITS = ('train', 'val', 'all')
 
@@ -54,7 +56,7 @@ class SamplingPlan:
         self._raw_slot = {int(f): k for k, f in enumerate(self.raw_frames)}
         self._gt_of = np.searchsorted(self.gt_frames, pairs[self.raw_frames]).astype(np.int32)   # raw slot -> GT slot
         half = n_frames // 2
-        spans = {'train': (0, half), 'val': (half, n_frames), 'all': (0, n_frames)}
+        self.spans = spans = {'train': (0, half), 'val': (half, n_frames), 'all': (0, n_frames)}
         self.shards = {s: np.array([self._raw_slot[int(f)] for f in self.raw_frames if lo <= f < hi], dtype=np.int64)
                        for s, (lo, hi) in spans.items()}
         self._perm = {}
@@ -68,6 +70,17 @@ class SamplingPlan:
                 self._perm.clear()
             self._perm[key] = self.shards[split][rng.permutation(len(self.shards[split]))]
         return self._perm[key]
+
+    def frames(self, split):
+        """This rank's frames of `split`, each once, in ascending global order -> (records int32 (n,4) = (raw slot, GT slot,
+        0, 0): whole frames; global frame indices int64 (n,))."""
+        if split not in SPLITS:
+            raise ValueError('split must be one of %s, got %r' % (SPLITS, split))
+        slots = self.shards[split]
+        out = np.zeros((len(slots), 4), dtype=np.int32)
+        out[:, 0] = slots
+        out[:, 1] = self._gt_of[slots]
+        return out, self.raw_frames[slots]
 
     def plan(self, split, step, B):
         """Records of batch `step` of B crops from `split`: int32 (B,4) = (raw slot, GT slot, y0, x0)."""
@@ -162,6 +175,8 @@ class DeviceDataset:
         self._upload(raw_list, gt_list, hwc)
         self.steps = {s: 0 for s in SPLITS}
         self._bufs = {}
+        self._eval = {}          # evaluate(): per split, the records on the device and where they land in the gathered result
+        self._eval_bufs = {}
 
     def _upload(self, raw_list, gt_list, hwc):
         if not torch.cuda.is_available():
@@ -212,3 +227,87 @@ class DeviceDataset:
         if bad:
             self.status.zero_()
             raise RuntimeError('risp_sample_crops skipped a record that was out of range or odd')
+
+    def _eval_records(self, split):
+        ev = self._eval.get(split)
+        if ev is None:
+            p = self.plan_
+            recs, _ = p.frames(split)
+            pos = torch.zeros((max(1, len(recs)), 4), device=self.device, dtype=torch.int32)
+            if len(recs):
+                pos[:len(recs)].copy_(torch.from_numpy(recs), non_blocking=True)
+            # rank r holds the frames f = r (mod world) of [lo, hi), ascending: its m-th result is frame lo + place[r][m]
+            lo, hi = p.spans[split]
+            place = np.concatenate([np.arange(lo + (r - lo) % p.world, hi, p.world) - lo for r in range(p.world)])
+            where = torch.from_numpy(place.astype(np.int64)).to(self.device, non_blocking=True)
+            ev = self._eval[split] = (pos, len(recs), where)
+        return ev
+
+    def evaluate(self, net, split='val', batch=4, ssim=False):
+        """Score `net` (a pipeline module, or a model holding one as `netG`) on every frame of `split`, whole, once, as the
+        reference's validation does -> (frames, sse) or with ssim=True (frames, sse, ssim_sums): int64 CUDA tensors over the
+        whole split (all ranks), in global frame order.  `metrics.psnr_from_sse(sse, 3*H*W)` and
+        `metrics.ssim_from_sums(ssim_sums, 3, H, W)` turn them into per-frame PSNR / SSIM; nothing here waits for the device.
+
+        When the pipeline is one fused head (skip-only segments aside) and W % 16 == 0, the pipeline kernels read the store's
+        codes directly (`ops.pipeline_eval_store`, `ops.ssim_u8_store`: 5 B/px with a 16-bit raw).  Otherwise each batch of
+        whole frames is decoded by `ops.sample_crops` into a persistent fp32 batch and scored by `net.evaluate`; both give the
+        same sums.  Runs under no_grad and leaves the parameters, `sample()` and its buffers and `steps` alone.  Under data
+        parallelism every rank scores its shard and the sums are all-gathered: every rank returns the same tensors.  A bad
+        record shows up through `check()`."""
+        net = getattr(net, 'netG', net)
+        if split not in SPLITS:
+            raise ValueError('split must be one of %s, got %r' % (SPLITS, split))
+        if batch < 1:
+            raise ValueError('batch must be positive, got %r' % (batch,))
+        lo, hi = self.plan_.spans[split]
+        if hi == lo:
+            raise ValueError("the '%s' split holds no frame" % split)
+        pos, n, where = self._eval_records(split)
+        H, W = self.H, self.W
+        sums = torch.zeros((2 if ssim else 1, n), device=self.device, dtype=torch.int64)
+        head = net.store_eval_plan() if hasattr(net, 'store_eval_plan') else None
+        with torch.no_grad():
+            if head is not None and W % 16 == 0:
+                dm_kind, chain, table = head
+                u8 = None
+                if ssim:
+                    u8 = self._eval_bufs.get('u8')
+                    if u8 is None or u8.shape[0] < batch:
+                        u8 = self._eval_bufs['u8'] = torch.empty((batch, H, W, 3), device=self.device, dtype=torch.uint8)
+                for i in range(0, n, batch):
+                    b = min(batch, n - i)
+                    p = pos[i:i + b]
+                    img8 = u8[:b] if ssim else None
+                    ops.pipeline_eval_store(self.raw_store, self.gt_store, p, self.white_level, self.status, dm_kind, chain,
+                                            table, u8=ssim, sse_out=sums[0, i:i + b], u8_out=img8)
+                    if ssim:
+                        ops.ssim_u8_store(img8, self.gt_store, p, self.status, out=sums[1, i:i + b])
+            else:
+                bufs = self._eval_bufs.get('f32')
+                if bufs is None or bufs[0].shape[0] < batch:
+                    bufs = self._eval_bufs['f32'] = (torch.empty((batch, 1, H, W), device=self.device, dtype=torch.float32),
+                                                     torch.empty((batch, 3, H, W), device=self.device, dtype=torch.float32))
+                for i in range(0, n, batch):
+                    b = min(batch, n - i)
+                    img, gt = bufs[0][:b], bufs[1][:b]
+                    ops.sample_crops(self.raw_store, self.gt_store, pos[i:i + b], H, W, self.white_level, self.status, img, gt)
+                    res = net.evaluate(img, gt, ssim=ssim)
+                    sums[0, i:i + b].copy_(res[0])
+                    if ssim:
+                        sums[1, i:i + b].copy_(res[2])
+        world = self.plan_.world
+        if world > 1:
+            if not dist.is_dist() or tdist.get_world_size() != world:
+                raise RuntimeError('evaluate: a dataset sharded over %d ranks needs torch.distributed with that world' % world)
+            m = -(-(hi - lo) // world)                     # the largest shard: shards differ by one frame at most
+            mine = torch.zeros((sums.shape[0], m), device=self.device, dtype=torch.int64)
+            mine[:, :n] = sums
+            parts = [torch.empty_like(mine) for _ in range(world)]
+            tdist.all_gather(parts, mine)
+            sizes = [len(range(lo + (r - lo) % world, hi, world)) for r in range(world)]
+            sums = torch.cat([q[:, :k] for q, k in zip(parts, sizes)], dim=1)
+        out = torch.empty_like(sums)
+        out[:, where] = sums
+        frames = torch.arange(lo, hi, device=self.device, dtype=torch.int64)
+        return (frames, out[0], out[1]) if ssim else (frames, out[0])

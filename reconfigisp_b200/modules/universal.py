@@ -256,6 +256,19 @@ class _Universal(nn.Module):
             img = torch.stack([ops.to_u8_hwc(y[n]) for n in range(y.shape[0])]) if u8 else None
             return (sse, img, ops.ssim_u8(y, gt)) if ssim else (sse, img)
 
+    def store_eval_plan(self):
+        """If the fused pipeline is [skip*] + one fused head (demosaic + per-pixel stages), returns (dm_kind, chain, params
+        table) for `ops.pipeline_eval_store` (what `DeviceDataset.evaluate` runs on the frame store); else None."""
+        if not self.fuse:
+            return None
+        if self._plan is None:
+            self._plan = self._make_plan()
+        segs = [s for s in self._plan if not (s[0] == 'chain' and not s[2])]
+        if len(segs) == 1 and segs[0][0] == 'head':
+            _, idx, keep, chain = segs[0]
+            return self.all_modules[idx].demosaic_kind, chain, self._segment_table(keep, 1)
+        return None
+
     # -- the whole proxy-tuning step in one pass (isp_model.py:128-142) ----------------------------------------
     def fused_mse_step_plan(self):
         """If the pipeline is [skip*] + classical demosaic + differentiable per-pixel stages, returns

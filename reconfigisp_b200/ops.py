@@ -712,6 +712,69 @@ def pipeline_eval(raw, gt, dm_kind, chain, params=None, clip_hi=1.0, u8=False):
     return sse, out8
 
 
+def _store_args(raw_store, gt_store, pos, status, who):
+    if raw_store.dtype not in (torch.uint8, torch.int16) or raw_store.dim() != 3:
+        raise ValueError('%s: raw codes must be uint8 or int16 (F,H,W), got %s %s' % (who, raw_store.dtype, tuple(raw_store.shape)))
+    F, H, W = raw_store.shape
+    if gt_store.dtype != torch.uint8 or tuple(gt_store.shape[1:]) != (3, H, W):
+        raise ValueError('%s: gt_store must be uint8 (G,3,%d,%d), got %s %s' % (who, H, W, gt_store.dtype, tuple(gt_store.shape)))
+    if pos.dtype != torch.int32 or pos.dim() != 2 or pos.shape[1] != 4:
+        raise ValueError('%s: pos must be int32 (N,4), got %s %s' % (who, pos.dtype, tuple(pos.shape)))
+    if status.dtype != torch.int32 or status.numel() < 1:
+        raise ValueError('%s: status must be an int32 tensor' % who)
+    return F, H, W
+
+
+def pipeline_eval_store(raw_store, gt_store, pos, white_level, status, dm_kind, chain, params=None, clip_hi=1.0, u8=False,
+                        sse_out=None, u8_out=None):
+    """`pipeline_eval` on whole frames of the stores of `sample_crops`, read as codes (`risp_pipeline_eval_store`):
+    image n is raw frame pos[n,0] / white_level against GT frame pos[n,1], pos (N,4) int32 CUDA records (raw frame, GT
+    frame, 0, 0).  -> (sse, u8_or_None), the values `pipeline_eval` gives on the batch `sample_crops` decodes from the same
+    records, written into sse_out / u8_out when given.  A bad record sets status (its sse is 0); nothing waits for the device."""
+    F, H, W = _store_args(raw_store, gt_store, pos, status, 'pipeline_eval_store')
+    N = pos.shape[0]
+    tab, stride = _param_table(params.detach(), N, chain.P) if chain.P else (None, 0)
+    sse = torch.empty((N,), device=raw_store.device, dtype=torch.int64) if sse_out is None else sse_out
+    out8 = None
+    if u8:
+        out8 = torch.empty((N, H, W, 3), device=raw_store.device, dtype=torch.uint8) if u8_out is None else u8_out
+    if tuple(sse.shape) != (N,) or sse.dtype != torch.int64 or (out8 is not None and (tuple(out8.shape) != (N, H, W, 3) or out8.dtype != torch.uint8)):
+        raise ValueError('pipeline_eval_store: outputs must be int64 (%d,) and uint8 (%d,%d,%d,3)' % (N, N, H, W))
+    ws = L.workspace(L.size('risp_pipeline_eval_workspace', N, H, W), raw_store.device)
+    L.call('risp_pipeline_eval_store', L.ptr(raw_store), raw_store.element_size(), F, L.ptr(gt_store), gt_store.shape[0], H, W,
+           L.ptr(pos), N, float(white_level), L.ptr(status), L.ptr(out8), L.ptr(sse), DM[dm_kind], float(clip_hi),
+           *chain.desc(), L.ptr(tab), stride, L.ptr(ws), ws.numel() * 4, L.stream())
+    return sse, out8
+
+
+def ssim_u8_store(y, gt_store, pos, status, out=None):
+    """`ssim_u8` of y against GT frames of a store (`risp_ssim_u8_store`): image n against frame pos[n,1] of gt_store (G,3,H,W)
+    uint8, the same bits as `ssim_u8` with the decoded fp32 GT.  y: the uint8 (N,H,W,3) image of `pipeline_eval_store` or
+    fp32 (N,3,H,W).  -> int64 (N,) CUDA sums (into out when given).  A bad record sets status (its sum is 0)."""
+    y = y.detach()
+    if pos.dtype != torch.int32 or pos.dim() != 2 or pos.shape[1] != 4:
+        raise ValueError('ssim_u8_store: pos must be int32 (N,4), got %s %s' % (pos.dtype, tuple(pos.shape)))
+    if status.dtype != torch.int32 or status.numel() < 1:
+        raise ValueError('ssim_u8_store: status must be an int32 tensor')
+    N = pos.shape[0]
+    G, _, H, W = gt_store.shape
+    if gt_store.dtype != torch.uint8 or gt_store.shape[1] != 3:
+        raise ValueError('ssim_u8_store: gt_store must be uint8 (G,3,H,W), got %s %s' % (gt_store.dtype, tuple(gt_store.shape)))
+    if y.dtype == torch.uint8:
+        if tuple(y.shape) != (N, H, W, 3):
+            raise ValueError('ssim_u8_store: the 8-bit y must be (N,H,W,3) = %s, got %s' % ((N, H, W, 3), tuple(y.shape)))
+        layout = L.ENUMS['RISP_IMG_U8_NHWC']
+    else:
+        y, layout = _img(y, 3), L.ENUMS['RISP_IMG_F32_NCHW']
+        if tuple(y.shape) != (N, 3, H, W):
+            raise ValueError('ssim_u8_store: y must be (%d,3,%d,%d), got %s' % (N, H, W, tuple(y.shape)))
+    if H < 7 or W < 7:
+        raise ValueError('ssim_u8_store: the 7x7 window needs H and W >= 7, got %d x %d' % (H, W))
+    out = torch.empty((N,), device=gt_store.device, dtype=torch.int64) if out is None else out
+    L.call('risp_ssim_u8_store', L.ptr(y), layout, L.ptr(gt_store), G, L.ptr(pos), L.ptr(status), L.ptr(out), N, H, W, L.stream())
+    return out
+
+
 class PipelineStep:
     """Pre-allocated state for repeated proxy-tuning steps on frames of one geometry."""
 
