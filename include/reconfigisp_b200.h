@@ -172,6 +172,29 @@ int risp_pipeline_l1_step(const float* raw, const float* gt, float* y_out, float
                           int param_stride, int P, void* workspace, size_t workspace_bytes,
                           risp_stream_t stream);
 
+/* risp_pipeline_mse_step / risp_pipeline_l1_step on N crops of h x w out of the frame stores of risp_sample_crops, read as
+ * codes (5 B/px with a 16-bit raw instead of the 16 B/px of a decoded batch).  Image n is the crop at (pos[n].z, pos[n].w) of
+ * raw frame pos[n].x, decoded in registers as code / white_level with the sampler's correctly rounded division, against the
+ * same crop of GT frame pos[n].y, decoded as code / 255.  loss_out and dparams are those of risp_pipeline_mse_step /
+ * risp_pipeline_l1_step on the batch risp_sample_crops decodes from the same records, bit for bit, with the same dispatch
+ * (RISP_FUSED=0 included); no image is written.
+ *   Stores: raw (F,H,W) of raw_bytes_per_code (1 or 2) byte codes, gt (G,3,H,W) 8-bit planar, as risp_pipeline_eval_store.
+ *   pos: DEVICE int32 [N][4] = (raw frame, GT frame, y0, x0), 16-byte aligned.  A record whose frames lie outside a store,
+ *   whose origin is odd or whose crop leaves the frame (the rule of risp_sample_crops) sets *status (DEVICE int32) and adds
+ *   nothing to the loss or to any gradient (the normaliser stays N*3*h*w); nothing outside the stores is read.
+ *   Geometry: W % 16 == 0 (the stores are read through tensor maps, rows of a 16-byte multiple), 16-byte aligned stores and
+ *   pos, w % 4 == 0 and h even; RISP_E_UNSUPPORTED otherwise.  Workspace: risp_pipeline_step_workspace(N, h, w, P). */
+int risp_pipeline_mse_step_store(const void* raw_store, int raw_bytes_per_code, int F, const unsigned char* gt_store, int G,
+                                 int H, int W, const int* pos, int N, float white_level, int* status, int h, int w,
+                                 float* loss_out, float* dparams, int dm_kind, float dm_clip_hi, const int* ops,
+                                 const int* param_off, const int* iarg, int S, const float* params, int param_stride, int P,
+                                 void* workspace, size_t workspace_bytes, risp_stream_t stream);
+int risp_pipeline_l1_step_store(const void* raw_store, int raw_bytes_per_code, int F, const unsigned char* gt_store, int G,
+                                int H, int W, const int* pos, int N, float white_level, int* status, int h, int w,
+                                float* loss_out, float* dparams, int dm_kind, float dm_clip_hi, const int* ops,
+                                const int* param_off, const int* iarg, int S, const float* params, int param_stride, int P,
+                                void* workspace, size_t workspace_bytes, risp_stream_t stream);
+
 /* Backward of risp_pipeline_fwd for an upstream gradient dy (N,3,H,W): recomputes the forward from
  * raw in registers (nothing was saved) and reduces d/dparams; 16 B/px.  No gradient w.r.t. raw: the
  * containers never need one (candidate-net weights are frozen, SURVEY.md §3.2).  Workspace as above. */

@@ -9,6 +9,7 @@ import concurrent.futures as cf
 import glob
 import hashlib
 import os
+import re
 import subprocess
 import sys
 
@@ -28,7 +29,10 @@ def _sources():
 
 def _digest(src):
     h = hashlib.sha1()
-    for f in [src] + sorted(glob.glob(os.path.join(CSRC, '*.cuh'))) + [os.path.join(ROOT, 'include', 'reconfigisp_b200.h')]:
+    # a source may compile another one a second time (risp_fused_store.cu): the included .cu is part of its inputs
+    with open(src) as fh:
+        included = [os.path.join(CSRC, f) for f in re.findall(r'^#include "(\w+\.cu)"', fh.read(), flags=re.M)]
+    for f in [src] + included + sorted(glob.glob(os.path.join(CSRC, '*.cuh'))) + [os.path.join(ROOT, 'include', 'reconfigisp_b200.h')]:
         with open(f, 'rb') as fh:
             h.update(fh.read())
     h.update(' '.join(FLAGS).encode())

@@ -112,6 +112,12 @@ __device__ __forceinline__ float decode_code(uint32_t c, float white_level) { re
 __device__ __forceinline__ bool whole_frame_record(int4 r, int F, int G) {
   return r.x >= 0 && r.x < F && r.y >= 0 && r.y < G && r.z == 0 && r.w == 0;
 }
+// the record of an h x w crop of H x W frames: (raw slot, GT slot, y0, x0) with both slots inside their stores, the crop
+// inside the frame and an even origin (the CFA phase) -- the rule risp_sample_crops applies to its records
+__device__ __forceinline__ bool crop_record(int4 r, int F, int G, int H, int W, int h, int w) {
+  return r.x >= 0 && r.x < F && r.y >= 0 && r.y < G && r.z >= 0 && r.w >= 0 && r.z <= H - h && r.w <= W - w &&
+         ((r.z | r.w) & 1) == 0;
+}
 __device__ __forceinline__ unsigned long long warp_sum_u64(unsigned long long v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -27,10 +27,18 @@ __constant__ float g_cpar[kCSlots][kCRows][kCRowFloats];
 
 // STEP: MSE loss; STEP_L1: L1 loss (isp_model.py:44-49); EVAL: inference arithmetic + squared 8-bit code differences to the GT
 // EVAL_S16 / EVAL_U8: EVAL reading a frame store (16-bit / 8-bit raw codes, 8-bit planar GT codes; frames named by records)
-enum { MODE_FWD = 0, MODE_STEP = 1, MODE_BWD = 2, MODE_STEP_L1 = 3, MODE_EVAL = 4, MODE_EVAL_S16 = 5, MODE_EVAL_U8 = 6 };
-__host__ __device__ constexpr bool is_store(int mode) { return mode == MODE_EVAL_S16 || mode == MODE_EVAL_U8; }
-__host__ __device__ constexpr bool is_eval(int mode) { return mode == MODE_EVAL || is_store(mode); }
-// A CTA is one warp (32 threads), so everything but the lane index is CTA-uniform (uniform datapath, no R2UR).  The warp
+// STEP_S16 / STEP_U8 / STEP_L1_S16 / STEP_L1_U8: STEP / STEP_L1 on h x w crops of a frame store (crops named by records)
+enum { MODE_FWD = 0, MODE_STEP = 1, MODE_BWD = 2, MODE_STEP_L1 = 3, MODE_EVAL = 4, MODE_EVAL_S16 = 5, MODE_EVAL_U8 = 6,
+       MODE_STEP_S16 = 7, MODE_STEP_U8 = 8, MODE_STEP_L1_S16 = 9, MODE_STEP_L1_U8 = 10 };
+// bytes per raw code of the store modes (0: fp32 batch)
+__host__ __device__ constexpr int code_bytes(int mode) {
+  return (mode == MODE_EVAL_S16 || mode == MODE_STEP_S16 || mode == MODE_STEP_L1_S16) ? 2
+       : (mode == MODE_EVAL_U8 || mode == MODE_STEP_U8 || mode == MODE_STEP_L1_U8) ? 1 : 0;
+}
+__host__ __device__ constexpr bool is_store(int mode) { return code_bytes(mode) != 0; }
+__host__ __device__ constexpr bool is_eval(int mode) { return mode == MODE_EVAL || mode == MODE_EVAL_S16 || mode == MODE_EVAL_U8; }
+__host__ __device__ constexpr bool is_l1(int mode) { return mode == MODE_STEP_L1 || mode == MODE_STEP_L1_S16 || mode == MODE_STEP_L1_U8; }
+__host__ __device__ constexpr bool is_store_step(int mode) { return is_store(mode) && !is_eval(mode); }// A CTA is one warp (32 threads), so everything but the lane index is CTA-uniform (uniform datapath, no R2UR).  The warp
 // owns a strip of kStrip columns.
 constexpr int kStrip = 128;
 
@@ -53,12 +61,14 @@ struct FusedArgs {
 };
 
 // store modes: image n of the launch is frame pos[n].x of the raw store against frame pos[n].y of the GT store (FusedArgs'
-// raw / gt hold the stores).  A kernel parameter of its own, after the others: the other modes' parameters keep their offsets
+// raw / gt hold the stores).  A kernel parameter of its own, after the others: the other modes' parameters keep their offsets.
+// Store step modes: image n is the crop of FusedArgs' H x W at (pos[n].z, pos[n].w) of those frames
 struct StoreArgs {
   const int4* pos;
-  int* status;          // set when a record is not a whole frame of the stores; that image adds nothing
+  int* status;          // set when a record is not a whole frame (eval) / a crop (step) of the stores; that image adds nothing
   float white_level;
   int F, G;             // frames in the raw / GT store
+  int FH, FW;           // frame size of the stores
 };
 
 // ---- preparation: derived constants of every parameter row ---------------------------------------------------------
@@ -172,25 +182,39 @@ __device__ __forceinline__ uint32_t lds_u8(uint32_t addr) {
   return v;
 }
 // raw window values out of a ring record: fp32 as copied, or store codes decoded in registers (decode_code)
+__device__ __forceinline__ float4 decode_u8x4(uint32_t v, float wl) {
+  return make_float4(decode_code(v & 0xffu, wl), decode_code((v >> 8) & 0xffu, wl), decode_code((v >> 16) & 0xffu, wl),
+                     decode_code(v >> 24, wl));
+}
 template <int MODE>
 __device__ __forceinline__ float4 ld_raw4(uint32_t addr, float wl) {
-  if constexpr (MODE == MODE_EVAL_S16) {
+  if constexpr (is_store_step(MODE) && code_bytes(MODE) == 2) {     // a crop's columns sit 4-byte aligned in the record
+    const uint32_t v0 = lds_u32(addr), v1 = lds_u32(addr + 4);
+    return make_float4(decode_code(v0 & 0xffffu, wl), decode_code(v0 >> 16, wl), decode_code(v1 & 0xffffu, wl),
+                       decode_code(v1 >> 16, wl));
+  } else if constexpr (is_store_step(MODE)) {                         // 2-byte aligned
+    return decode_u8x4(lds_u16(addr) | (lds_u16(addr + 2) << 16), wl);
+  } else if constexpr (code_bytes(MODE) == 2) {
     const uint2 v = lds_u64(addr);
     return make_float4(decode_code(v.x & 0xffffu, wl), decode_code(v.x >> 16, wl), decode_code(v.y & 0xffffu, wl),
                        decode_code(v.y >> 16, wl));
-  } else if constexpr (MODE == MODE_EVAL_U8) {
-    const uint32_t v = lds_u32(addr);
-    return make_float4(decode_code(v & 0xffu, wl), decode_code((v >> 8) & 0xffu, wl), decode_code((v >> 16) & 0xffu, wl),
-                       decode_code(v >> 24, wl));
+  } else if constexpr (code_bytes(MODE) == 1) {
+    return decode_u8x4(lds_u32(addr), wl);
   } else {
     return lds4(addr);
   }
 }
 template <int MODE>
 __device__ __forceinline__ float ld_raw1(uint32_t addr, float wl) {
-  if constexpr (MODE == MODE_EVAL_S16) return decode_code(lds_u16(addr), wl);
-  else if constexpr (MODE == MODE_EVAL_U8) return decode_code(lds_u8(addr), wl);
+  if constexpr (code_bytes(MODE) == 2) return decode_code(lds_u16(addr), wl);
+  else if constexpr (code_bytes(MODE) == 1) return decode_code(lds_u8(addr), wl);
   else return lds1(addr);
+}
+// the step's target: fp32 as copied, or 8-bit GT codes decoded as the sampler decodes them (code / 255, correctly rounded)
+template <int MODE>
+__device__ __forceinline__ float4 ld_gt4(uint32_t addr) {
+  if constexpr (is_store(MODE)) return decode_u8x4(lds_u16(addr) | (lds_u16(addr + 2) << 16), 255.f);   // 2-byte aligned
+  else return lds4(addr);
 }
 __device__ __forceinline__ void sts4(uint32_t addr, float4 v) {
   asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
@@ -210,15 +234,20 @@ struct RingCfg {
   // (measured: 1 KB boxes deliver 1.9 TB/s chip-wide), so the inference kernel, which has nothing but the copies to wait
   // for, uses 4-row boxes; the backward-carrying kernels are issue-bound and keep the smaller ring
   static constexpr int RR = (MODE == MODE_FWD) ? 4 : 2;
-  static constexpr int ES = (MODE == MODE_EVAL_S16) ? 2 : (MODE == MODE_EVAL_U8) ? 1 : 4;   // bytes per raw value
+  static constexpr int ES = is_store(MODE) ? code_bytes(MODE) : 4;                          // bytes per raw value
   static constexpr int GES = is_store(MODE) ? 1 : 4;                                         // bytes per GT value
   // columns of left pad: 16 bytes, so that a box starts on a 16-byte boundary of the row (kPad floats; 8 / 16 codes)
   static constexpr int PADL = 16 / ES;
   // one raw row of the box (left pad, strip, the right halo), widened to a 16-byte multiple (a tensor-map rule): 544 B of
   // fp32 (136 columns), 288 B of 16-bit codes (144), 160 B of 8-bit codes (160)
   static constexpr int RAWROWB = ((PADL + kStrip + 2) * ES + 15) / 16 * 16;
-  static constexpr int RAWB = (RR * RAWROWB + 127) / 128 * 128;          // RR rows, padded to a 128-B multiple
-  static constexpr int GTPLANEB = RR * kStrip * GES;
+  // Store step modes: a crop's origin is only even, while a box must start on a 16-byte boundary of its row.  A box starts
+  // at the crop's column rounded down to one, and the lanes read their columns that many codes further on: the raw rows
+  // above have that slack already; the GT box is 192 columns wide (128 + up to 14); a narrow record needs 96 B x 8 raw rows.
+  // Narrow GT boxes are 48 x 8 / 96 x 4, so that every GT plane of a record is RR x 192 bytes
+  static constexpr int GTW = is_store_step(MODE) ? 192 : kStrip;          // GT box columns of a full record
+  static constexpr int RAWB = is_store_step(MODE) ? 768 : (RR * RAWROWB + 127) / 128 * 128;   // RR rows, padded to 128 B
+  static constexpr int GTPLANEB = RR * GTW * GES;
   static constexpr int GTB = (MODE == MODE_FWD) ? 0 : 3 * GTPLANEB;  // [plane][row][128]
   static constexpr int RECB = RAWB + GTB;                                // multiple of 128
   static constexpr int WARPB = D * RECB;
@@ -331,10 +360,11 @@ struct Tail {
       yout = x;
       if constexpr (MODE == MODE_BWD) return tgt;
       // d loss / d y up to the constant 2/numel (applied by the finaliser).  lane_w = 1 for lanes inside the frame (1*x - t is
-      // exactly x - t) and 0 for the lanes of the last strip that hang over the right edge (their t is 0): no divergent branch
+      // exactly x - t) and 0 for the lanes of the last strip that hang over the right edge (their t is 0: zero fill of the
+      // fp32 batch, zeroed by do_row for crops of a store): no divergent branch
       const float2 dd = SC ? make_float2(fmaf(lane_w, x.x, -tgt.x), fmaf(lane_w, x.y, -tgt.y))
                            : __ffma2_rn(make_float2(lane_w, lane_w), x, make_float2(-tgt.x, -tgt.y));
-      if constexpr (MODE == MODE_STEP_L1) {      // nn.L1Loss: sum |y - t| ; gradient sign(y - t) (0 at equality), 1/numel later
+      if constexpr (is_l1(MODE)) {               // nn.L1Loss: sum |y - t| ; gradient sign(y - t) (0 at equality), 1/numel later
         acc_add<SC>(loss, make_float2(fabsf(dd.x), fabsf(dd.y)));
         return make_float2((dd.x > 0.f ? 1.f : 0.f) - (dd.x < 0.f ? 1.f : 0.f), (dd.y > 0.f ? 1.f : 0.f) - (dd.y < 0.f ? 1.f : 0.f));
       }
@@ -495,14 +525,28 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
   const int n = blockIdx.y, j0 = blockIdx.x;       // frame, CTA within the frame (both uniform)
   const int H = a.H, W = a.W;
   int zraw = 0, zgt = 0;                           // store modes: tensor-map frame / first GT plane of image n
-  if constexpr (is_store(MODE)) {
+  int xo = 0, yo = 0;                              // store step modes: the crop's origin in the frame
+  if constexpr (is_eval(MODE) && is_store(MODE)) {
     const int4 rec = sa.pos[n];
     if (!whole_frame_record(rec, sa.F, sa.G)) {
       if (lane == 0) { *sa.status = 1; a.sse[(long long)n * a.cpf + j0] = 0ull; }
       return;
     }
     zraw = rec.x; zgt = 3 * rec.y;
+  } else if constexpr (is_store(MODE)) {
+    const int4 rec = sa.pos[n];
+    if (!crop_record(rec, sa.F, sa.G, sa.FH, sa.FW, H, W)) {      // a zero partial row: the image adds nothing
+      if (lane == 0) *sa.status = 1;
+      float* __restrict__ out = a.partial + ((long long)n * a.cpf + j0) * RISP_NSLOT;
+      for (int i = lane; i < RISP_NSLOT; i += 32) out[i] = 0.f;
+      return;
+    }
+    zraw = rec.x; zgt = 3 * rec.y; yo = rec.z; xo = rec.w;
   }
+  // store step modes: the boxes start at the crop's column rounded down to 16 bytes (PADL raw codes, 16 GT codes); the lanes'
+  // columns sit dxb / dgb bytes further into the records (0 in every other mode)
+  const int xra = xo & ~(RingCfg<MODE>::PADL - 1), xga = xo & ~15;
+  const uint32_t dxb = (uint32_t)(xo - xra) * RingCfg<MODE>::ES, dgb = (uint32_t)(xo - xga) * RingCfg<MODE>::GES;
   const long long plane = (long long)H * W;
   float* __restrict__ yb = a.y ? a.y + (long long)n * 3 * plane : nullptr;
   // derived constants of this frame's parameter row (written by fused_prep_kernel earlier on the stream): they enter the
@@ -550,8 +594,8 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
   };
   // ---- backward-carrying kernels (issue-bound): a private window per row read with plain LDS ----
   // one row: read the window (wa(j): shared-memory address of its raw row j) and the GT row, demosaic, chain, store.
-  // Narrow items: the lane's row may belong to another item while its GT is real data: such a lane's target is zeroed so
-  // that it adds exactly nothing.
+  // Narrow items, and every item of a crop of a store: the lane's row / columns may lie outside the item while its GT is
+  // real data: such a lane's target is zeroed so that it adds exactly nothing.
   auto do_row = [&](auto odd_tag, auto slow_tag, auto narrow_tag, int r, auto wa, uint32_t gta, const LanePos& L) {
     constexpr bool ODD = decltype(odd_tag)::value;
     constexpr bool slow = decltype(slow_tag)::value;     // shadows the run-time flag: the chain's branches on it fold away
@@ -604,8 +648,9 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
       float4 tg[3];
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
-        tg[c] = lds4(gta + c * RC::GTPLANEB + L.gt);
-        if constexpr (narrow_item) {
+        tg[c] = ld_gt4<MODE>(gta + c * RC::GTPLANEB + L.gt);
+        // a crop's right neighbours are frame pixels with a real GT: masked lanes of full items are zeroed as well
+        if constexpr (narrow_item || is_store(MODE)) {
           if (!L.active) tg[c] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
       }
@@ -642,8 +687,8 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
       const uint32_t rec = ring + (g & (D - 1)) * RC::RECB, bar = bars + (g & (D - 1)) * 8;
       const bool has_gt = (MODE != MODE_FWD) && (k >= 1) && (k < nrec - 1);
       mbar_expect_tx(bar, (uint32_t)(RR * RC::RAWROWB) + (has_gt ? (uint32_t)RC::GTB : 0u));
-      tma_load_3d(rec, &tm_raw, c0s - RC::PADL, rbase + RR * k, is_store(MODE) ? zraw : n, bar);
-      if (has_gt) tma_load_3d(rec + RC::RAWB, &tm_gt, c0s, rbase + RR * k, is_store(MODE) ? zgt : 3 * n, bar);
+      tma_load_3d(rec, &tm_raw, c0s - RC::PADL + xra, rbase + RR * k + yo, is_store(MODE) ? zraw : n, bar);
+      if (has_gt) tma_load_3d(rec + RC::RAWB, &tm_gt, c0s + xga, rbase + RR * k + yo, is_store(MODE) ? zgt : 3 * n, bar);
     };
     auto wait_rec = [&](int k) {
       const unsigned g = gcount + (unsigned)k;
@@ -665,7 +710,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
 
     // lane offsets inside a raw row (bytes): own 4 columns; the strip's first / last lane reads its outer halo from the
     // record (frame border folded into the offset), every other lane gets it from its neighbour by shuffle
-    const uint32_t own = (uint32_t)(RC::PADL + lane * 4) * ES;
+    const uint32_t own = (uint32_t)(RC::PADL + lane * 4) * ES + dxb;
     const bool endL = (lane == 0), endR = (lane == 31) || last;
     // byte offsets of columns; ES == 4 spelled out (the fp32 kernels' instruction stream stays as it was)
     const uint32_t oL0 = own + (ES == 4 ? (first ? (HL == 1 ? 4 : 8) : -4 * HL) : ES * (first ? (HL == 1 ? 1 : 2) : -HL));  // column c0-HL (reflect: -1 -> 1, -2 -> 2)
@@ -675,7 +720,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
 
     if constexpr (MODE != MODE_FWD) {
       // ---- backward-carrying kernels: 2-row records ----
-      const LanePos L{own, oL0, oL1, oR0, oR1, (uint32_t)lane * (4u * GES), c0, 0, active, lane_w};
+      const LanePos L{own, oL0, oL1, oR0, oR1, (uint32_t)lane * (4u * GES) + dgb, c0, 0, active, lane_w};
 
       // iteration m computes rows r = ra + 2(m-1) (even) and r+1 (odd) from records m-1, m, m+1.
       // The loop exists twice, with the tone curve's slow flag (a knot outside [0,1]: final clamp active) as a compile-time
@@ -702,7 +747,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
           for (int j = 0; j < WR; ++j) { we[j] = row_addr(r - HL + j); wo[j] = row_addr(r + 1 - HL + j); }
         }
         do_row(std::false_type{}, slow_tag, std::false_type{}, r, [&](int j) { return we[j]; }, recB + RC::RAWB, L);
-        do_row(std::true_type{}, slow_tag, std::false_type{}, r + 1, [&](int j) { return wo[j]; }, recB + RC::RAWB + kStrip * GES, L);
+        do_row(std::true_type{}, slow_tag, std::false_type{}, r + 1, [&](int j) { return wo[j]; }, recB + RC::RAWB + RC::GTW * GES, L);
         __syncwarp();                              // every lane has read record m-1: its slot may be refilled
         if (m - 1 + D < nrec) {
           if (elect_one()) issue(m - 1 + D);
@@ -797,10 +842,12 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
     const int grp = lane >> (6 - sh), li = lane & ((1 << (6 - sh)) - 1);
     const int c0s = a.strip_blocks * kStrip, c0 = c0s + 4 * li;
     // bytes per box row: fp32 rows are 16-byte multiples already, code rows widen to one (a tensor-map rule)
-    const uint32_t rowb = ES == 4 ? (uint32_t)(nw + kPad) * 4u : ((uint32_t)(nw + RC::PADL) * ES + 15u) & ~15u;
+    const uint32_t rowb = ES == 4 ? (uint32_t)(nw + kPad) * 4u
+                                  : ((uint32_t)(nw + RC::PADL + (is_store_step(MODE) ? RC::PADL - 2 : 0)) * ES + 15u) & ~15u;
+    const int nwg = is_store_step(MODE) ? (RC::GTPLANEB / GES) >> sh : nw;    // GT columns of a narrow box
     const bool incol = c0 < W, first = (c0 == 0), last = incol && (c0 + 4 >= W);
     LanePos L;
-    L.own = (uint32_t)(RC::PADL + 4 * li) * ES;
+    L.own = (uint32_t)(RC::PADL + 4 * li) * ES + dxb;
     L.oL0 = L.own + (ES == 4 ? (first ? (HL == 1 ? 4 : 8) : -4 * HL) : ES * (first ? (HL == 1 ? 1 : 2) : -HL));
     L.oL1 = L.own + (ES == 4 ? (first ? 4 : -4) : ES * (first ? 1 : -1));
     // a lane with c0 + 4 < W is never the last of its group (W <= c0s + nw).  Lanes past the frame read inside their row
@@ -810,7 +857,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
     L.oR1 = L.own + (ES == 4 ? (fold ? 4 : 20) : ES * (fold ? 1 : 5));
     L.c0 = c0;
     L.dr = 2 * grp;
-    const uint32_t gt_even = (uint32_t)(2 * grp * nw + 4 * li) * GES;
+    const uint32_t gt_even = (uint32_t)(2 * grp * nwg + 4 * li) * GES + dgb;
     for (int t = a.cpf - 1 - j0; t < a.nchunks; t += a.cpf) {
       const int ra = t * a.nrows_per_chunk;
       const int rb = min(H, ra + a.nrows_per_chunk);
@@ -821,8 +868,8 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
         const uint32_t rec = ring + (g & (D - 1)) * RC::RECB, bar = bars + (g & (D - 1)) * 8;
         const bool has_gt = (k >= 1) && (k < nrec - 1);
         mbar_expect_tx(bar, (uint32_t)RRn * rowb + (has_gt ? (uint32_t)RC::GTB : 0u));
-        tma_load_3d(rec, &tm_rawn, c0s - RC::PADL, rbase + RRn * k, is_store(MODE) ? zraw : n, bar);
-        if (has_gt) tma_load_3d(rec + RC::RAWB, &tm_gtn, c0s, rbase + RRn * k, is_store(MODE) ? zgt : 3 * n, bar);
+        tma_load_3d(rec, &tm_rawn, c0s - RC::PADL + xra, rbase + RRn * k + yo, is_store(MODE) ? zraw : n, bar);
+        if (has_gt) tma_load_3d(rec + RC::RAWB, &tm_gtn, c0s + xga, rbase + RRn * k + yo, is_store(MODE) ? zgt : 3 * n, bar);
       };
       auto wait_rec = [&](int k) {
         const unsigned g = gcount + (unsigned)k;
@@ -851,7 +898,7 @@ fused_kernel(FusedArgs a, ChainDesc d, const __grid_constant__ CUtensorMap tm_ra
           const uint32_t gta = ring + ((gcount + (unsigned)m) & (D - 1)) * RC::RECB + RC::RAWB;
           // window rows are computed where they are read: per-lane addresses live across the chain would cost registers
           do_row(std::false_type{}, slow_tag, std::true_type{}, R, [&](int j) { return row_addr(R + L.dr - HL + j); }, gta, L);
-          L.gt = gt_even + (uint32_t)nw * GES;
+          L.gt = gt_even + (uint32_t)nwg * GES;
           do_row(std::true_type{}, slow_tag, std::true_type{}, R + 1, [&](int j) { return row_addr(R + L.dr + 1 - HL + j); }, gta, L);
           __syncwarp();                              // every lane has read record m-1: its slot may be refilled
           if (m - 1 + D < nrec) {
@@ -1075,26 +1122,40 @@ static int make_map(CUtensorMap* tm, const void* base, int W, int H, long long Z
   return RISP_OK;
 }
 
+}  // namespace fused
+// resident CTAs per SM of the fp32 step kernel of (dm, l1, sig, narrow): the layout of the store step modes
+int fused_step_resident(int dm, bool l1, unsigned sig, bool narrow);
+namespace fused {
+
 template <int DM, int MODE, unsigned SIG>
 static int launch_one(FusedArgs a, const ChainDesc& d, int N, cudaStream_t st, int* rows_per_frame, const StoreArgs& sa) {
   // RISP_FUSED_STEP_ROWS: cap of the rows per item of the backward-carrying and evaluation kernels (many short items)
   static const int cap = [] { const char* e = MODE == MODE_FWD ? nullptr : getenv("RISP_FUSED_STEP_ROWS"); return e ? atoi(e) : 0; }();
   // narrow items where the kernel that runs them keeps the occupancy of the one that does not
   bool narrow = false;
-  if constexpr (MODE != MODE_FWD) narrow = resident_ctas<DM, MODE, SIG, true>() == resident_ctas<DM, MODE, SIG, false>();
-  const Geometry g = geometry(N, a.H, a.W, resident_ctas<DM, MODE, SIG, false>(), RingCfg<MODE>::RR,
-                              cap >= RingCfg<MODE>::RR ? cap : kMaxRows, narrow);
+  int ctas;
+  if constexpr (is_store(MODE) && !is_eval(MODE)) {
+    // the items, and with them the order of every sum, of the fp32 step on the decoded batch: the same loss and gradients
+    narrow = fused_step_resident(DM, is_l1(MODE), SIG, true) == fused_step_resident(DM, is_l1(MODE), SIG, false);
+    ctas = fused_step_resident(DM, is_l1(MODE), SIG, false);
+  } else {
+    if constexpr (MODE != MODE_FWD) narrow = resident_ctas<DM, MODE, SIG, true>() == resident_ctas<DM, MODE, SIG, false>();
+    ctas = resident_ctas<DM, MODE, SIG, false>();
+  }
+  const Geometry g = geometry(N, a.H, a.W, ctas, RingCfg<MODE>::RR, cap >= RingCfg<MODE>::RR ? cap : kMaxRows, narrow);
   if (rows_per_frame) *rows_per_frame = g.cpf;
   a.rows_per_chunk = g.rows_per_chunk; a.chunks = g.chunks; a.strip_blocks = g.strip_blocks; a.cpf = g.cpf;
   a.nw = g.nw; a.nrows_per_chunk = g.nrows_per_chunk; a.nchunks = g.nchunks;
   CUtensorMap tm_raw, tm_gt, tm_rawn, tm_gtn;
   using RC = RingCfg<MODE>;
-  // store modes: the maps span the whole stores (F raw frames, 3G GT planes); the kernel picks frames by record
+  // store modes: the maps span the whole stores (F raw frames, 3G GT planes of FH x FW); the kernel picks frames (and the
+  // step modes the crop's origin) by record.  Everything else -- item grid, reflection, masks -- is the h x w of a.H, a.W
   const long long zr = is_store(MODE) ? sa.F : N, zg = 3ll * (is_store(MODE) ? sa.G : N);
-  int rc = make_map(&tm_raw, a.raw, a.W, a.H, zr, RC::RAWROWB / RC::ES, RC::RR, 1, RC::ES);
+  const int mh = is_store(MODE) ? sa.FH : a.H, mw = is_store(MODE) ? sa.FW : a.W;
+  int rc = make_map(&tm_raw, a.raw, mw, mh, zr, RC::RAWROWB / RC::ES, RC::RR, 1, RC::ES);
   if (rc != RISP_OK) return rc;
   if (MODE != MODE_FWD) {
-    rc = make_map(&tm_gt, a.gt, a.W, a.H, zg, kStrip, RC::RR, 3, RC::GES);
+    rc = make_map(&tm_gt, a.gt, mw, mh, zg, RC::GTW, RC::RR, 3, RC::GES);
     if (rc != RISP_OK) return rc;
   } else {
     tm_gt = tm_raw;
@@ -1109,10 +1170,15 @@ static int launch_one(FusedArgs a, const ChainDesc& d, int N, cudaStream_t st, i
                   RingCfg<MODE_EVAL_U8>::RAWB >= 48 * 8 && RingCfg<MODE_EVAL_U8>::RAWB >= 80 * 4 &&
                   RingCfg<MODE_EVAL_U8>::GTB == 3 * 32 * 8 && RingCfg<MODE_EVAL_U8>::GTB == 3 * 64 * 4,
                   "a narrow record of codes must fit the ring's record");
-    const int ncols = (((g.nw + RC::PADL) * RC::ES + 15) / 16 * 16) / RC::ES;
-    rc = make_map(&tm_rawn, a.raw, a.W, a.H, zr, ncols, rrn, 1, RC::ES);
+    static_assert(RingCfg<MODE_STEP_S16>::RAWB >= 96 * 8 && RingCfg<MODE_STEP_S16>::RAWB >= 160 * 4 &&
+                  RingCfg<MODE_STEP_U8>::RAWB >= 64 * 8 && RingCfg<MODE_STEP_U8>::RAWB >= 96 * 4 &&
+                  RingCfg<MODE_STEP_U8>::GTPLANEB == 48 * 8 && RingCfg<MODE_STEP_U8>::GTPLANEB == 96 * 4,
+                  "a narrow record of a crop must fit the ring's record");
+    const int slack = is_store_step(MODE) ? RC::PADL - 2 : 0;      // store step modes: room for the crop's offset
+    const int ncols = (((g.nw + RC::PADL + slack) * RC::ES + 15) / 16 * 16) / RC::ES;
+    rc = make_map(&tm_rawn, a.raw, mw, mh, zr, ncols, rrn, 1, RC::ES);
     if (rc != RISP_OK) return rc;
-    rc = make_map(&tm_gtn, a.gt, a.W, a.H, zg, g.nw, rrn, 3, RC::GES);
+    rc = make_map(&tm_gtn, a.gt, mw, mh, zg, is_store_step(MODE) ? RC::GTPLANEB / RC::GES / rrn : g.nw, rrn, 3, RC::GES);
     if (rc != RISP_OK) return rc;
   } else {
     tm_rawn = tm_raw; tm_gtn = tm_gt;
@@ -1157,12 +1223,32 @@ static int prep_constants(const float* params, int pstride, int N, const ChainDe
 }  // namespace fused
 
 // true if the packed kernels take this chain (a pre-instantiated signature, parameter rows fit a constant slot)
+bool fused_handles(const ChainDesc& d, int N, int param_stride, int H, int W);
+
+// The entry points are split over four objects, so that their kernel instantiations compile in parallel (one object holding
+// them all takes several times as long as the four together): RISP_FUSED_PART unset -- forward, fp32 step and backward;
+// 1 -- evaluation (risp_fused_eval.cu); 2 / 3 -- the step on crops of a store of 16- / 8-bit raw codes
+// (risp_fused_store.cu / risp_fused_store_u8.cu).  Each object keeps its own constant parameter block.
+#if !defined(RISP_FUSED_PART)
 bool fused_handles(const ChainDesc& d, int N, int param_stride, int H, int W) {
   if ((long long)H * W * 3 >= (1ll << 31)) return false;     // 32-bit element offsets inside a frame
   const unsigned sig = chain_signature(d);
   if (sig != RISP_SIG_A && sig != RISP_SIG_B && sig != RISP_SIG_C && sig != RISP_SIG_D && sig != RISP_SIG_SKIP) return false;
   if (param_stride != 0 && N > fused::kCRows) return false;
   return fused::eff_from_ops(d.op, d.iarg, d.S).ok;
+}
+
+int fused_step_resident(int dm, bool l1, unsigned sig, bool narrow) {
+  using namespace fused;
+#define RISP_F_RES(DMK, SG)                                                                                                   \
+  if (dm == (DMK) && sig == (SG))                                                                                             \
+    return l1 ? (narrow ? resident_ctas<DMK, MODE_STEP_L1, (SG), true>() : resident_ctas<DMK, MODE_STEP_L1, (SG), false>())    \
+              : (narrow ? resident_ctas<DMK, MODE_STEP, (SG), true>() : resident_ctas<DMK, MODE_STEP, (SG), false>());
+#define RISP_F_RES_DM(DMK) RISP_F_RES(DMK, RISP_SIG_A) RISP_F_RES(DMK, RISP_SIG_B) RISP_F_RES(DMK, RISP_SIG_C) RISP_F_RES(DMK, RISP_SIG_D)
+  RISP_F_RES_DM(RISP_DM_NEAREST) RISP_F_RES_DM(RISP_DM_BILINEAR) RISP_F_RES_DM(RISP_DM_MALVAR)
+#undef RISP_F_RES_DM
+#undef RISP_F_RES
+  return 1;
 }
 
 // partial rows the step / backward kernels write: [N][rows_per_frame][RISP_NSLOT]
@@ -1172,6 +1258,25 @@ int fused_partial_rows_per_frame(int N) {
   return slots / N < 1 ? 1 : slots / N;
 }
 
+// mode: 0 forward, 1 MSE step, 2 backward with upstream dy, 3 L1 step.  Returns RISP_OK, an error, or 1 when the chain is not handled.
+// *rows_per_frame (nullable) receives the number of partial rows per frame actually written (modes 1-3).
+int fused_launch(int mode, const float* raw, const float* gt, float* y, float* partial, const float* params, int pstride,
+                 int N, int H, int W, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st, int* rows_per_frame) {
+  using namespace fused;
+  if (!fused_handles(d, N, pstride, H, W)) return 1;
+  int slot;
+  const int rc = prep_constants(params, pstride, N, d, st, &slot);
+  if (rc != RISP_OK) return rc;
+  const FusedArgs a{raw, gt, y, partial, params, pstride, H, W, 0, 0, 0, 0, clip_hi, slot};
+  switch (mode) {
+    case 0: return dispatch<MODE_FWD>(a, d, N, dm_kind, st, rows_per_frame);
+    case 1: return dispatch<MODE_STEP>(a, d, N, dm_kind, st, rows_per_frame);
+    case 3: return dispatch<MODE_STEP_L1>(a, d, N, dm_kind, st, rows_per_frame);
+    default: return dispatch<MODE_BWD>(a, d, N, dm_kind, st, rows_per_frame);
+  }
+}
+
+#elif RISP_FUSED_PART == 1
 // evaluation mode: inference arithmetic, squared 8-bit code differences to gt -> partial[N][*rows_per_frame], optional 8-bit
 // HWC image.  Returns RISP_OK, an error, or 1 when the chain is not handled.
 int fused_eval_launch(const float* raw, const float* gt, unsigned char* u8, unsigned long long* partial, const float* params,
@@ -1203,27 +1308,60 @@ int fused_eval_store_launch(const void* raw_store, int raw_bpc, int F, const uns
   if (rc != RISP_OK) return rc;
   const FusedArgs a{static_cast<const float*>(raw_store), reinterpret_cast<const float*>(gt_store), nullptr, nullptr, params,
                     pstride, H, W, 0, 0, 0, 0, clip_hi, slot, u8, partial};
-  const StoreArgs sa{reinterpret_cast<const int4*>(pos), status, white_level, F, G};
+  const StoreArgs sa{reinterpret_cast<const int4*>(pos), status, white_level, F, G, H, W};
   return raw_bpc == 2 ? dispatch<MODE_EVAL_S16>(a, d, N, dm_kind, st, rows_per_frame, sa)
                       : dispatch<MODE_EVAL_U8>(a, d, N, dm_kind, st, rows_per_frame, sa);
 }
 
-// mode: 0 forward, 1 MSE step, 2 backward with upstream dy, 3 L1 step.  Returns RISP_OK, an error, or 1 when the chain is not handled.
-// *rows_per_frame (nullable) receives the number of partial rows per frame actually written (modes 1-3).
-int fused_launch(int mode, const float* raw, const float* gt, float* y, float* partial, const float* params, int pstride,
-                 int N, int H, int W, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st, int* rows_per_frame) {
-  using namespace fused;
-  if (!fused_handles(d, N, pstride, H, W)) return 1;
+#else
+namespace fused {
+// MSE / L1 step on h x w crops of frame stores: image n is the crop at (pos[n].z, pos[n].w) of raw frame pos[n].x against GT
+// frame pos[n].y (code / 255), of H x W frames; MSE / L1 are the store step modes of one raw code width
+template <int MSE, int L1>
+static int step_store_launch(bool l1, const void* raw_store, int F, const unsigned char* gt_store, int G, int H, int W,
+                             const int* pos, int* status, float white_level, float* partial, const float* params, int pstride,
+                             int N, int h, int w, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st,
+                             int* rows_per_frame) {
+  if (!fused_handles(d, N, pstride, h, w)) return 1;
   int slot;
   const int rc = prep_constants(params, pstride, N, d, st, &slot);
   if (rc != RISP_OK) return rc;
-  const FusedArgs a{raw, gt, y, partial, params, pstride, H, W, 0, 0, 0, 0, clip_hi, slot};
-  switch (mode) {
-    case 0: return dispatch<MODE_FWD>(a, d, N, dm_kind, st, rows_per_frame);
-    case 1: return dispatch<MODE_STEP>(a, d, N, dm_kind, st, rows_per_frame);
-    case 3: return dispatch<MODE_STEP_L1>(a, d, N, dm_kind, st, rows_per_frame);
-    default: return dispatch<MODE_BWD>(a, d, N, dm_kind, st, rows_per_frame);
-  }
+  const FusedArgs a{static_cast<const float*>(raw_store), reinterpret_cast<const float*>(gt_store), nullptr, partial, params,
+                    pstride, h, w, 0, 0, 0, 0, clip_hi, slot};
+  const StoreArgs sa{reinterpret_cast<const int4*>(pos), status, white_level, F, G, H, W};
+  return l1 ? dispatch<L1>(a, d, N, dm_kind, st, rows_per_frame, sa) : dispatch<MSE>(a, d, N, dm_kind, st, rows_per_frame, sa);
 }
+}  // namespace fused
+
+int fused_step_store_u8_launch(bool l1, const void* raw_store, int F, const unsigned char* gt_store, int G, int H, int W,
+                               const int* pos, int* status, float white_level, float* partial, const float* params,
+                               int pstride, int N, int h, int w, int dm_kind, float clip_hi, const ChainDesc& d,
+                               cudaStream_t st, int* rows_per_frame);
+#if RISP_FUSED_PART == 2
+// MSE / L1 step on h x w crops of frame stores (codes of raw_bpc bytes, decoded as code / white_level).  The caller has
+// checked the geometry (W % 16 == 0, 16-byte aligned stores: the tensor maps' rules).  Returns RISP_OK, an error, or 1 when
+// the chain is not handled.
+int fused_step_store_launch(bool l1, const void* raw_store, int raw_bpc, int F, const unsigned char* gt_store, int G, int H,
+                            int W, const int* pos, int* status, float white_level, float* partial, const float* params,
+                            int pstride, int N, int h, int w, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st,
+                            int* rows_per_frame) {
+  if (raw_bpc == 1)
+    return fused_step_store_u8_launch(l1, raw_store, F, gt_store, G, H, W, pos, status, white_level, partial, params, pstride,
+                                      N, h, w, dm_kind, clip_hi, d, st, rows_per_frame);
+  return fused::step_store_launch<fused::MODE_STEP_S16, fused::MODE_STEP_L1_S16>(
+      l1, raw_store, F, gt_store, G, H, W, pos, status, white_level, partial, params, pstride, N, h, w, dm_kind, clip_hi, d,
+      st, rows_per_frame);
+}
+#else
+int fused_step_store_u8_launch(bool l1, const void* raw_store, int F, const unsigned char* gt_store, int G, int H, int W,
+                               const int* pos, int* status, float white_level, float* partial, const float* params,
+                               int pstride, int N, int h, int w, int dm_kind, float clip_hi, const ChainDesc& d,
+                               cudaStream_t st, int* rows_per_frame) {
+  return fused::step_store_launch<fused::MODE_STEP_U8, fused::MODE_STEP_L1_U8>(
+      l1, raw_store, F, gt_store, G, H, W, pos, status, white_level, partial, params, pstride, N, h, w, dm_kind, clip_hi, d,
+      st, rows_per_frame);
+}
+#endif
+#endif
 
 }  // namespace risp

@@ -68,6 +68,29 @@ __device__ __forceinline__ void row_issue_codes(CodeRow<HL>& q, const unsigned c
   if (active && lane == 0 && c0 > 0) q.l = ld(c0 - HL);
   if (active && lane == 31 && c0 + 4 < W) q.r = ld(c0 + 4);
 }
+// the same row of a crop: img is the crop's first code in frames of `stride` codes per row (W: the crop's width).  The crop's
+// origin is only even, so the 4 codes are loaded as two halves (4 / 2-byte aligned) instead of one 8 / 4-byte vector; the
+// halo codes at c0-HL and c0+4 stay 2-byte aligned
+template <int HL, int ES>
+__device__ __forceinline__ void row_issue_crop_codes(CodeRow<HL>& q, const unsigned char* __restrict__ img, int row, int stride,
+                                                     int W, int c0, bool active, int lane) {
+  const unsigned char* rp = img + (long long)row * stride * ES;
+  q.v = make_uint2(0u, 0u); q.l = 0u; q.r = 0u;
+  if (active) {
+    if constexpr (ES == 2)
+      q.v = make_uint2(__ldg(reinterpret_cast<const uint32_t*>(rp + 2 * c0)), __ldg(reinterpret_cast<const uint32_t*>(rp + 2 * c0 + 4)));
+    else
+      q.v.x = (uint32_t)__ldg(reinterpret_cast<const unsigned short*>(rp + c0)) |
+              ((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(rp + c0 + 2)) << 16);
+  }
+  auto ld = [&](int c) -> uint32_t {
+    if constexpr (ES == 2) return HL == 1 ? (uint32_t)__ldg(reinterpret_cast<const unsigned short*>(rp + 2 * c))
+                                          : __ldg(reinterpret_cast<const uint32_t*>(rp + 2 * c));
+    else return HL == 1 ? (uint32_t)__ldg(rp + c) : (uint32_t)__ldg(reinterpret_cast<const unsigned short*>(rp + c));
+  };
+  if (active && lane == 0 && c0 > 0) q.l = ld(c0 - HL);
+  if (active && lane == 31 && c0 + 4 < W) q.r = ld(c0 + 4);
+}
 template <int HL, int ES>
 __device__ __forceinline__ RawRow<HL> row_decode(const CodeRow<HL>& q, float wl) {
   constexpr int B = 8 * ES;                 // bits per code
@@ -159,9 +182,24 @@ __device__ __forceinline__ void demosaic4(const float (&w)[2 * HL + 1][4 + 2 * H
 
 // EVAL: the forward of MODE_FWD, then the squared 8-bit code differences to the GT (per-image PSNR numerator); writes no y
 // EVAL_S16 / EVAL_U8: EVAL reading a frame store (16-bit / 8-bit raw codes, 8-bit planar GT codes; frames named by records)
-enum { MODE_FWD = 0, MODE_STEP = 1, MODE_EVAL = 2, MODE_EVAL_S16 = 3, MODE_EVAL_U8 = 4 };
-constexpr bool is_store(int mode) { return mode == MODE_EVAL_S16 || mode == MODE_EVAL_U8; }
-constexpr bool is_eval(int mode) { return mode == MODE_EVAL || is_store(mode); }
+// STEP_S16 / STEP_U8: STEP (MSE target, not dy) on h x w crops of a frame store (crops named by records)
+enum { MODE_FWD = 0, MODE_STEP = 1, MODE_EVAL = 2, MODE_EVAL_S16 = 3, MODE_EVAL_U8 = 4, MODE_STEP_S16 = 5, MODE_STEP_U8 = 6 };
+constexpr bool is_store(int mode) { return mode == MODE_EVAL_S16 || mode == MODE_EVAL_U8 || mode == MODE_STEP_S16 || mode == MODE_STEP_U8; }
+constexpr bool is_eval(int mode) { return mode == MODE_EVAL || mode == MODE_EVAL_S16 || mode == MODE_EVAL_U8; }
+constexpr bool is_step(int mode) { return mode == MODE_STEP || mode == MODE_STEP_S16 || mode == MODE_STEP_U8; }
+
+// 4 GT codes of a crop row (2-byte aligned: the crop's origin is even) decoded as the sampler decodes them, code / 255
+__device__ __forceinline__ float4 gt_codes4(const unsigned char* __restrict__ p) {
+  const uint32_t v = (uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p)) |
+                     ((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p + 2)) << 16);
+  return make_float4(decode_code(v & 0xffu, 255.f), decode_code((v >> 8) & 0xffu, 255.f), decode_code((v >> 16) & 0xffu, 255.f),
+                     decode_code(v >> 24, 255.f));
+}
+// the 3 planes of a crop's GT row (o: offset of the lane's first pixel in the first plane, fplane: codes per frame plane)
+__device__ __forceinline__ void crop_gt_row(const unsigned char* __restrict__ sgt, long long fplane, long long o, float4& b,
+                                            float4& g, float4& r) {
+  b = gt_codes4(sgt + o); g = gt_codes4(sgt + fplane + o); r = gt_codes4(sgt + 2 * fplane + o);
+}
 
 // packed-fp32 / constant-bank kernels for the pre-instantiated signatures (risp_fused.cu)
 bool fused_handles(const ChainDesc& d, int N, int param_stride, int H, int W);
@@ -174,6 +212,10 @@ int fused_eval_launch(const float* raw, const float* gt, unsigned char* u8, unsi
 int fused_eval_store_launch(const void* raw_store, int raw_bpc, int F, const unsigned char* gt_store, int G, const int* pos,
                             int* status, float white_level, unsigned char* u8, unsigned long long* partial, const float* params,
                             int pstride, int N, int H, int W, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st,
+                            int* rows_per_frame);
+int fused_step_store_launch(bool l1, const void* raw_store, int raw_bpc, int F, const unsigned char* gt_store, int G, int H,
+                            int W, const int* pos, int* status, float white_level, float* partial, const float* params,
+                            int pstride, int N, int h, int w, int dm_kind, float clip_hi, const ChainDesc& d, cudaStream_t st,
                             int* rows_per_frame);
 
 struct PipeArgs {
@@ -192,7 +234,7 @@ struct PipeArgs {
   const unsigned char* store;
   const unsigned char* gstore;
   const int4* pos;
-  int* status;        // set when a record is not a whole frame of the stores; that image adds nothing
+  int* status;        // set when a record is not a whole frame (eval) / a crop (step) of the stores; that image adds nothing
   float white_level;
   int F, G;
 };
@@ -206,9 +248,9 @@ constexpr int kPairUnroll = 2;
 // took 0.242 ms against 0.234 ms for one -- the kernel is not latency-bound.
 
 template <int DM, int MODE, unsigned SIG, bool BIGG>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, (MODE == MODE_STEP) ? ((SIG == 0) ? 1 : kStepMinBlocks)
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, is_step(MODE) ? ((SIG == 0) ? 1 : kStepMinBlocks)
                                                     : is_eval(MODE) ? kEvalMinBlocks : kFwdMinBlocks)
-pipeline_kernel(PipeArgs a, ChainDesc d) {
+pipeline_kernel(PipeArgs a, ChainDesc d, const int2 frame) {   // frame: store step modes, (H, W) of the stores' frames
   using SG = Sig<SIG>;
   constexpr int SMAX = SG::S;
   constexpr bool BIG = SG::generic ? BIGG : SG::big_c();
@@ -224,11 +266,19 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
   const int rb = min(H, ra + a.rows_per_chunk);
   const long long plane = (long long)H * W;
   constexpr bool ST = is_store(MODE);
-  constexpr int ES = (MODE == MODE_EVAL_S16) ? 2 : 1;      // store modes: bytes per raw code
-  bool ok = true;                                          // store modes: the record names a whole frame of the stores
+  constexpr bool CROP = ST && is_step(MODE);               // store step modes: the image is a crop of a frame
+  constexpr int ES = (MODE == MODE_EVAL_S16 || MODE == MODE_STEP_S16) ? 2 : 1;      // store modes: bytes per raw code
+  bool ok = true;                                          // store modes: the record names a whole frame / crop of the stores
   const unsigned char* __restrict__ simg = nullptr;        // store modes: the raw frame's codes and the GT frame's planes
-  const unsigned char* __restrict__ sgt = nullptr;
-  if constexpr (ST) {
+  const unsigned char* __restrict__ sgt = nullptr;         // (store step modes: their codes at the crop's origin)
+  if constexpr (CROP) {
+    const int4 rec = a.pos[n];
+    ok = crop_record(rec, a.F, a.G, frame.x, frame.y, H, W);
+    if (!ok && threadIdx.x == 0) *a.status = 1;
+    const long long fplane = (long long)frame.x * frame.y, org = ok ? (long long)rec.z * frame.y + rec.w : 0;
+    simg = a.store + ((ok ? rec.x : 0) * fplane + org) * ES;
+    sgt = a.gstore + (ok ? rec.y : 0) * 3 * fplane + org;
+  } else if constexpr (ST) {
     const int4 rec = a.pos[n];
     ok = whole_frame_record(rec, a.F, a.G);
     if (!ok && threadIdx.x == 0) *a.status = 1;
@@ -244,7 +294,7 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
   float2 accB[RISP_BIG_ACC];
   float loss = 0.f;
   unsigned long long sse = 0;     // MODE_EVAL: this lane's sum of squared code differences
-  if (MODE == MODE_STEP) {
+  if (is_step(MODE)) {
 #pragma unroll
     for (int s = 0; s < SMAX; ++s)
 #pragma unroll
@@ -259,19 +309,24 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
 #pragma unroll
     for (int j = 0; j < WR - 1; ++j) {
       if constexpr (ST) {
-        row_issue_codes<HL, ES>(q, simg, reflect101(ra - HL + j, H), W, c0, active, lane);
+        if constexpr (CROP) row_issue_crop_codes<HL, ES>(q, simg, reflect101(ra - HL + j, H), frame.y, W, c0, active, lane);
+        else row_issue_codes<HL, ES>(q, simg, reflect101(ra - HL + j, H), W, c0, active, lane);
         row_finish<HL>(w[j], row_decode<HL, ES>(q, a.white_level), W, c0, active, lane);
       } else {
         row_issue<HL>(q, img, reflect101(ra - HL + j, H), W, c0, active, lane);
         row_finish<HL>(w[j], q, W, c0, active, lane);
       }
     }
-    if constexpr (ST) row_issue_codes<HL, ES>(q, simg, reflect101(ra + HL, H), W, c0, active, lane);
+    if constexpr (CROP) row_issue_crop_codes<HL, ES>(q, simg, reflect101(ra + HL, H), frame.y, W, c0, active, lane);
+    else if constexpr (ST) row_issue_codes<HL, ES>(q, simg, reflect101(ra + HL, H), W, c0, active, lane);
     else row_issue<HL>(q, img, reflect101(ra + HL, H), W, c0, active, lane);
     float4 gB = make_float4(0.f, 0.f, 0.f, 0.f), gG = gB, gR = gB;   // GT of the row being computed, fetched one row ahead
     if (MODE == MODE_STEP && active) {
       const long long o = (long long)ra * W + c0;
       gB = ld_stream4(gtb + o); gG = ld_stream4(gtb + plane + o); gR = ld_stream4(gtb + 2 * plane + o);
+    }
+    if constexpr (CROP) {
+      if (active) crop_gt_row(sgt, (long long)frame.x * frame.y, (long long)ra * frame.y + c0, gB, gG, gR);
     }
     for (int r = ra; r < rb; ++r) {
       if constexpr (ST) row_finish<HL>(w[WR - 1], row_decode<HL, ES>(q, a.white_level), W, c0, active, lane);
@@ -293,11 +348,15 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
         }
       }
       if (r + 1 < rb) {
-        if constexpr (ST) row_issue_codes<HL, ES>(q, simg, reflect101(r + 1 + HL, H), W, c0, active, lane);
+        if constexpr (CROP) row_issue_crop_codes<HL, ES>(q, simg, reflect101(r + 1 + HL, H), frame.y, W, c0, active, lane);
+        else if constexpr (ST) row_issue_codes<HL, ES>(q, simg, reflect101(r + 1 + HL, H), W, c0, active, lane);
         else row_issue<HL>(q, img, reflect101(r + 1 + HL, H), W, c0, active, lane);
         if (MODE == MODE_STEP && active) {
           const long long o = (long long)(r + 1) * W + c0;
           gB = ld_stream4(gtb + o); gG = ld_stream4(gtb + plane + o); gR = ld_stream4(gtb + 2 * plane + o);
+        }
+        if constexpr (CROP) {
+          if (active) crop_gt_row(sgt, (long long)frame.x * frame.y, (long long)(r + 1) * frame.y + c0, gB, gG, gR);
         }
       }
       Px<4> px;
@@ -386,7 +445,7 @@ pipeline_kernel(PipeArgs a, ChainDesc d) {
     }
   }
 
-  if (MODE == MODE_STEP) {
+  if (is_step(MODE)) {
     const int warps_per_image = gridDim.y * gridDim.x * kWarpsPerBlock;
     const int widx = (blockIdx.y * gridDim.x + blockIdx.x) * kWarpsPerBlock + wid;
     float* __restrict__ out = a.partial + ((long long)n * warps_per_image + widx) * RISP_NSLOT;
@@ -437,7 +496,8 @@ static PipeGeom pipe_geometry(int N, int H, int W) {
 }
 
 template <int MODE>
-static int launch_pipeline(const PipeArgs& a, const ChainDesc& d, int N, int dm_kind, bool big, cudaStream_t st) {
+static int launch_pipeline(const PipeArgs& a, const ChainDesc& d, int N, int dm_kind, bool big, cudaStream_t st,
+                           int2 frame = int2{0, 0}) {
   PipeGeom g = pipe_geometry(N, a.H, a.W);
   PipeArgs b = a;
   b.rows_per_chunk = g.rows_per_chunk;
@@ -448,7 +508,7 @@ static int launch_pipeline(const PipeArgs& a, const ChainDesc& d, int N, int dm_
 #define RISP_PIPE_SIG(DMK, SG)                                                       \
   if constexpr (!is_eval(MODE)) {                                                    \
     if (!done && sig == (SG)) {                                                      \
-      pipeline_kernel<DMK, MODE, (SG), false><<<grid, block, 0, st>>>(b, d);         \
+      pipeline_kernel<DMK, MODE, (SG), false><<<grid, block, 0, st>>>(b, d, frame);  \
       done = true;                                                                   \
     }                                                                                \
   }
@@ -456,9 +516,9 @@ static int launch_pipeline(const PipeArgs& a, const ChainDesc& d, int N, int dm_
   do {                                                                               \
     RISP_PIPE_SIG(DMK, RISP_SIG_A) RISP_PIPE_SIG(DMK, RISP_SIG_B) RISP_PIPE_SIG(DMK, RISP_SIG_C) RISP_PIPE_SIG(DMK, RISP_SIG_D) \
     if (!done) {                                                                     \
-      if constexpr (is_eval(MODE)) pipeline_kernel<DMK, MODE, 0u, false><<<grid, block, 0, st>>>(b, d);    \
-      else if (big) pipeline_kernel<DMK, MODE, 0u, true><<<grid, block, 0, st>>>(b, d); \
-      else pipeline_kernel<DMK, MODE, 0u, false><<<grid, block, 0, st>>>(b, d);      \
+      if constexpr (is_eval(MODE)) pipeline_kernel<DMK, MODE, 0u, false><<<grid, block, 0, st>>>(b, d, frame);    \
+      else if (big) pipeline_kernel<DMK, MODE, 0u, true><<<grid, block, 0, st>>>(b, d, frame); \
+      else pipeline_kernel<DMK, MODE, 0u, false><<<grid, block, 0, st>>>(b, d, frame);      \
     }                                                                                \
   } while (0)
   switch (dm_kind) {
@@ -633,13 +693,43 @@ extern "C" size_t risp_pipeline_step_workspace(int N, int H, int W, int P) {
   return (size_t)N * rows * RISP_NSLOT * sizeof(float) + finalize_rows_workspace(N, RISP_NSLOT);
 }
 
+// the inputs of the store steps: N crops of H x W (the step's geometry) out of frame stores of FH x FW frames
+struct StepStore {
+  const void* raw;
+  int bpc, F;
+  const unsigned char* gt;
+  int G, FH, FW;
+  const int* pos;
+  float white_level;
+  int* status;
+};
+
+static int check_store_step(const char* who, const StepStore& s, float* loss_out, int N, int h, int w) {
+  RISP_REQUIRE(s.raw && s.gt && s.pos && s.status && loss_out, RISP_E_INVALID,
+               "%s: raw_store, gt_store, pos, status and loss_out must be non-null", who);
+  RISP_REQUIRE(s.bpc == 1 || s.bpc == 2, RISP_E_INVALID, "%s: 1 or 2 bytes per raw code", who);
+  RISP_REQUIRE(s.F > 0 && s.G > 0 && N > 0 && N <= 65535 && h >= 4 && w >= 4 && h <= s.FH && w <= s.FW && s.white_level > 0.f,
+               RISP_E_INVALID, "%s: bad store arguments (F %d, G %d, N %d, %dx%d crops of %dx%d frames, white_level %g)", who, s.F,
+               s.G, N, h, w, s.FH, s.FW, (double)s.white_level);
+  RISP_REQUIRE((long long)s.F * s.FH * s.FW < (1ll << 40) && (long long)s.G * 3 * s.FH * s.FW < (1ll << 40), RISP_E_INVALID,
+               "%s: stores of %d / %d frames of %dx%d are too large", who, s.F, s.G, s.FH, s.FW);
+  // the packed kernels read the stores through tensor maps (16-byte aligned base, rows of a 16-byte multiple); both kernels
+  // march 4-column lanes down row pairs
+  RISP_REQUIRE(s.FW % 16 == 0 && w % 4 == 0 && h % 2 == 0 && aligned16(s.raw) && aligned16(s.gt) && aligned16(s.pos),
+               RISP_E_UNSUPPORTED, "%s: needs 16-byte aligned stores and pos, frames with W %% 16 == 0 and crops with w %% 4 == 0 "
+               "and h even (got %dx%d crops of %dx%d frames)", who, h, w, s.FH, s.FW);
+  return RISP_OK;
+}
+
+// gt_is_dy: gt holds dL/dy (risp_pipeline_bwd).  store (nullable): the store steps, whose raw and gt come from the stores
 static int pipeline_step_impl(const char* who, bool gt_is_dy, bool l1, const float* raw, const float* gt, float* y_out,
                               float* loss_out, float* dparams, int N, int H, int W, int dm_kind, float dm_clip_hi,
                               const int* ops, const int* param_off, const int* iarg, int S, const float* params,
-                              int param_stride, int P, void* workspace, size_t workspace_bytes, risp_stream_t stream) {
-  int rc = check_frame(who, raw, N, H, W);
+                              int param_stride, int P, void* workspace, size_t workspace_bytes, risp_stream_t stream,
+                              const StepStore* store = nullptr) {
+  int rc = store ? check_store_step(who, *store, loss_out, N, H, W) : check_frame(who, raw, N, H, W);
   if (rc != RISP_OK) return rc;
-  RISP_REQUIRE(gt && aligned16(gt) && (gt_is_dy || loss_out), RISP_E_ALIGN, "%s: gt/dy/loss_out null or unaligned", who);
+  RISP_REQUIRE(store || (gt && aligned16(gt) && (gt_is_dy || loss_out)), RISP_E_ALIGN, "%s: gt/dy/loss_out null or unaligned", who);
   RISP_REQUIRE(!y_out || aligned16(y_out), RISP_E_ALIGN, "%s: y_out must be 16-byte aligned", who);
   ChainDesc d;
   int Pn = 0;
@@ -662,8 +752,21 @@ static int pipeline_step_impl(const char* who, bool gt_is_dy, bool l1, const flo
   int frows = 0;
   RISP_REQUIRE(!l1 || (P > 0 && use_fused() && fused_handles(d, N, param_stride, H, W)), RISP_E_UNSUPPORTED,
                "%s: the fused L1 step exists for the pre-instantiated chain signatures only (run the unfused path)", who);
-  rc = (P > 0 && use_fused()) ? fused_launch(gt_is_dy ? 2 : (l1 ? 3 : 1), raw, gt, y_out, partial, params, param_stride, N, H, W, dm_kind, dm_clip_hi, d, st, &frows) : 1;
-  if (rc == 1) {
+  if (P > 0 && use_fused())
+    rc = store ? fused_step_store_launch(l1, store->raw, store->bpc, store->F, store->gt, store->G, store->FH, store->FW,
+                                         store->pos, store->status, store->white_level, partial, params, param_stride, N, H,
+                                         W, dm_kind, dm_clip_hi, d, st, &frows)
+               : fused_launch(gt_is_dy ? 2 : (l1 ? 3 : 1), raw, gt, y_out, partial, params, param_stride, N, H, W, dm_kind,
+                              dm_clip_hi, d, st, &frows);
+  else
+    rc = 1;
+  if (rc == 1 && store) {
+    PipeArgs a{nullptr, nullptr, nullptr, partial, params, param_stride, H, W, 0, dm_clip_hi, 0, nullptr, nullptr,
+               static_cast<const unsigned char*>(store->raw), store->gt, reinterpret_cast<const int4*>(store->pos),
+               store->status, store->white_level, store->F, store->G};
+    rc = store->bpc == 2 ? launch_pipeline<MODE_STEP_S16>(a, d, N, dm_kind, big, st, int2{store->FH, store->FW})
+                         : launch_pipeline<MODE_STEP_U8>(a, d, N, dm_kind, big, st, int2{store->FH, store->FW});
+  } else if (rc == 1) {
     PipeArgs a{raw, gt, y_out, partial, params, param_stride, H, W, 0, dm_clip_hi, gt_is_dy ? 1 : 0};
     rc = launch_pipeline<MODE_STEP>(a, d, N, dm_kind, big, st);
   } else if (rc == RISP_OK) {
@@ -730,4 +833,30 @@ extern "C" int risp_pipeline_l1_step(const float* raw, const float* gt, float* y
   return pipeline_step_impl("risp_pipeline_l1_step", false, true, raw, gt, y_out, loss_out, dparams, N, H, W, dm_kind,
                             dm_clip_hi, ops, param_off, iarg, S, params, param_stride, P, workspace, workspace_bytes,
                             stream);
+}
+
+// The MSE / L1 step on N crops of h x w out of frame stores (see the header): the dispatch and the finaliser of
+// risp_pipeline_mse_step / risp_pipeline_l1_step, with raw and gt read as codes.
+extern "C" int risp_pipeline_mse_step_store(const void* raw_store, int raw_bytes_per_code, int F, const unsigned char* gt_store,
+                                            int G, int H, int W, const int* pos, int N, float white_level, int* status, int h,
+                                            int w, float* loss_out, float* dparams, int dm_kind, float dm_clip_hi,
+                                            const int* ops, const int* param_off, const int* iarg, int S, const float* params,
+                                            int param_stride, int P, void* workspace, size_t workspace_bytes,
+                                            risp_stream_t stream) {
+  const StepStore s{raw_store, raw_bytes_per_code, F, gt_store, G, H, W, pos, white_level, status};
+  return pipeline_step_impl("risp_pipeline_mse_step_store", false, false, nullptr, nullptr, nullptr, loss_out, dparams, N, h,
+                            w, dm_kind, dm_clip_hi, ops, param_off, iarg, S, params, param_stride, P, workspace,
+                            workspace_bytes, stream, &s);
+}
+
+extern "C" int risp_pipeline_l1_step_store(const void* raw_store, int raw_bytes_per_code, int F, const unsigned char* gt_store,
+                                           int G, int H, int W, const int* pos, int N, float white_level, int* status, int h,
+                                           int w, float* loss_out, float* dparams, int dm_kind, float dm_clip_hi,
+                                           const int* ops, const int* param_off, const int* iarg, int S, const float* params,
+                                           int param_stride, int P, void* workspace, size_t workspace_bytes,
+                                           risp_stream_t stream) {
+  const StepStore s{raw_store, raw_bytes_per_code, F, gt_store, G, H, W, pos, white_level, status};
+  return pipeline_step_impl("risp_pipeline_l1_step_store", false, true, nullptr, nullptr, nullptr, loss_out, dparams, N, h,
+                            w, dm_kind, dm_clip_hi, ops, param_off, iarg, S, params, param_stride, P, workspace,
+                            workspace_bytes, stream, &s);
 }

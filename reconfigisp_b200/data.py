@@ -7,7 +7,8 @@ as codes (2 + 3 B per pixel for a 16-bit raw and its 8-bit GT), and fills each b
 plan -- B records of 16 bytes -- crosses PCIe per batch.
 
     ds = DeviceDataset(raws, gts, white_level=1023., crop=224, rank=rank, world=world)
-    model.feed_data(ds.sample(8, 'all'))                        # tuning (IspModel): every frame of the shard
+    model.feed_data(ds.records(8, 'all'))                       # tuning (IspModel): the step reads the store's codes
+    model.feed_data(ds.sample(8, 'all'))                        # the same crops, decoded to fp32 first
     model.feed_data(ds.sample(4) + ds.sample(4, 'val'))         # search (DartsModel): DARTS train / validation halves
     frames, sse = ds.evaluate(net, 'val')                       # validation: every frame of the split, whole, once
 
@@ -119,6 +120,26 @@ def _host_codes(f):
     return f.contiguous()
 
 
+class StoreBatch:
+    """B crops of a `DeviceDataset` named by their records and not decoded: what `records()` returns.  `pos` is the
+    persistent (B,4) int32 device tensor of the (split, B) key; the next `records()` of that key overwrites it in stream
+    order.  A fused tuning step reads the crops straight from the stores (`ops.PipelineStep.store`); `decode()` gives the
+    fp32 (img (B,1,h,w), gt (B,3,h,w)) that `sample()` gives for the same records, in persistent buffers of the key."""
+
+    def __init__(self, ds, key, pos):
+        self.ds, self.key, self.pos = ds, key, pos
+        self.B, self.h, self.w = pos.shape[0], ds.h, ds.w
+
+    def decode(self):
+        """-> (img, gt) fp32 device tensors decoded from the records by one `ops.sample_crops` launch."""
+        ds = self.ds
+        bufs = ds._dec_bufs.get(self.key)
+        if bufs is None:
+            bufs = ds._dec_bufs[self.key] = (torch.empty((self.B, 1, self.h, self.w), device=ds.device, dtype=torch.float32),
+                                              torch.empty((self.B, 3, self.h, self.w), device=ds.device, dtype=torch.float32))
+        return ops.sample_crops(ds.raw_store, ds.gt_store, self.pos, self.h, self.w, ds.white_level, ds.status, *bufs)
+
+
 class DeviceDataset:
     """A dataset resident in HBM and its batched crop sampler (module docstring).
 
@@ -175,6 +196,7 @@ class DeviceDataset:
         self._upload(raw_list, gt_list, hwc)
         self.steps = {s: 0 for s in SPLITS}
         self._bufs = {}
+        self._recs, self._dec_bufs = {}, {}      # records(): per (split, B), the records and their decoded batch
         self._eval = {}          # evaluate(): per split, the records on the device and where they land in the gathered result
         self._eval_bufs = {}
 
@@ -221,12 +243,26 @@ class DeviceDataset:
         ops.sample_crops(self.raw_store, self.gt_store, pos, self.h, self.w, self.white_level, self.status, img, gt)
         return img, gt
 
+    def records(self, B, split='train'):
+        """The next batch of `split` as records, not decoded -> `StoreBatch`.  Advances the same plan step as `sample(B,
+        split)`, so records() and sample() draw the same crops from one sequence.  One copy of B*16 bytes into the same
+        (B,4) device tensor on every call with this (split, B), so a CUDA-graph step that reads it keeps replaying; no launch."""
+        plan = self.plan_.plan(split, self.steps[split], B)
+        self.steps[split] += 1
+        key = (split, B)
+        pos = self._recs.get(key)
+        if pos is None:
+            pos = self._recs[key] = torch.empty((B, 4), device=self.device, dtype=torch.int32)
+        pos.copy_(torch.from_numpy(plan), non_blocking=True)
+        return StoreBatch(self, key, pos)
+
     def check(self):
         """Wait for the device and raise if any launch since the last check met a bad record (then clear the flag)."""
         bad = int(self.status.item())
         if bad:
             self.status.zero_()
-            raise RuntimeError('risp_sample_crops skipped a record that was out of range or odd')
+            raise RuntimeError('a launch on the stores (sampler, store step or evaluation) skipped a record that was out of '
+                               'range or odd')
 
     def _eval_records(self, split):
         ev = self._eval.get(split)

@@ -793,6 +793,20 @@ class PipelineStep:
                self.chain.P, L.ptr(self.ws), self.ws.numel() * 4, L.stream())
         return self.loss, self.dparams
 
+    def store(self, raw_store, gt_store, pos, white_level, status, params):
+        """The same step on the N crops of H x W that the records pos (N,4) int32 CUDA name in the frame stores of
+        `sample_crops`, read as codes (`risp_pipeline_*_step_store`) -> (loss (1,), dparams), bitwise the values `__call__`
+        gives on `sample_crops(raw_store, gt_store, pos, H, W, white_level, ...)`.  A bad record sets status and adds nothing
+        (the normaliser stays N*3*H*W).  Needs frames with W % 16 == 0 (NotImplementedError otherwise)."""
+        F, FH, FW = _store_args(raw_store, gt_store, pos, status, 'PipelineStep.store')
+        if pos.shape[0] != self.N:
+            raise ValueError('PipelineStep.store: %d records for a step of %d images' % (pos.shape[0], self.N))
+        L.call(self.entry + '_store', L.ptr(raw_store), raw_store.element_size(), F, L.ptr(gt_store), gt_store.shape[0], FH, FW,
+               L.ptr(pos), self.N, float(white_level), L.ptr(status), self.H, self.W, L.ptr(self.loss), L.ptr(self.dparams),
+               self.dm, self.clip_hi, *self.chain.desc(), L.ptr(params), self.stride, self.chain.P, L.ptr(self.ws),
+               self.ws.numel() * 4, L.stream())
+        return self.loss, self.dparams
+
 
 class _PipelineMseFn(torch.autograd.Function):
     """loss = mse(pipeline(raw; params), gt) with d loss / d params from the same single pass."""

@@ -27,6 +27,7 @@ class IspModel:
         self.is_train = opt.get('is_train', True)
         self.netG = define_G(opt).to(self.device)
         self.netG_attr = self.netG
+        self._records = None
         self.img = self.gt = self.val_img = self.val_gt = self.meta = None
         self._output = None
         self.log_dict = OrderedDict()
@@ -58,14 +59,46 @@ class IspModel:
         self.load()
 
     # -- data ------------------------------------------------------------------------------------------------
+    @property
+    def img(self):
+        """The fed batch's raw (N,1,H,W) fp32; after a records feed, decoded from the stores on first use."""
+        if self._img is None and self._records is not None:
+            self._img, self._gt = self._records.decode()
+        return self._img
+
+    @img.setter
+    def img(self, v):
+        self._img = v
+
+    @property
+    def gt(self):
+        """The fed batch's target (N,3,H,W) fp32, decoded on first use like `img`."""
+        if self._gt is None and self._records is not None:
+            self._img, self._gt = self._records.decode()
+        return self._gt
+
+    @gt.setter
+    def gt(self, v):
+        self._gt = v
+
     def feed_data(self, data):
-        """(img, gt[, val_img, val_gt]) host or device tensors.
+        """(img, gt[, val_img, val_gt]) host or device tensors, or a `data.StoreBatch` (`DeviceDataset.records`).
+
+        A StoreBatch is kept as its records: when the fused step applies (`_fast_plan`, frames with W % 16 == 0, crops with
+        w % 4 == 0 and h even) `optimize_parameters` reads the crops' codes straight from the stores; `img` / `gt` are
+        decoded only when something needs them (`output`, `test`, `evaluate`, the step of any other pipeline).
 
         Host tensors are copied on a side stream into one of TWO persistent device buffer sets (alternating), and integer
         sensor / display codes are decoded there as well, so the copy of batch k+1 overlaps the step of batch k when the
         caller feeds the next batch before reading the loss:  optimize_parameters(); feed_data(next); loss.item().
         The step waits for its own batch's copy (event), and a buffer set is not overwritten before the step that read it
         has finished -- the plain feed_data(); optimize_parameters() order of the reference keeps working unchanged."""
+        from .data import StoreBatch
+        if isinstance(data, StoreBatch):
+            self._records, self._pending, self._output = data, None, None
+            self.img = self.gt = None
+            return
+        self._records = None
         if len(data) == 2:
             img, gt = data
         elif len(data) == 4:
@@ -174,20 +207,35 @@ class IspModel:
                           table=torch.empty((1, P), device=self.device), steps={})
         return self._fast
 
+    def _store_step(self):
+        """The fed StoreBatch when the fused step can read its crops from the stores, else None."""
+        rec = self._records
+        if rec is None or not self.opt.get('fast_step', True) or self._fast_plan() is None:
+            return None
+        if rec.h % 2 or rec.w % 4 or rec.ds.W % 16 or self.loss_type not in ('l1', 'l2'):
+            return None
+        return rec
+
     def _fast_loss_and_grads(self):
         f = self._fast_plan()
-        H, W = self.img.shape[2:]
-        if f is None or H % 2 or W % 4 or self.loss_type not in ('l1', 'l2'):
+        rec = self._store_step()
+        if f is None:
+            return False
+        N, H, W = (rec.B, rec.h, rec.w) if rec is not None else (self.img.shape[0],) + tuple(self.img.shape[2:])
+        if H % 2 or W % 4 or self.loss_type not in ('l1', 'l2'):
             return False
         from . import _lib as L
-        N = self.img.shape[0]
         key = (N, H, W)
         step = f['steps'].get(key)
         if step is None:
             step = f['steps'][key] = ops.PipelineStep(N, H, W, f['dm'], f['chain'], self.device, l1=(self.loss_type == 'l1'))
         P = f['logits'].numel()
         L.call('risp_param_table_fwd', L.ptr(f['logits']), L.ptr(f['a']), L.ptr(f['b']), L.ptr(f['table']), P, L.stream())
-        loss, dtable = step(self.img, self.gt, f['table'])
+        if rec is not None:
+            ds = rec.ds
+            loss, dtable = step.store(ds.raw_store, ds.gt_store, rec.pos, ds.white_level, ds.status, f['table'])
+        else:
+            loss, dtable = step(self.img, self.gt, f['table'])
         L.call('risp_param_table_bwd', L.ptr(f['logits']), L.ptr(f['a']), L.ptr(dtable), L.ptr(f['grad']), P, L.stream())
         self.l_pix = loss.view(())
         # device scalar living in the step's persistent buffer: the NEXT step overwrites it, so read (`.item()`) or clone it
@@ -217,8 +265,12 @@ class IspModel:
         self._mark_used()
 
     def _graph_signature(self):
-        return (self.img.data_ptr(), self.gt.data_ptr(), tuple(self.img.shape), tuple(self.gt.shape),
-                tuple(float(g['lr']) for g in self.optimizer_G.param_groups))
+        lrs = tuple(float(g['lr']) for g in self.optimizer_G.param_groups)
+        rec = self._store_step()
+        if rec is not None:          # the captured store step reads the record buffer and the stores
+            return ('records', rec.pos.data_ptr(), rec.ds.raw_store.data_ptr(), rec.ds.gt_store.data_ptr(),
+                    (rec.B, rec.h, rec.w), lrs)
+        return (self.img.data_ptr(), self.gt.data_ptr(), tuple(self.img.shape), tuple(self.gt.shape), lrs)
 
     def _graph_replay(self):
         key = self._graph_signature()

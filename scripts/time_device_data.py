@@ -5,10 +5,13 @@
 Prints the card and its power limit, then per workload the ms per step of
   (a) the step on resident fp32 data (`bench.py`'s `value` loop),
   (b) `DeviceDataset.sample` + step, with and without reading the loss every step,
+  (d) `DeviceDataset.records` + the step reading the store's codes (MSE and L1 models),
   (c) `feed_data` of pinned host int16 raw + uint8 GT codes + step + loss read (`bench.py`'s `e2e` loop),
 for the bench's tuning workload (4 x 12 MP whole-frame crops, store of 16 synthetic frames) and the reference's tuning
-shape (8 x 224^2 crops from the same 12 MP frames), and the sampler kernel alone: 21 B per output pixel (2 B raw code +
-3 B GT codes read, 16 B fp32 written) over CUDA-event time.  Each figure is timed `--reps` times (min / max shown)."""
+shape (8 x 224^2 crops from the same 12 MP frames); then the kernels alone, records already on the device: the sampler
+(21 B per output pixel: 2 B raw code + 3 B GT codes read, 16 B fp32 written, over CUDA-event time) and the MSE / L1 step
+(parameter table, step kernel, finaliser) on the decoded fp32 batch against the same step reading the store.  Each figure is
+timed `--reps` times (min / max shown); the arms of a workload take turns within each repetition."""
 import argparse
 import os
 import subprocess
@@ -56,27 +59,45 @@ def card():
     return q or torch.cuda.get_device_name()
 
 
+def alternate(arms, n, warmup, reps):
+    """timed() of every arm, the arms taking turns within each repetition -> {name: ms list}."""
+    res = {k: [] for k in arms}
+    for r in range(reps):
+        for k, (fn, nk) in arms.items():
+            res[k] += timed(fn, nk or n, warmup if r == 0 else 2, 1)
+    return res
+
+
 def workload(ds, raws, gts, B, crop, reps, steps):
-    """(a), (b), (c) for B crops of `crop` per step; -> dict of ms lists."""
+    """(a), (b), (d), (c) and the kernels for B crops of `crop` per step; -> dict of ms lists."""
     dev = torch.device('cuda')
     h, w = crop
-    res = {}
     # (a) resident fp32 data: decoded once from the store's first frames
     model = IspModel(opt_tuning())
     img0, gt0 = ds.sample(B, 'all')
     model.feed_data((img0.clone(), gt0.clone()))
-    res['a_resident'] = timed(model.optimize_parameters, steps, 5, reps)
-
     # (b) sample + step (the model reads the sampler's persistent buffers in place: the captured step keeps replaying)
+    model_b = IspModel(opt_tuning())
+
     def step_b():
-        model.feed_data(ds.sample(B, 'all'))
-        model.optimize_parameters()
+        model_b.feed_data(ds.sample(B, 'all'))
+        model_b.optimize_parameters()
 
     def step_b_item():
         step_b()
-        return float(model.log_dict['loss'].item())
-    res['b_sample_step'] = timed(step_b, steps, 5, reps)
-    res['b_sample_step_loss_read'] = timed(step_b_item, steps, 5, reps)
+        return float(model_b.log_dict['loss'].item())
+    # (d) records + the step reading the store (the captured step reads the persistent record buffer)
+    models_d = {loss: IspModel(dict(opt_tuning(), train=dict(opt_tuning()['train'], pixel_criterion=loss))) for loss in ('l2', 'l1')}
+
+    def step_d(loss):
+        def fn():
+            models_d[loss].feed_data(ds.records(B, 'all'))
+            models_d[loss].optimize_parameters()
+        return fn
+    res = alternate({'a_resident': (model.optimize_parameters, 0), 'b_sample_step': (step_b, 0),
+                     'd_records_store_step_mse': (step_d('l2'), 0), 'd_records_store_step_l1': (step_d('l1'), 0),
+                     'b_sample_step_loss_read': (step_b_item, 0)}, steps, 5, reps)
+    assert all(m._store_step() is not None for m in models_d.values()), 'the store step did not run'
 
     # (c) pinned host codes, double-buffered feed, loss read every step (bench.py's e2e loop)
     rec = ds.plan('all', 0, B)
@@ -98,9 +119,19 @@ def workload(ds, raws, gts, B, crop, reps, steps):
     ref = torch.stack([raws[f][:, y:y + h, x:x + w] for f, y, x in zip(fr, rec[:, 2], rec[:, 3])]).to(dev)
     assert torch.equal(img, ops.decode_codes(ref.contiguous(), 1023.)), 'sampled crops differ from the decoded codes'
 
-    # the sampler kernel alone, records already on the device
+    # the kernels alone, records already on the device: the sampler, and each step on the decoded batch / on the store
     pos = torch.from_numpy(rec).to(dev)
-    res['kernel'] = timed(lambda: ops.sample_crops(ds.raw_store, ds.gt_store, pos, h, w, 1023., ds.status, img, gt), 200, 10, reps)
+    f = models_d['l2']._fast_plan()
+    tab = f['table']
+    kern = {'kernel': (lambda: ops.sample_crops(ds.raw_store, ds.gt_store, pos, h, w, 1023., ds.status, img, gt), 200)}
+    for loss in ('l2', 'l1'):
+        st = ops.PipelineStep(B, h, w, f['dm'], f['chain'], dev, l1=(loss == 'l1'))
+        kern['step_%s_fp32' % loss] = ((lambda st=st: st(img, gt, tab)), 200)
+        kern['step_%s_store' % loss] = ((lambda st=st: st.store(ds.raw_store, ds.gt_store, pos, 1023., ds.status, tab)), 200)
+        a = [t.clone() for t in st(img, gt, tab)]
+        b = [t.clone() for t in st.store(ds.raw_store, ds.gt_store, pos, 1023., ds.status, tab)]
+        assert all(torch.equal(x, y) for x, y in zip(a, b)), 'the store step differs from the step on the decoded batch'
+    res.update(alternate(kern, 200, 10, reps))
     ds.check()
     return res
 
